@@ -2,7 +2,7 @@
 """Headline benchmark: flow.log_prob samples/s of an 8-layer spline-coupling flow, d=64
 (BASELINE.json metric / configs[2]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--kind quadratic|cubic] [--hidden 64]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--kind quadratic|cubic] [--hidden 64] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...        # the CPU arm (oracle port of the reference)
 
@@ -11,6 +11,9 @@ ranks, no data-path collective: strong scaling, total work fixed as BASELINE.jso
 `value` is timed with CUDA events with the shard already resident in HBM; `e2e` runs the same
 pass from pinned HOST memory through the public API (H2D copy of the rows and D2H copy of the
 log-probabilities inside the timed region).  Prints ONE JSON line on rank 0.
+
+Weights and inputs come from fixed seeds, so two builds run with the same arguments see the same inputs;
+`--dump-outputs DIR` writes what the last timed step of each timed workload returned (`dump`) to compare them.
 """
 from __future__ import annotations
 
@@ -77,7 +80,12 @@ def parse():
     ap.add_argument('--workload', default='logprob', choices=['logprob', 'cubic', 'quadratic_h256', 'affine', 'neural', 'train'],
                     help='logprob = BASELINE.json configs[2] (the headline, default); affine = configs[1]; '
                          'neural = configs[3]; train = configs[4] (side measurements, same JSON schema)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed step returned as DIR/<name>.npy (see dump)')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    return args
 
 
 def build_layers(kind, hidden):
@@ -92,6 +100,23 @@ def build_layers(kind, hidden):
         tr = st.Spline(D, BINS, latent_net=net, lower=LOWER, upper=UPPER, spline_type=kind)
         layers.append(st.Coupling(tr, mask=MASKS[i % 2]))
     return layers
+
+
+def dump(dirname, outputs, max_elems):
+    """Write the outputs of the last timed step, {name: tensor}, as dirname/<name>.npy in float32 (float64 stays
+    float64), rank 0's rows.  A tensor of more than `max_elems` elements is written as a fixed sample of its rows
+    (first dimension): the rows a generator seeded with 0 draws first, in ascending order, the same in every run
+    of the same shape.  The callers' limits keep all files of one run under 64 MB."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        if t.numel() > max_elems:
+            keep = max(1, max_elems // (t[0].numel() if t.dim() > 1 else 1))
+            idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[idx.to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(dirname, name + '.npy'), a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 def workload_name(kind, hidden, batch):
@@ -200,8 +225,10 @@ def run_reference(args):
             O.flow_log_prob(spec, y)
         t = time.perf_counter()
         for _ in range(args.steps):
-            O.flow_log_prob(spec, y)
+            lp = O.flow_log_prob(spec, y)
         dt = time.perf_counter() - t
+    if args.dump_outputs:
+        dump(args.dump_outputs, {'log_prob': lp}, 1 << 22)
     value = rows * args.steps / dt
     sample = (f'{rows} rows per step of the same workload; oracle port of the reference (torch CPU ops, '
               f'no O(N^2) domain re-check), {n_threads} threads, {cpu_model()}')
@@ -244,7 +271,7 @@ def _profile_traffic(key):
 
 def _timed(step, steps, warmup, dev, world):
     """W warm-up steps, K timed steps between barriers; CUDA events on the launching stream, max over ranks.
-    -> (ms per step, library launches inside the timed region)"""
+    -> (ms per step, library launches inside the timed region, what the last step returned)"""
     import torch.distributed as dist
     from stribor_b200 import _ops
 
@@ -259,13 +286,13 @@ def _timed(step, steps, warmup, dev, world):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        step()
+        out = step()
     e1.record()
     barrier()
     tm = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(tm, op=dist.ReduceOp.MAX)
-    return tm.item() / steps, int(_ops.launch_count() - n0)
+    return tm.item() / steps, int(_ops.launch_count() - n0), out
 
 
 def _cpu_rate(fn, units, min_seconds=0.0):
@@ -302,8 +329,7 @@ def side_config(workload, args, dev, rank, world, want_cpu):
     from oracle import coupling_flow_oracle as O          # cpu_baseline leg only (rank 0, N = 1)
 
     hbm_peak, tf_peak, peak_src = _peaks()
-    steps = max(3, min(args.steps, 5))
-    warmup = max(3, min(args.warmup, 3))
+    steps, warmup = args.steps, args.warmup
     torch.manual_seed(123)
     res = {'steps': steps, 'warmup': warmup, 'n_gpus': world, 'higher_is_better': True, 'scaling': 'strong',
            'dtype': 'f32', 'data': 'synthetic'}
@@ -322,6 +348,7 @@ def side_config(workload, args, dev, rank, world, want_cpu):
                 return flow.log_prob(y)
         unit, per_step = 'samples/s', rows_g
         ins, n_out = [y], 1
+        out_names = ('log_prob',)
         pipe_fn = lambda yy: flow.log_prob(yy)
         if workload == 'cubic':
             bytes_unit, flops_unit, bound = LAYERS * (8 * d + 8), 2 * (32 * 64 + 64 * 32 * 34) * LAYERS, 'hbm'
@@ -351,6 +378,7 @@ def side_config(workload, args, dev, rank, world, want_cpu):
                 return flow.log_prob(y), flow.inverse(y)
         unit, per_step = 'samples/s (log_prob + inverse per sample)', rows_g
         ins, n_out = [y], 2
+        out_names = ('log_prob', 'inverse')
         pipe_fn = lambda yy: (flow.log_prob(yy), flow.inverse(yy))
         bytes_unit = LAYERS * (8 * d + 8) + LAYERS * 8 * d
         flops_unit, bound = 2 * LAYERS * 2 * (32 * 256 + 256 * 256 + 256 * 64), 'tensor'
@@ -379,6 +407,7 @@ def side_config(workload, args, dev, rank, world, want_cpu):
                 return flow(x, t=t)
         unit, per_step = 'rows/s', B * T
         ins, n_out = [x, t], 1
+        out_names = ('y',)
         pipe_fn = lambda xx, tt: flow(xx, t=tt)
         bytes_unit, flops_unit, bound = nl * (2 * 4 * d + 4), nl * 2 * (9 * 64 + 64 * 16), 'hbm'
         traffic_key = 'neural_dram_bytes_per_row'
@@ -408,12 +437,12 @@ def side_config(workload, args, dev, rank, world, want_cpu):
             os.environ['STRIBOR_B200_TRAIN_HYBRID'] = '1'
         name += (f', micro-batches of {args.micro_rows} rows' + (', hybrid path' if args.hybrid else ', fused backward kernel'))
         dp = DataParallelNLL(flow, micro_rows=args.micro_rows)
-        steps = 3
 
         def step():
             return dp.step(y, rows_g)
         unit, per_step = 'samples/s', rows_g
         ins, n_out = [y], 0
+        out_names = ('loss',)               # and the gradients, all-reduced, as one flat 'grad'
         pipe_fn = None
         bytes_unit = LAYERS * (8 * d + 8) + LAYERS * 12 * d
         flops_unit, bound = 3 * LAYERS * 2 * (64 * 64 + 64 * 64 * P), 'tensor'
@@ -432,10 +461,14 @@ def side_config(workload, args, dev, rank, world, want_cpu):
             cpu_step()
             cpu = _cpu_rate(cpu_step, n) + (f'{n} rows, one fwd+bwd of the same flow through torch autograd on the oracle port',)
 
-    ms_step, launches = _timed(step, steps, warmup, dev, world)
+    ms_step, launches, last = _timed(step, steps, warmup, dev, world)
+    if args.dump_outputs and rank == 0:
+        outs = dict(zip(out_names, last if isinstance(last, (tuple, list)) else (last,)))
+        if workload == 'train':
+            outs['grad'] = torch.cat([p.grad.reshape(-1) for p in flow.parameters()])
+        dump(args.dump_outputs, {f'{workload}.{k}': v for k, v in outs.items()}, 1 << 20)
     value = per_step / (ms_step * 1e-3)
     rows_local = ins[0].shape[0] * (ins[0].shape[1] if workload == 'neural' else 1)
-    res['steps'] = steps
     res.update({'metric': f'{workload} throughput', 'value': value, 'unit': unit, 'ms_per_step': ms_step,
                 'config': {'workload': name, 'l2_policy': 'inputs larger than L2' if ins[0].numel() * 4 > L2_BYTES
                            else 'inputs + outputs of one step exceed L2 together'},
@@ -473,7 +506,7 @@ def side_config(workload, args, dev, rank, world, want_cpu):
         sample = sample if isinstance(sample, (tuple, list)) else (sample,)
         outs_h = [torch.empty((ins[0].shape[0],) + tuple(o.shape[1:]), pin_memory=True) for o in sample]
         k = 3
-        ms_e, _ = _timed(lambda: pipe.map(pipe_fn, ins_h, outs_h), k, 2, dev, world)
+        ms_e = _timed(lambda: pipe.map(pipe_fn, ins_h, outs_h), k, 2, dev, world)[0]
         res['e2e'] = {'value': per_step / (ms_e * 1e-3), 'unit': unit,
                       'h2d_bytes_per_step': sum(t_.numel() * 4 for t_ in ins_h) * world,
                       'd2h_bytes_per_step': sum(o.numel() * 4 for o in outs_h) * world,
@@ -487,7 +520,7 @@ def side_config(workload, args, dev, rank, world, want_cpu):
         def e2e_step():
             ybuf.copy_(y_h, non_blocking=True)
             return float(dp.step(ybuf, rows_g))
-        ms_e, _ = _timed(e2e_step, 2, 1, dev, world)
+        ms_e = _timed(e2e_step, 2, 1, dev, world)[0]
         res['e2e'] = {'value': per_step / (ms_e * 1e-3), 'unit': unit, 'h2d_bytes_per_step': y_h.numel() * 4 * world,
                       'd2h_bytes_per_step': 4 * world, 'how': 'pinned host batch -> H2D -> DataParallelNLL.step -> loss.item()'}
         res['allreduce_bytes_per_step'] = int(dp.last_allreduce_bytes)
@@ -595,8 +628,7 @@ def main():
     time.sleep(0.25)
     t_load0 = time.perf_counter()
     for _ in range(args.warmup):
-        lp = step()
-    assert torch.isfinite(lp).all().item(), 'non-finite log_prob'
+        step()
     barrier()
     n0 = _ops.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -616,6 +648,9 @@ def main():
         t1 = time.perf_counter()
     clocks = sampler.stop(t_load0, t1)
     clocks['window'] = 'warm-up + timed steps (same workload)'
+    assert torch.isfinite(lp).all().item(), 'non-finite log_prob'
+    if args.dump_outputs and rank == 0:
+        dump(args.dump_outputs, {'log_prob': lp}, 1 << 22)
     tmax = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)

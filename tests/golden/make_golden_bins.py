@@ -9,12 +9,20 @@ after the other in fp32.  ``stribor.util.searchsorted`` (util/search_sorted.py:3
 layer runs, and its flat result -- the reference gathers the in-box elements into a 1-D vector
 (rational_quadratic_spline.py:161-164, cubic_spline.py:55-67) -- is scattered back to ``[rows, dim]`` with -1
 for out-of-box elements and for the pass-through dims of a coupling (the reference transforms those too and
-discards the result; the kernels never touch them).  Per spline layer ``i``:
+discards the result; the kernels never touch them).  Per spline layer ``i`` the recording holds
 
-    case|L{i}|x        layer input                        case|L{i}|fwd.bins   search on cumwidths at x
-    case|L{i}|y        reference forward output           case|L{i}|inv.bins   search on cumheights at y
-    case|L{i}|xr       reference inverse of y             case|L{i}|inv.fbins  forward re-search at xr (couplings:
-                                                                               flow.py:42-47 -> coupling.py:84-95)
+    x        layer input                        fwd.bins   search on cumwidths at x
+    y        reference forward output           inv.bins   search on cumheights at y
+    xr       reference inverse of y             inv.fbins  forward re-search at xr (couplings:
+                                                           flow.py:42-47 -> coupling.py:84-95)
+
+and ``stored_form`` writes it compactly (``tests/test_bins_golden.py:recorded_layers`` reads it back):
+
+    case|L{i}|x        only when it is neither the case input nor the previous spline layer's y
+    case|L{i}|y^x      bits of y XOR bits of x (int32; exact, and zero on the pass-through dims)
+    case|L{i}|xr^x     bits of xr XOR bits of x (int32; near zero: xr is x up to the round trip)
+    case|L{i}|fwd.bins, inv.bins, inv.fbins
+    case|rows          the larger BIN_CASES keep a fixed half of their rows, these (sorted) ones
 """
 import os
 import sys
@@ -100,11 +108,33 @@ def record_case(name):
     return out
 
 
+def stored_form(name, rec):
+    """record_case(name) -> the arrays reference_bins.npz stores for the case (module docstring)"""
+    layers = sorted({int(k.split('|')[1][1:]) for k in rec})
+    rows = None
+    if name in cases.BIN_CASES:
+        n = rec[f'{name}|L{layers[0]}|x'].shape[0]
+        rows = np.sort(np.random.RandomState(0).choice(n, n // 2, replace=False))
+    pick = (lambda a: a) if rows is None else (lambda a: a[rows])
+    out = {} if rows is None else {f'{name}|rows': rows}
+    for i in layers:
+        p = f'{name}|L{i}|'
+        x = rec[p + 'x']
+        if i > 0 and f'{name}|L{i - 1}|y' not in rec:
+            out[p + 'x'] = pick(x)
+        for k in ('y', 'xr'):
+            out[p + k + '^x'] = pick(rec[p + k].view(np.int32) ^ x.view(np.int32))
+        for k in ('fwd.bins', 'inv.bins', 'inv.fbins'):
+            if p + k in rec:
+                out[p + k] = pick(rec[p + k])
+    return out
+
+
 def main():
     blob = {}
     for name in cases.spline_cases():
         r = record_case(name)
-        blob.update(r)
+        blob.update(stored_form(name, r))
         n_el = sum(int((v >= 0).sum()) for k, v in r.items() if k.endswith('fwd.bins'))
         print(name, len(r), 'arrays,', n_el, 'searched elements')
     path = os.path.join(HERE, 'reference_bins.npz')

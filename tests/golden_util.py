@@ -25,6 +25,18 @@ def has(case, key, prec='f32'):
     return f'{case}|{key}|{prec}' in blob()
 
 
+def rows(case, key):
+    """Indices of the rows recorded for (case, key) when a large output is stored as a fixed sample of its rows
+    (make_golden.sample_large), else None."""
+    return torch.from_numpy(blob()[f'{case}|{key}|rows']) if has(case, key, 'rows') else None
+
+
+def pick(case, key, got):
+    """`got` restricted to the rows recorded for (case, key)"""
+    r = rows(case, key)
+    return got if r is None else got[r.to(got.device)]
+
+
 def case_names(prefixes=None, ops=None):
     out = []
     for n in cases.CASES:

@@ -30,25 +30,47 @@ def spline_layers(name):
     return case, out
 
 
-@pytest.mark.parametrize('name', cases.spline_cases())
-def test_oracle_bins_match_reference(name):
+def recorded_layers(name):
+    """-> (case, rows, [(layer index, layer spec, record)]) for the spline layers of a case, decoded from the
+    compact stored form (make_golden_bins.stored_form).  A record holds numpy arrays: the layer input x, the
+    reference's output y and its inverse xr of y, and its searches fwd.bins, inv.bins (and inv.fbins when
+    recorded), over the recorded rows: `rows` indexes the case's rows, None when all of them are recorded."""
     case, layers = spline_layers(name)
     b = bins_blob()
+    rows = b.get(f'{name}|rows')
+    x = case['inputs']['x'].numpy()
+    if rows is not None:
+        x = x.reshape(-1, x.shape[-1])[rows]
+    out = []
+    for i, layer in layers:
+        p = f'{name}|L{i}|'
+        x = b.get(p + 'x', x)                   # else: the case input, or the previous spline layer's y
+        bits = x.view(np.int32)
+        rec = {'x': x, 'y': (bits ^ b[p + 'y^x']).view(np.float32), 'xr': (bits ^ b[p + 'xr^x']).view(np.float32)}
+        rec.update({k: b[p + k] for k in ('fwd.bins', 'inv.bins', 'inv.fbins') if p + k in b})
+        out.append((i, layer, rec))
+        x = rec['y']
+    return case, rows, out
+
+
+@pytest.mark.parametrize('name', cases.spline_cases())
+def test_oracle_bins_match_reference(name):
+    case, _, layers = recorded_layers(name)
     latent = case['inputs'].get('latent')
     assert layers
-    for i, layer in layers:
-        x = torch.from_numpy(b[f'{name}|L{i}|x'])
-        y = torch.from_numpy(b[f'{name}|L{i}|y'])
-        xr = torch.from_numpy(b[f'{name}|L{i}|xr'])
+    for i, layer, rec in layers:
+        x = torch.from_numpy(rec['x'])
+        y = torch.from_numpy(rec['y'])
+        xr = torch.from_numpy(rec['xr'])
         lead = x.shape[:-1]
-        want_f = torch.from_numpy(b[f'{name}|L{i}|fwd.bins']).long()
+        want_f = torch.from_numpy(rec['fwd.bins']).long()
         got_f = O.layer_bins(layer, x, inverse=False, latent=latent).reshape(want_f.shape)
         assert torch.equal(got_f, want_f), f'{name} L{i}: forward bins differ'
-        want_i = torch.from_numpy(b[f'{name}|L{i}|inv.bins']).long()
+        want_i = torch.from_numpy(rec['inv.bins']).long()
         got_i = O.layer_bins(layer, y, inverse=True, latent=latent).reshape(want_i.shape)
         assert torch.equal(got_i, want_i), f'{name} L{i}: inverse bins differ'
-        if f'{name}|L{i}|inv.fbins' in b:
-            want_r = torch.from_numpy(b[f'{name}|L{i}|inv.fbins']).long()
+        if 'inv.fbins' in rec:
+            want_r = torch.from_numpy(rec['inv.fbins']).long()
             got_r = O.layer_bins(layer, xr, inverse=False, latent=latent).reshape(want_r.shape)
             assert torch.equal(got_r, want_r), f'{name} L{i}: re-searched forward bins differ'
         # the recorded layer outputs are the oracle's too (same tolerance as test_oracle_golden)

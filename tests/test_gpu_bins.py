@@ -22,7 +22,7 @@ import cases
 from oracle import coupling_flow_oracle as O
 from stribor_b200 import _lib, _ops
 from stribor_b200.spec import layers_from_spec
-from test_bins_golden import bins_blob, spline_layers
+from test_bins_golden import recorded_layers
 
 pytestmark = pytest.mark.gpu
 DEV = 'cuda'
@@ -79,39 +79,57 @@ def compare_bins(got, want, layer, point, inverse, latent):
 
 def run_case(name):
     """-> list of per-layer dicts with the flip counts of the three searches"""
-    case, layers = spline_layers(name)
-    b = bins_blob()
+    case, rows, layers = recorded_layers(name)
     mods = [m.to(DEV) for m in layers_from_spec(case['spec'])]
     latent = case['inputs'].get('latent')
     lat_dev = None if latent is None else latent.to(DEV)
-    rows = []
-    for i, layer in layers:
+    # where only some rows of a case are recorded, the kernels still run on the whole batch (its tile shapes):
+    # the recorded rows take their places in it, the others carry the kernels' own values, and the recorded
+    # rows are compared
+    whole = None if rows is None else case['inputs']['x'].to(DEV)
+    rows = None if rows is None else torch.from_numpy(rows).to(DEV)
+
+    def batch(v):
+        v = torch.from_numpy(v).to(DEV)
+        if rows is None:
+            return v
+        out = whole.clone()
+        out[rows] = v
+        return out
+
+    def recorded(t):
+        return t if rows is None else t[rows]
+
+    out = []
+    for i, layer, r in layers:
         mod = mods[i]
-        x = torch.from_numpy(b[f'{name}|L{i}|x'])
-        y = torch.from_numpy(b[f'{name}|L{i}|y'])
+        x, y = torch.from_numpy(r['x']), torch.from_numpy(r['y'])
         rec = {'case': name, 'layer': i}
         # forward search at the layer input
-        yc, fb, tp = cuda_bins(mod, x.to(DEV), lat_dev, _lib.FORWARD)
+        yc, fb, tp = cuda_bins(mod, batch(r['x']), lat_dev, _lib.FORWARD)
+        whole = yc
+        fb = recorded(fb)
         rec['tensor_path'] = tp
-        rec['fwd'] = compare_bins(fb, torch.from_numpy(b[f'{name}|L{i}|fwd.bins']), layer, x, False, latent)
+        rec['fwd'] = compare_bins(fb, torch.from_numpy(r['fwd.bins']), layer, x, False, latent)
         # inverse search at the reference's layer output
-        xc, ib, _ = cuda_bins(mod, y.to(DEV), lat_dev, _lib.INVERSE)
-        rec['inv'] = compare_bins(ib, torch.from_numpy(b[f'{name}|L{i}|inv.bins']), layer, y, True, latent)
+        xc, ib, _ = cuda_bins(mod, batch(r['y']), lat_dev, _lib.INVERSE)
+        ib = recorded(ib)
+        rec['inv'] = compare_bins(ib, torch.from_numpy(r['inv.bins']), layer, y, True, latent)
         # forward re-search at the RECOVERED point (what the reference does for the inverse log-det): the
         # kernels' own recovered x vs the reference's recorded re-search at its recovered x
-        key = f'{name}|L{i}|inv.fbins'
-        if key in b:
+        if 'inv.fbins' in r:
             _, rb, _ = cuda_bins(mod, xc, lat_dev, _lib.FORWARD)
-            want = torch.from_numpy(b[key]).to(DEV)
+            rb = recorded(rb)
+            want = torch.from_numpy(r['inv.fbins']).to(DEV)
             same_pattern = torch.equal(rb < 0, want < 0)
             rec['refwd_flips'] = int((rb != want).sum()) if same_pattern else -1
             # the tensor-core kernels evaluate the inverse log-det in the bin the INVERSE search found instead of
             # re-searching (DESIGN 4.1): how often do the two differ?
             both = (ib >= 0) & (rb >= 0)
             rec['inv_vs_refwd'] = int(((ib != rb) & both).sum())
-            rec['inv_vs_refwd_ref'] = int(((torch.from_numpy(b[f'{name}|L{i}|inv.bins']).to(DEV) != want) & both).sum())
-        rows.append(rec)
-    return rows
+            rec['inv_vs_refwd_ref'] = int(((torch.from_numpy(r['inv.bins']).to(DEV) != want) & both).sum())
+        out.append(rec)
+    return out
 
 
 @pytest.mark.parametrize('name', cases.spline_cases())

