@@ -20,9 +20,7 @@ ACTIVATIONS = {None: 0, 'Identity': 0, 'Tanh': 1, 'ReLU': 2, 'Sigmoid': 3, 'ELU'
                'LeakyReLU': 6, 'SiLU': 7, 'GELU': 8}
 E_INVAL, E_CUDA, E_NOTSUP = -1, -2, -3
 
-# STRIBOR_B200_LIB: profiling builds of the same library (tools/build_variants.py); there is no other fallback
-LIB_PATH = os.environ.get('STRIBOR_B200_LIB') or \
-    os.path.join(os.path.dirname(os.path.abspath(__file__)), 'libstribor_b200.so')
+LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'libstribor_b200.so')
 
 EXPORTS = ['stb_abi_version', 'stb_sizeof_layer', 'stb_last_error', 'stb_layer_apply', 'stb_layer_apply_diag',
            'stb_layer_apply_bins', 'stb_flow_apply',

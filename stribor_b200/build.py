@@ -59,16 +59,14 @@ def _compile_one(nvcc, src, obj, flags):
     return src, ' '.join(cmd), r.returncode, r.stdout
 
 
-def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT) -> str:
-    """`defines` / `out`: profiling variants only (tools/build_variants.py); the product is the default."""
-    if not force and out == OUT and up_to_date():
+def build(force: bool = False, verbose: bool = False) -> str:
+    if not force and up_to_date():
         return OUT
     nvcc = os.environ.get('NVCC', 'nvcc')
-    flags = CC_FLAGS + [f'-D{d}' for d in defines]
-    tag = hashlib.sha1(' '.join(flags).encode()).hexdigest()[:8]
+    tag = hashlib.sha1(' '.join(CC_FLAGS).encode()).hexdigest()[:8]
     objdir = os.path.join(OBJ, tag)
     os.makedirs(objdir, exist_ok=True)
-    hdr = _digest(_headers(), ' '.join(flags))
+    hdr = _digest(_headers(), ' '.join(CC_FLAGS))
     jobs, objs = [], []
     for src in sources():
         base = os.path.splitext(os.path.basename(src))[0]
@@ -83,7 +81,7 @@ def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT
     failed = False
     if jobs:
         with cf.ThreadPoolExecutor(max_workers=min(len(jobs), os.cpu_count() or 4)) as ex:
-            futs = {ex.submit(_compile_one, nvcc, s, o, flags): (s, o, st, w) for s, o, st, w in jobs}
+            futs = {ex.submit(_compile_one, nvcc, s, o, CC_FLAGS): (s, o, st, w) for s, o, st, w in jobs}
             for fu in cf.as_completed(futs):
                 s, o, st, w = futs[fu]
                 src, cmd, rc, text = fu.result()
@@ -97,19 +95,19 @@ def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT
                         f.write(w)
     link_text = ''
     if not failed:
-        cmd = [nvcc] + ARCH_FLAGS + ['-shared', '-o', out] + objs + ['-lcuda']
+        cmd = [nvcc] + ARCH_FLAGS + ['-shared', '-o', OUT] + objs + ['-lcuda']
         r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
         link_text = ' '.join(cmd) + '\n' + r.stdout
         failed = r.returncode != 0
     text = '\n'.join(logs) + '\n' + link_text
-    log = os.path.join(HERE, 'build.log' if out == OUT else os.path.basename(out) + '.build.log')
+    log = os.path.join(HERE, 'build.log')
     with open(log, 'w') as f:
         f.write(text)
     if verbose or failed:
         print(text)
     if failed:
         raise RuntimeError(f'nvcc failed; see {log}')
-    return out
+    return OUT
 
 
 if __name__ == '__main__':

@@ -1,7 +1,6 @@
 // extern "C" surface of libstribor_b200.so (see include/stribor_b200.h).
 #include <stdarg.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include "common.cuh"
 
 namespace stb {
@@ -17,6 +16,17 @@ int set_error(int code, const char* fmt, ...) {
     return code;
 }
 void count_launch() { ++g_launches; }
+
+int sm_count() {
+    static thread_local int n_sm = 0;
+    if (n_sm == 0) {
+        int dev = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+        if (n_sm <= 0) n_sm = 148;
+    }
+    return n_sm;
+}
 
 static int apply_one(const stb_layer* L, int direction, const float* x, const float* latent,
                      const float* t, float* y, float* ldj, int ldj_mode, int base_lp, int64_t rows,
@@ -49,10 +59,6 @@ static int apply_one(const stb_layer* L, int direction, const float* x, const fl
     return generic_layer_apply(L, direction, x, latent, t, y, ldj, ldj_mode, base_lp, ldiag, rows, s, bins);
 }
 
-// A sequence of layers (already in application order).  Maximal runs of 2..8 packed spline couplings of the
-// 256-row tensor-core kernel with the same dim and kind go out as ONE launch each (tc_layer.cu, CHAIN: the
-// tile stays in shared memory between the layers); everything else layer by layer.
-// STRIBOR_B200_NO_CHAIN=1: one launch per layer, for comparison.
 // A run of layers that goes out as ONE chained launch: 2..8 packed couplings of one tensor-core family -- spline
 // couplings of the 256-row kernel (tc_layer.cu, CHAIN) or affine / continuous-affine couplings with small conditioners
 // (tc_mlp.cu, CHAIN) -- of the same dim, with any permutations (flows/permute.py) before, between or after them folded
@@ -133,18 +139,17 @@ static bool single_chain(const stb_layer* const* seq, int n, int direction) {
 }
 
 // A sequence of layers (already in application order).  Maximal chainable runs (ChainRun) go out as ONE launch each;
-// everything else layer by layer.  STRIBOR_B200_NO_CHAIN=1: one launch per layer, for comparison.
+// everything else layer by layer.
 static int apply_sequence(const stb_layer* const* seq, int n, int direction, const float* x, const float* latent,
                           const float* t, float* out, float* ldj, int ldj_mode, int base_lp_last, int64_t rows,
                           cudaStream_t s) {
-    static const bool chain_off = [] { const char* e = getenv("STRIBOR_B200_NO_CHAIN"); return e && e[0] == '1'; }();
     const float* cur = x;
     int mode = ldj_mode;
     int i = 0;
     while (i < n) {
         ChainRun run;
         bool chained = false;
-        if (!chain_off && rows > 0 && x && !(ldj_mode != STB_LDJ_NONE && !ldj))
+        if (rows > 0 && x && !(ldj_mode != STB_LDJ_NONE && !ldj))
             chained = scan_run(seq + i, n - i, direction, &run) && (out || (i == 0 && run.consumed == n));
         const int j = chained ? i + run.consumed : i + 1;
         const int last = (j == n);
@@ -217,8 +222,7 @@ int stb_flow_apply(const stb_layer* layers, int n_layers, int direction, const f
 }
 
 int stb_flow_log_prob_needs_x_out(const stb_layer* layers, int n_layers) {
-    static const bool chain_off = [] { const char* e = getenv("STRIBOR_B200_NO_CHAIN"); return e && e[0] == '1'; }();
-    if (chain_off || n_layers < 2 || n_layers > 8 || !layers) return 1;
+    if (n_layers < 2 || n_layers > 8 || !layers) return 1;
     const stb_layer* order[8];
     for (int i = 0; i < n_layers; ++i) order[i] = &layers[n_layers - 1 - i];
     return single_chain(order, n_layers, STB_INVERSE) ? 0 : 1;

@@ -1,5 +1,5 @@
 // Host-side plumbing shared by the translation units of libstribor_b200.so:
-// thread-local error text, launch counter, internal entry points.
+// thread-local error text, launch counter, SM count, internal entry points.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -9,6 +9,8 @@ namespace stb {
 
 int set_error(int code, const char* fmt, ...);
 void count_launch();
+// multiprocessors of the current device, looked up once per host thread (148, a B200's count, if the query fails)
+int sm_count();
 
 int validate_layer(const stb_layer* L);
 

@@ -147,27 +147,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
         : "memory");
 }
 
-// ---- thread-block clusters: one weight stream for several SMs ---------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// the same bytes land at the same shared-memory offset of every CTA in `cta_mask` and complete_tx on the mbarrier at the
-// same offset there (TMA multicast): a weight block is read from L2 once per cluster
-__device__ __forceinline__ void bulk_g2s_multicast(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar,
-                                                   uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)), "h"(cta_mask)
-        : "memory");
-}
-
 // ---- TMEM ------------------------------------------------------------------------------------------
 // one full warp; writes the TMEM base address to *dst (shared memory)
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst, uint32_t ncols) {
@@ -277,15 +256,6 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(
                      smem_u32(bar))
-                 : "memory");
-}
-
-// ... on the mbarrier at this offset in EVERY CTA of `cta_mask` (a stage shared through multicast is free once all
-// consumers of the cluster are done with it)
-__device__ __forceinline__ void umma_commit_multicast(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                     smem_u32(bar)),
-                 "h"(cta_mask)
                  : "memory");
 }
 

@@ -22,7 +22,6 @@
 //
 // Reference semantics restated here: flows/coupling.py:53-95, flows/spline.py:76-105, net/mlp.py:46-58,
 // util/rational_quadratic_spline.py, util/cubic_spline.py, flow.py:42-47.
-#include <stdlib.h>
 #include "common.cuh"
 #include "stb_math.cuh"
 #include "tc_common.cuh"
@@ -111,7 +110,6 @@ struct Args {
     float lower, upper;
     long long rows;
     int n_tiles;
-    int cluster;             // CTAs per cluster (1, 2 or 4) sharing every weight item through TMA multicast
 };
 
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
@@ -172,8 +170,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
 
     if (tid == 0) {
         mbar_init(&bars->setup, 1);
-        // a stage is shared by the cluster: every CTA's issuer releases it in every CTA (multicast commit)
-        for (int i = 0; i < kStages; ++i) { mbar_init(&bars->b_full[i], 1); mbar_init(&bars->b_empty[i], (uint32_t)A.cluster); }
+        for (int i = 0; i < kStages; ++i) { mbar_init(&bars->b_full[i], 1); mbar_init(&bars->b_empty[i], 1); }
         mbar_init(&bars->a1_ready, kEpiWarps);
         mbar_init(&bars->acc1_full, 1);
         mbar_init(&bars->h1_ready, kEpiWarps);
@@ -186,10 +183,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    const int CL = A.cluster;
-    const uint32_t crank = (CL > 1) ? cluster_ctarank() : 0u;
-    const uint16_t cmask = (uint16_t)((1u << CL) - 1u);
-    if (CL > 1) cluster_sync_all();               // every CTA's mbarriers exist before a peer multicasts into them
     const uint32_t tmem = tmem_base_s;
     if (tid == 0) {
         mbar_arrive_expect_tx(&bars->setup, kSmallBytes);
@@ -205,14 +198,11 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
     const uint32_t col_h_last = (n_hidden == 2) ? 256u : 0u;                // A operand of the chunk GEMMs
     const uint32_t col_chunk = (n_hidden == 2) ? 0u : (uint32_t)H;          // two 96-column accumulators
     const int n_chunks = (n_tr + 1) / 2;
-    // every CTA of a cluster runs the same number of tiles (the weight stream is shared): the trip count is that of the
-    // cluster's FIRST CTA; a CTA whose last tile does not exist runs it as a ghost (no rows loaded, nothing stored)
-    const int first_cta = (int)blockIdx.x - (int)crank;
-    const int my_tiles = (A.n_tiles > first_cta) ? (A.n_tiles - 1 - first_cta) / (int)gridDim.x + 1 : 0;
+    const int my_tiles = (A.n_tiles > (int)blockIdx.x) ? (A.n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
 
     // ---- one chunk = TWO transformed dims: [128 x H] x [H x 96] into accumulator buffer `buf`, A = the last hidden layer
-    // in TMEM.  The chunk UMMAs cost a fixed ~38 clocks each whatever N (measured: N = 16 and N = 48 take the same time,
-    // -DSTB_HW_EXP), so two dims per UMMA halve the chunk phase's tensor time.  A chunk's weights travel as two ring
+    // in TMEM.  The chunk UMMAs cost a fixed ~38 clocks each whatever N (measured: N = 16 and N = 48 take the same
+    // time), so two dims per UMMA halve the chunk phase's tensor time.  A chunk's weights travel as two ring
     // items -- the fp16 lo parts, then the hi parts, each [96 x H] K-major in K blocks of 16 -- and the three passes
     // go hi*lo (item 0, released), then lo*hi and hi*hi (item 1): corrections first, the accumulator truncates.
     // Every mbarrier of the chunk phase is a PRIVATE channel, so that a waiter's successive waits are successive phases
@@ -220,10 +210,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
     // buffer b is written by issuer b only and read by epilogue groups 2b, 2b + 1 only; a ring stage is refilled only
     // after the issuer that consumed its previous item has released it.
     auto issue_chunk = [&](uint32_t rc, uint32_t buf, uint32_t buse) {
-#ifndef STB_HW_EXP
-#define STB_HW_EXP 0                       // timing experiments only (wrong results): 1 no chunk UMMAs, 2 chunk UMMAs with N = 16
-#endif
-        const uint32_t idesc3 = make_idesc(FMT_F16, 128, (STB_HW_EXP & 2) ? 16 : kChunkN);
+        const uint32_t idesc3 = make_idesc(FMT_F16, 128, kChunkN);
         const uint32_t dcol = tmem + col_chunk + buf * kChunkN;
         const uint32_t ad0 = tmem + col_h_last;
         uint32_t acc = 0;
@@ -241,14 +228,14 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
                 uint32_t ad = ad0 + ((p == 1) ? 8u : 0u);
 #pragma unroll 4
                 for (int kb = 0; kb < kb_h; ++kb) {
-                    if (!(STB_HW_EXP & 1)) umma_f16_ts(dcol, ad, bd, idesc3, acc);
+                    umma_f16_ts(dcol, ad, bd, idesc3, acc);
                     acc = 1;
                     bd += (uint64_t)(w3_block() >> 4);
                     ad += 16u;
                 }
             }
             if (item == 1) umma_commit(&bars->acc_full[buf]);
-            if (CL > 1) umma_commit_multicast(&bars->b_empty[st], cmask); else umma_commit(&bars->b_empty[st]);
+            umma_commit(&bars->b_empty[st]);
         }
     };
 
@@ -260,18 +247,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
                 const uint32_t st = rc % kStages, use = rc / kStages;
                 mbar_wait_relaxed(&bars->b_empty[st], (use & 1) ^ 1);
                 mbar_arrive_expect_tx(&bars->b_full[st], bytes);
-                if (CL == 1) {
-                    bulk_g2s(ring + st * stage, src, bytes, &bars->b_full[st]);
-                } else {                                   // this CTA fetches its 1 / CL of the item for the whole cluster
-                    const uint32_t part = bytes / (uint32_t)CL;
-                    bulk_g2s_multicast(ring + st * stage + crank * part, src + crank * part, part, &bars->b_full[st], cmask);
-                }
+                bulk_g2s(ring + st * stage, src, bytes, &bars->b_full[st]);
                 ++rc;
             };
             for (int it = 0; it < my_tiles; ++it) {
                 if (it + 1 < my_tiles) {
                     const long long nrow0 = ((long long)blockIdx.x + (long long)(it + 1) * gridDim.x) * kRows;
-                    const long long nb = max(0LL, min((long long)kRows, A.rows - nrow0)) * d * 4;
+                    const long long nb = min((long long)kRows, A.rows - nrow0) * d * 4;
                     const char* src = reinterpret_cast<const char*>(A.x + nrow0 * d);
                     if (nb >= 16 && ((reinterpret_cast<uintptr_t>(src) & 15) == 0))
                         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"((uint32_t)(nb & ~15LL)) : "memory");
@@ -314,7 +296,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
                         }
                     }
                     umma_commit(&bars->acc1_full);
-                    if (CL > 1) umma_commit_multicast(&bars->b_empty[st], cmask); else umma_commit(&bars->b_empty[st]);
+                    umma_commit(&bars->b_empty[st]);
                     ++rc;
                 }
                 if (n_hidden == 2) {   // ---- GEMM2': A = h1 from TMEM, per K block lo*hi, hi*lo, hi*hi ---------------------
@@ -334,7 +316,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
                             umma_f16_ts(tmem + 256, a_hi, b_lo, idesc2, 1);
                             umma_f16_ts(tmem + 256, a_hi, b_hi, idesc2, 1);
                         }
-                        if (CL > 1) umma_commit_multicast(&bars->b_empty[st], cmask); else umma_commit(&bars->b_empty[st]);
+                        umma_commit(&bars->b_empty[st]);
                     }
                     umma_commit(&bars->acc2_full);
                 }
@@ -378,7 +360,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
 
         for (int it = 0; it < my_tiles; ++it, tp ^= 1) {
             const long long row0 = ((long long)blockIdx.x + (long long)it * gridDim.x) * kRows;
-            const int nrows = (int)max(0LL, min((long long)kRows, A.rows - row0));      // 0: ghost tile
+            const int nrows = (int)min((long long)kRows, A.rows - row0);
             {   // ---- stage the x tile ------------------------------------------------------------------------------------
                 const float* xg = A.x + row0 * d;
                 const int n = nrows * d;
@@ -547,7 +529,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
     }
     tc_fence_before();
     __syncthreads();
-    if (CL > 1) cluster_sync_all();               // no CTA leaves while a peer may still multicast into it
     if (warp == 1) tmem_dealloc(tmem, 512);
 }
 
@@ -774,13 +755,6 @@ int tch_layer_apply(const stb_layer* L, int direction, const float* x, const flo
     const long long tiles = (rows + kRows - 1) / kRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
     const bool inv = direction == STB_INVERSE;
     void (*kern)(Args);
     if (L->n_bins == kBins) {
@@ -793,45 +767,11 @@ int tch_layer_apply(const stb_layer* L, int direction, const float* x, const flo
     const uint32_t smem = smem_bytes(H);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    // Clusters of CTAs can share the weight stream (1.85 MB per 128-row tile at MLP[256,256]) through TMA multicast:
-    // STRIBOR_B200_HW_CLUSTER = 2 | 4.  Measured at MLP[256,256] (1 M rows, 8 layers): 22.2 ms without clusters,
-    // 23.0 ms with pairs, 24.4 ms with quads (fewer resident CTAs) -- L2 delivers the stream, the default stays 1.
-    static const int want_cluster = [] {
-        const char* ev = getenv("STRIBOR_B200_HW_CLUSTER");
-        const int v = ev ? atoi(ev) : 1;               // measured: 1 is fastest (the stream is not what binds)
-        return (v == 1 || v == 2 || v == 4) ? v : 1;
-    }();
-    int cl = want_cluster;
-    while (cl > 1 && (tiles < cl || (n_sm % cl) != 0)) cl >>= 1;
-    A.cluster = cl;
-    int grid = (int)min((long long)n_sm, tiles);
-    grid -= grid % cl;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)cl;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    if (cl > 1) {
-        // persistent kernel: every cluster must be resident at once (GPC sizes are not all multiples of the cluster size)
-        int max_clusters = 0;
-        e = cudaOccupancyMaxActiveClusters(&max_clusters, kern, &cfg);
-        if (e == cudaSuccess && max_clusters > 0 && max_clusters * cl < grid) {
-            grid = max_clusters * cl;
-            cfg.gridDim = dim3((unsigned)grid);
-        } else if (e != cudaSuccess) {
-            (void)cudaGetLastError();
-        }
-    }
-    e = cudaLaunchKernelEx(&cfg, kern, A);
+    // one CTA per SM, each streaming its own weights: clusters of CTAs sharing one weight stream measured slower
+    // (DESIGN.md 4.1f)
+    const int grid = (int)min((long long)sm_count(), tiles);
+    kern<<<grid, kThreads, smem, stream>>>(A);
     count_launch();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_hw_spline_kernel launch: %s", cudaGetErrorString(e));
     e = cudaGetLastError();
     if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_hw_spline_kernel launch: %s", cudaGetErrorString(e));
     return STB_OK;

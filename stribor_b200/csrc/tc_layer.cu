@@ -27,7 +27,6 @@
 //
 // Reference semantics restated here: flows/coupling.py:53-95, flows/spline.py:76-105,
 // util/rational_quadratic_spline.py, util/cubic_spline.py, net/mlp.py:46-58, flow.py:42-47.
-#include <stdlib.h>
 #include "common.cuh"
 #include "stb_math.cuh"
 #include "tc_common.cuh"
@@ -51,42 +50,7 @@ constexpr int kTileRows = 256;
 constexpr int kXsStride = kMaxDim + 1;
 constexpr int kStages = 3;
 constexpr int kMaxChain = 8;           // layers of a flow fused into one launch (CHAIN kernels)
-#ifndef STB_TC_EPI_PER_SUB
-#define STB_TC_EPI_PER_SUB 2
-#endif
-#if STB_TC_EXP & 64
-#define MBAR_WAIT_SLOW mbar_wait
-#else
-#define MBAR_WAIT_SLOW mbar_wait_relaxed
-#endif
-// bit 128: per-warp phase clocks (tools/tc_phase_prof.py reads them back through stb_tc_prof_read)
-#if STB_TC_EXP & 128
-__device__ unsigned int g_tc_prof[160 * 32 * 8];
-#define PROF_DECL unsigned int _pt = clock(), _pa[6] = {0, 0, 0, 0, 0, 0};
-#define PROF(i) { const unsigned int _n = clock(); _pa[i] += _n - _pt; _pt = _n; }
-#if STB_TC_EXP & 256
-#define PROFH(i) PROF(i)
-#define PROFC(i)
-#else
-#define PROFH(i)
-#define PROFC(i) PROF(i)
-#endif
-#define PROF_FLUSH { if ((threadIdx.x & 31) == 0) for (int _i = 0; _i < 6; ++_i) g_tc_prof[(blockIdx.x * 32 + (threadIdx.x >> 5)) * 8 + _i] = _pa[_i]; }
-#else
-#define PROF_DECL
-#define PROF(i)
-#define PROFH(i)
-#define PROFC(i)
-#define PROF_FLUSH
-#endif
-// -DSTB_PLAIN_ARRIVE: release the accumulator buffers through the generic-address helper instead of the pre-converted
-// shared address (tool experiments only: compute-sanitizer synccheck, see profiles/r02_synccheck.txt)
-#ifdef STB_PLAIN_ARRIVE
-#define STB_ARRIVE_EMPTY(buf) mbar_arrive(&bars->acc_empty[s][buf])
-#else
-#define STB_ARRIVE_EMPTY(buf) mbar_arrive_a(empty_bar + (buf) * 8)
-#endif
-constexpr int kEpiPerSub = STB_TC_EPI_PER_SUB;   // epilogue warps per (subtile, TMEM sub-partition)
+constexpr int kEpiPerSub = 2;          // epilogue warps per (subtile, TMEM sub-partition)
 constexpr int kEpiWarps = 2 * 4 * kEpiPerSub;
 constexpr int kEpiWarp0 = 3;           // warp 0 producer, warps 1 / 2 UMMA issuers of subtile 0 / 1
 constexpr int kThreads = (kEpiWarp0 + kEpiWarps) * 32;
@@ -255,14 +219,14 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                     const int nch = CHAIN ? A.n_chunks_l[l] : n_chunks;
                     if (CHAIN) {                   // the layer's head: header | biases | first Linear
                         const uint32_t st = cc % kStages, use = cc / kStages;
-                        MBAR_WAIT_SLOW(&bars->b_empty[st], (use & 1) ^ 1);
+                        mbar_wait_relaxed(&bars->b_empty[st], (use & 1) ^ 1);
                         mbar_arrive_expect_tx(&bars->b_full[st], kHeadBytes);
                         bulk_g2s(bst + st * kChunkBytes, img, kHeadBytes, &bars->b_full[st]);
                         ++cc;
                     }
                     for (int c = 0; c < nch; ++c, ++cc) {
                         const uint32_t st = cc % kStages, use = cc / kStages;
-                        MBAR_WAIT_SLOW(&bars->b_empty[st], (use & 1) ^ 1);
+                        mbar_wait_relaxed(&bars->b_empty[st], (use & 1) ^ 1);
                         mbar_arrive_expect_tx(&bars->b_full[st], kChunkBytes);
                         bulk_g2s(bst + st * kChunkBytes, img + kOffW2 + (size_t)c * kChunkBytes, kChunkBytes,
                                  &bars->b_full[st]);
@@ -282,7 +246,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
             uint32_t cc = 0;                       // chunk counter (accumulator buffers)
             uint32_t rc = 0;                       // ring item counter (== cc unless CHAIN adds the layer heads)
             uint32_t hp = 0;                       // layer applications so far (phase of the head barriers)
-            PROF_DECL
             for (int it = 0; it < my_tiles; ++it)
             for (int l = 0; l < n_layers; ++l, ++hp) {
                 const uint32_t tpar = hp & 1;
@@ -291,11 +254,10 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                     uint32_t b0 = smem_u32(w1s);
                     const uint32_t hst = rc % kStages;
                     if (CHAIN) {
-                        MBAR_WAIT_SLOW(&bars->b_full[hst], (rc / kStages) & 1);
+                        mbar_wait_relaxed(&bars->b_full[hst], (rc / kStages) & 1);
                         b0 = smem_u32(bst + hst * kChunkBytes) + kOffW1;
                     }
-                    MBAR_WAIT_SLOW(&bars->a1_ready[s], tpar);
-                    PROF(0)
+                    mbar_wait_relaxed(&bars->a1_ready[s], tpar);
                     tc_fence_after();
                     const uint32_t a0 = smem_u32(abuf + s * kABytes);
                     const uint32_t dcol = tmem + kColAcc1 + s * kHid;
@@ -317,16 +279,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                     }
                     umma_commit(&bars->acc1_full[s]);
                     if (CHAIN) { umma_commit(&bars->b_empty[hst]); ++rc; }
-                    PROF(1)
                 }
                 for (int c = 0; c < nch; ++c, ++cc, ++rc) {
                     const uint32_t st = rc % kStages, use = rc / kStages;
-                    MBAR_WAIT_SLOW(&bars->b_full[st], use & 1);
-                    PROF(2)
+                    mbar_wait_relaxed(&bars->b_full[st], use & 1);
                     const uint32_t buf = cc & 1, buse = cc >> 1;
-                    if (c == 0) { MBAR_WAIT_SLOW(&bars->h_ready[s], tpar); PROF(3) }
-                    MBAR_WAIT_SLOW(&bars->acc_empty[s][buf], (buse & 1) ^ 1);
-                    PROF(4)
+                    if (c == 0) mbar_wait_relaxed(&bars->h_ready[s], tpar);
+                    mbar_wait_relaxed(&bars->acc_empty[s][buf], (buse & 1) ^ 1);
                     tc_fence_after();
                     const uint32_t a_hi = smem_u32(abuf + s * kABytes), a_lo = a_hi + 16384;
                     const uint32_t b_hi = smem_u32(bst + st * kChunkBytes), b_lo = b_hi + 12288;
@@ -345,10 +304,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                     }
                     umma_commit(&bars->acc_full[s][buf]);
                     umma_commit(&bars->b_empty[st]);       // stage reusable once both subtiles' UMMAs retire (count 2)
-                    PROF(5)
                 }
             }
-            PROF_FLUSH
         }
     } else if (warp >= kEpiWarp0) {
         // ======================= epilogue warps ==================================================
@@ -377,7 +334,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
         const uint32_t xrow_a = pin(smem_u32(xrow));
         uint32_t noshift_mask = CHAIN ? 0u : hdr->noshift_mask;
         uint32_t cc = 0, rc = 0, hp = 0;           // chunk / ring item / layer application counters (as the issuers')
-        PROF_DECL
 
         for (int it = 0; it < my_tiles; ++it) {
             const long long tile = (long long)blockIdx.x + (long long)it * gridDim.x;
@@ -416,7 +372,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                 }
             }
             named_bar_sync(1, kEpiThreads);
-            PROFH(0)
             float ld_acc = 0.f;                    // running log|det J| of this thread's elements (all layers)
 #pragma unroll 1
             for (int l = 0; l < n_layers; ++l, ++hp) {
@@ -476,7 +431,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&bars->a1_ready[sp]);
             }
-            PROFH(1)
             // hidden layer: h = act(acc1 + b1) -> fp16 hi | lo A operand of GEMM2, 8 units at a time
 #pragma unroll 1
             for (int sp = 0; sp < 2; ++sp) {
@@ -509,7 +463,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
             }
 
             // ---- last Linear chunks out of TMEM + spline in registers: this warp's dim of each chunk ----
-            PROFC(0) PROFH(3)
             // dims round-robin over the triple.  A warp visits chunks in increasing order with gaps <= 2,
             // so the phase parity it waits for on an accumulator buffer is never ambiguous: the
             // buffer's previous use (two chunks earlier) completed before a chunk this warp has
@@ -526,9 +479,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                 asm volatile("ld.shared.f32 %0, [%1];" : "=f"(xv) : "r"(xrow_a + j4));
                 const bool inside = (ji < n_tr) && (xv >= lo) && (xv <= hi);
                 const float* bb = b2s + ji * kPPad;
-                PROFC(5)
-                if (!(STB_TC_EXP & 4)) mbar_wait_a(full_bar + buf * 8, buse & 1);
-                PROFC(1)
+                mbar_wait_a(full_bar + buf * 8, buse & 1);
                 tc_fence_after();
                 const uint32_t col0 = col_base + buf * kChunkN + (uint32_t)g * kPPad;
                 float out = xv, ld = 0.f;
@@ -545,24 +496,21 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                         // bias table holds b * log2(e) for those 32 columns
 #pragma unroll
                         for (int i = 0; i < kBins; ++i) t[i] = __ffma2_rn(t[i], f2(s2l), bb2[i]);
-                        if (STB_TC_EXP & 8) { loc.Ek = t[0]; loc.Ek1 = t[15]; loc.c = t[7]; loc.k = 3; }
-                        else loc = rqs16_locate<INVERSE>(t, shift, lo, inv_span, xv);
+                        loc = rqs16_locate<INVERSE>(t, shift, lo, inv_span, xv);
                     }
                     float dd[16];
                     tmem_ld16(col0 + 2 * kBins, dd);
                     tmem_ld_wait();
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) STB_ARRIVE_EMPTY(buf);     // TMEM buffer free again
-                    PROFC(2)
+                    if (lane == 0) mbar_arrive_a(empty_bar + buf * 8);     // TMEM buffer free again
                     if (inside) {
                         // derivative parameter AT knot i (1..15) is column 32 + i - 1; box ends are constants
                         float r0, r1;
                         pick_pair16(dd, loc.k, r0, r1);
                         const float u0 = (loc.k == 0) ? STB_RQS_EDGE_CONST : fmaf(r0, s2, bb[2 * kBins + loc.k - 1]);
                         const float u1 = (loc.k == kBins - 1) ? STB_RQS_EDGE_CONST : fmaf(r1, s2, bb[2 * kBins + loc.k]);
-                        if (STB_TC_EXP & 9) { out = xv + 1e-30f * (loc.Ek.x + loc.Ek1.y + loc.c.x + u0 + u1); ld = loc.Ek.y; }
-                        else rqs16_finish<INVERSE>(loc, u0, u1, lo, hi, want_ld, xv, out, ld);
+                        rqs16_finish<INVERSE>(loc, u0, u1, lo, hi, want_ld, xv, out, ld);
                     }
                     if (BINS && ji < n_tr && rt < nrows) A.bins[(row0 + rt) * d + (j4 >> 2)] = inside ? loc.k : -1;
                 } else {
@@ -583,7 +531,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                     tmem_ld_wait();
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) STB_ARRIVE_EMPTY(buf);
+                    if (lane == 0) mbar_arrive_a(empty_bar + buf * 8);
                     if (inside) {
                         const float ul = fmaf(dd[0], s2, bb[2 * kBins]), ur = fmaf(dd[1], s2, bb[2 * kBins + 1]);
                         cubic16_finish<INVERSE>(sel, ul, ur, lo, hi, want_ld, u, out, ld);
@@ -592,10 +540,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                 }
                 if (ji < n_tr) asm volatile("st.shared.f32 [%0], %1;" ::"r"(xrow_a + j4), "f"(out) : "memory");
                 ld_acc += ld;
-                PROFC(3)
             }
             cc += (uint32_t)n_chunks;
-            PROFH(5)
             // next layer of the chain: every warp's outputs are in the tile, nobody reads this layer's biases any more
             if (CHAIN && l + 1 < n_layers) named_bar_sync(1, kEpiThreads);
             }   // layers
@@ -641,9 +587,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
                 }
             }
             named_bar_sync(1, kEpiThreads);
-            PROFC(4) PROFH(4)
         }
-        PROF_FLUSH
     }
 
     // ---- teardown --------------------------------------------------------------------------------------
@@ -656,7 +600,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_spline_layer_kernel(const Args
 // the whole-flow kernel as TWO independent CTAs per SM: tc_spline_pair_kernel
 // -----------------------------------------------------------------------------------------------
 // Same layers, same arithmetic, same packed image and the same bits out as the CHAIN kernel above, reorganised around
-// what its phase clocks show (tools/tc_phase_prof.py, 8 layers): per 256-row tile and layer the 16 epilogue warps spend
+// what its per-warp phase clocks showed (8 layers): per 256-row tile and layer the 16 epilogue warps spend
 // 8.5 k of 46.8 k clocks in the layer HEAD (A1 split -> GEMM1 -> tanh -> first chunk) with the tensor pipe idle, and the
 // issuers 26 % of theirs waiting for accumulator buffers.  One CTA cannot overlap a layer's head with anything: the next
 // layer needs every output of this one.  Two CTAs per SM, each with its own 128-row tile, do -- their heads fall into
@@ -747,7 +691,7 @@ __global__ void __launch_bounds__(kPThreads, 2) tc_spline_pair_kernel(const Args
                     const int nch = A.n_chunks_l[l];
                     for (int c = -1; c < nch; ++c, ++rc) {
                         const uint32_t st = rc % kStages, use = rc / kStages;
-                        MBAR_WAIT_SLOW(&bars->b_empty[st], (use & 1) ^ 1);
+                        mbar_wait_relaxed(&bars->b_empty[st], (use & 1) ^ 1);
                         const uint32_t bytes = (c < 0) ? kHeadBytes : kChunkBytes;
                         mbar_arrive_expect_tx(&bars->b_full[st], bytes);
                         bulk_g2s(bst + st * kChunkBytes, (c < 0) ? img : img + kOffW2 + (size_t)c * kChunkBytes, bytes, &bars->b_full[st]);
@@ -767,9 +711,9 @@ __global__ void __launch_bounds__(kPThreads, 2) tc_spline_pair_kernel(const Args
                 const int nch = A.n_chunks_l[l];
                 {
                     const uint32_t hst = rc % kStages;
-                    MBAR_WAIT_SLOW(&bars->b_full[hst], (rc / kStages) & 1);
+                    mbar_wait_relaxed(&bars->b_full[hst], (rc / kStages) & 1);
                     const uint32_t b0 = smem_u32(bst + hst * kChunkBytes) + kOffW1;
-                    MBAR_WAIT_SLOW(&bars->a1_ready, tpar);
+                    mbar_wait_relaxed(&bars->a1_ready, tpar);
                     tc_fence_after();
                     uint32_t acc = 0;
                     // the same eight partial products in the same order as the kernel above (smallest first)
@@ -790,10 +734,10 @@ __global__ void __launch_bounds__(kPThreads, 2) tc_spline_pair_kernel(const Args
                 }
                 for (int c = 0; c < nch; ++c, ++cc, ++rc) {
                     const uint32_t st = rc % kStages, use = rc / kStages;
-                    MBAR_WAIT_SLOW(&bars->b_full[st], use & 1);
+                    mbar_wait_relaxed(&bars->b_full[st], use & 1);
                     const uint32_t buf = cc & 1, buse = cc >> 1;
-                    if (c == 0) MBAR_WAIT_SLOW(&bars->h_ready, tpar);
-                    MBAR_WAIT_SLOW(&bars->acc_empty[buf], (buse & 1) ^ 1);
+                    if (c == 0) mbar_wait_relaxed(&bars->h_ready, tpar);
+                    mbar_wait_relaxed(&bars->acc_empty[buf], (buse & 1) ^ 1);
                     tc_fence_after();
                     const uint32_t b_hi = smem_u32(bst + st * kChunkBytes), b_lo = b_hi + 12288;
                     const uint32_t dcol = tmem + kPColAcc + buf * kChunkN;
@@ -1214,12 +1158,6 @@ bool tc_layer_supported(const stb_layer* L) {
 
 uint64_t tc_packed_bytes(const stb_layer*) { return tcl::kPackedBytes; }
 
-#if STB_TC_EXP & 128
-extern "C" int stb_tc_prof_read(unsigned int* host, int n) {
-    return (int)cudaMemcpyFromSymbol(host, tcl::g_tc_prof, (size_t)n * 4);
-}
-#endif
-
 int tc_pack_layer(const stb_layer* L, void* out, cudaStream_t stream) {
     using namespace tcl;
     PackArgs a;
@@ -1239,17 +1177,6 @@ int tc_pack_layer(const stb_layer* L, void* out, cudaStream_t stream) {
 }
 
 namespace tcl {
-static int sm_count() {
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
-    return n_sm;
-}
-
 // the two-CTA whole-flow kernel over A.n_layers >= 1 layers (A.chain_packed / lower_l / upper_l / n_chunks_l filled)
 static int launch_pair(Args& A, int kind, bool full, int64_t rows, cudaStream_t stream) {
     void (*kern)(Args);
@@ -1309,13 +1236,6 @@ int tc_layer_apply(const stb_layer* L, int direction, const float* x, const floa
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
 
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
     void (*kern)(Args);
     if (L->kind == STB_RQS) kern = A.inverse ? tc_spline_layer_kernel<STB_RQS, true, false> : tc_spline_layer_kernel<STB_RQS, false, false>;
     else kern = A.inverse ? tc_spline_layer_kernel<STB_CUBIC, true, false> : tc_spline_layer_kernel<STB_CUBIC, false, false>;
@@ -1325,7 +1245,7 @@ int tc_layer_apply(const stb_layer* L, int direction, const float* x, const floa
     }
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
     if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    const int grid = (int)min((long long)n_sm, tiles);
+    const int grid = (int)min((long long)sm_count(), tiles);
     kern<<<grid, kThreads, kSmemBytes, stream>>>(A);
     count_launch();
     e = cudaGetLastError();
@@ -1376,23 +1296,16 @@ int tc_chain_apply(const stb_layer* const* layers, int n, int direction, const f
     const long long tiles = (rows + kTileRows - 1) / kTileRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
+    const int n_sm = sm_count();
     void (*kern)(Args);
     // Two independent 128-row CTAs per SM instead of one 256-row CTA.  Measured on the headline workload (2^22 rows):
     // 1.73e8 vs 1.77e8 samples/s -- the heads do fall into the other CTA's chunk phases, but the kernel is bound by
     // the epilogue's instruction stream, not by that bubble, so nothing is gained; it IS faster when there are fewer
     // 256-row tiles than SMs (twice as many CTAs to spread over the machine), which is when it is selected -- and it
-    // is the kernel of layers with fewer than 16 bins.  STRIBOR_B200_PAIR=1 / 0 forces / forbids it (16-bin flows).
-    static const int pair_env = [] { const char* ev = getenv("STRIBOR_B200_PAIR"); return (ev && ev[0]) ? (ev[0] == '1' ? 1 : 0) : -1; }();
+    // is the kernel of layers with fewer than 16 bins.
     bool full = true;
     for (int i = 0; i < n; ++i) full = full && layers[i]->n_bins == kBins;
-    const bool use_pair = !full || (pair_env >= 0 ? pair_env == 1 : tiles < (long long)n_sm);
+    const bool use_pair = !full || tiles < (long long)n_sm;
     if (use_pair) return launch_pair(A, layers[0]->kind, full, rows, stream);
     if (layers[0]->kind == STB_RQS) kern = A.inverse ? tc_spline_layer_kernel<STB_RQS, true, true> : tc_spline_layer_kernel<STB_RQS, false, true>;
     else kern = A.inverse ? tc_spline_layer_kernel<STB_CUBIC, true, true> : tc_spline_layer_kernel<STB_CUBIC, false, true>;

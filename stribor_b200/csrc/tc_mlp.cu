@@ -27,7 +27,6 @@
 // tc_mlp_chain4_kernel (a whole affine / continuous-affine flow in one launch, weights resident in shared memory).
 //
 // Reference semantics: flows/coupling.py:53-95, flows/affine.py:59-109, net/mlp.py:46-58.
-#include <stdlib.h>
 #include "common.cuh"
 #include "stb_math.cuh"
 #include "tc_common.cuh"
@@ -545,21 +544,7 @@ __global__ void __launch_bounds__(Cfg<NCG>::kThreads, (NCG == 4) ? 1 : 2) tc_mlp
 //     last K blocks drain, its A1 operand is split while GEMM3's drain, and its GEMM1 runs under tile i's affine
 //     output / store phase (the issuer only waits until the output accumulator has been read: d3_read).
 // Weights stream one 16-wide K block per ring item (<= 16 KB), in the order the issuer consumes them.
-// per-warp phase clocks of the chain and pipe kernels (profiling builds: -DSTB_TCM_PROF, tools/tcm_phase_prof.py)
-#ifdef STB_TCM_PROF
-__device__ unsigned int g_tcm_prof[160 * 32 * 8];
-#define TPROF_DECL unsigned int _pt = clock(), _pa[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#define TPROF(i) { const unsigned int _n = clock(); _pa[i] += _n - _pt; _pt = _n; }
-#define TPROF_FLUSH { if ((threadIdx.x & 31) == 0) for (int _i = 0; _i < 8; ++_i) g_tcm_prof[(blockIdx.x * 32 + (threadIdx.x >> 5)) * 8 + _i] = _pa[_i]; }
-#else
-#define TPROF_DECL
-#define TPROF(i)
-#define TPROF_FLUSH
-#endif
-#ifndef STB_PIPE_STAGES
-#define STB_PIPE_STAGES 6
-#endif
-constexpr int kPipeStages = STB_PIPE_STAGES;
+constexpr int kPipeStages = 6;
 constexpr int kPipeThreads = (2 + 16) * 32;
 
 struct PipeBars {
@@ -686,13 +671,11 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
             const uint32_t a0 = smem_u32(a1buf);
             constexpr uint32_t a_part = (uint32_t)kRows * kK1 * 2;
             uint32_t rc = 0, tp = 0;
-            TPROF_DECL
             for (int it = 0; it < my_tiles; ++it, tp ^= 1) {
                 // ---- layer 1: bf16x3 x bf16x3 into one accumulator, blocks (pb = 2, 1, 0) x (kb = 0, 1) as they arrive ----
                 mbar_wait_relaxed(&bars->a1_ready, tp);
                 if (it > 0) mbar_wait_relaxed(&bars->d3_read, tp ^ 1);      // tile it-1's output accumulator has been read
                 tc_fence_after();
-                TPROF(0)
                 uint32_t acc = 0;
                 for (int b = 0; b < 6; ++b, ++rc) {
                     const int pb = 2 - b / 2, kb = b & 1;
@@ -708,7 +691,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
                     umma_commit(&bars->empty[st]);
                 }
                 umma_commit(&bars->acc1_full);
-                TPROF(1)
                 // ---- hidden -> hidden (optional) and hidden -> output, four K blocks per activation wave --------------------
                 for (int layer = (n_hidden == 2 ? 0 : 1); layer < 2; ++layer) {
                     const bool last = (layer == 1);
@@ -720,12 +702,10 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
                     acc = 0;
                     for (int j = 0; j < nw; ++j) {
                         mbar_wait_relaxed(&wave[j], tp);
-                        TPROF(2 + 3 * layer)
                         for (int g = 0; g < 4; ++g, ++rc) {
                             const int kb = g * nw + j;
                             const uint32_t st = rc % kPipeStages, use = rc / kPipeStages;
                             mbar_wait_relaxed(&bars->full[st], use & 1);
-                            TPROF(3 + 3 * layer)
                             tc_fence_after();
                             const uint32_t bb = smem_u32(ring + st * slot);
                             const uint64_t b_hi = make_smem_desc(bb, 128, 256), b_lo = make_smem_desc(bb + lo_off, 128, 256);
@@ -734,13 +714,11 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
                             umma_f16_ts(dcol, a_hi, b_lo, idesc, 1);
                             umma_f16_ts(dcol, a_hi, b_hi, idesc, 1);
                             umma_commit(&bars->empty[st]);
-                            TPROF(4 + 3 * layer)
                         }
                     }
                     umma_commit(last ? &bars->acc3_full : &bars->acc2_full);
                 }
             }
-            TPROF_FLUSH
         }
     } else {
         // ======================= epilogue warps ===========================================================================
@@ -754,7 +732,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
         const float s_mid = hdr->s_mid, s_out = hdr->s_out;
         const int dshift = ((d & (d - 1)) == 0) ? (31 - __clz(d)) : -1;
         uint32_t tp = 0;
-        TPROF_DECL
 
         // rows of tile `it` -> xs buffer it & 1 (zero rows past the end), t likewise
         auto stage_x = [&](int it) {
@@ -808,7 +785,6 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
             stage_x(0);
             split_a1(0);       // the A1 buffer is free: nothing has been issued yet
         }
-        TPROF(0)
         for (int it = 0; it < my_tiles; ++it, tp ^= 1) {
             const long long row0 = ((long long)blockIdx.x + (long long)it * gridDim.x) * kRows;
             const int nrows = (int)min((long long)kRows, A.rows - row0);
@@ -817,36 +793,27 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
             // ---- hidden layer 1 in place, wave by wave: the next GEMM runs behind ---------------------------------------------
             mbar_wait_sleep(&bars->acc1_full, tp, 32);       // GEMM1(it) done: the A1 buffer is free as well
             tc_fence_after();
-            TPROF(2)
             for (int j = 0; j < nw; ++j) {
                 pipe_activate16(tmem + lane_sel, g * cq + 16 * j, 1.f, b1s, act);
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&bars->wave1[j]);
             }
-            TPROF(3)
-            if (more) {                                      // while the next GEMM's last K blocks drain
-                stage_x(it + 1);
-                TPROF(0)
-            }
+            if (more) stage_x(it + 1);                       // while the next GEMM's last K blocks drain
             if (n_hidden == 2) {
                 mbar_wait_sleep(&bars->acc2_full, tp, 32);
                 tc_fence_after();
-                TPROF(4)
                 for (int j = 0; j < nw; ++j) {
                     pipe_activate16(tmem + lane_sel + 256, g * cq + 16 * j, s_mid, b2s, act);
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&bars->wave2[j]);
                 }
-                TPROF(5)
             }
             if (more) split_a1(it + 1);                      // the A1 buffer is free since acc1_full; GEMM3's last blocks drain
-            TPROF(1)
             // ---- output layer: [log_scale | shift] of this warp's 8 transformed dims (one accumulator) ------------------
             mbar_wait_sleep(&bars->acc3_full, tp, 32);
             tc_fence_after();
-            TPROF(6)
             float ld_acc = 0.f;
             {
                 float lm[8], sm[8];
@@ -909,9 +876,7 @@ __global__ void __launch_bounds__(kPipeThreads, 1) tc_mlp_pipe_kernel(const Args
                 }
             }
             named_bar_sync(1, kEpiThreads);      // ld_s, and this xs buffer (staged again two tiles on), are free
-            TPROF(7)
         }
-        TPROF_FLUSH
     }
     tc_fence_before();
     __syncthreads();
@@ -1044,7 +1009,6 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
             const uint32_t dmain = tmem, dcorr = tmem + H;
             uint32_t ause = 0;
             tc_fence_after();
-            TPROF_DECL
             for (int it = 0; it < my_tiles; ++it)
             for (int l = 0; l < L; ++l) {
                 const Header* hdr = reinterpret_cast<const Header*>(smem + (uint32_t)l * kSmallSlot);
@@ -1052,7 +1016,6 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                 const int k1b = (hdr->n_cond + (hdr->time_col >= 0 ? 1 : 0) <= 16) ? 1 : 2;   // K blocks of layer 1 in use
                 uint32_t roff = smem_u32(smem + A.sm_w + A.w_off[l]);
                 mbar_wait(&bars->a_ready, ause & 1); ++ause;
-                TPROF(0)
                 tc_fence_after();
                 uint32_t acc_m = 0, acc_c = 0;
                 for (int b = 0; b < 6; ++b, roff += w1b) {
@@ -1067,10 +1030,8 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                     }
                 }
                 umma_commit(&bars->acc_ready);
-                TPROF(1)
                 for (int layer = (n_hidden == 2 ? 0 : 1); layer < 2; ++layer) {
                     mbar_wait(&bars->a_ready, ause & 1); ++ause;
-                    TPROF(2)
                     tc_fence_after();
                     const bool last = (layer == 1);
                     const uint32_t idesc = last ? idesc3 : idesc2;
@@ -1086,10 +1047,8 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                         umma_f16(dmain, a_hi, b_hi, idesc, acc_m); acc_m = 1;
                     }
                     umma_commit(&bars->acc_ready);
-                    TPROF(3)
                 }
             }
-            TPROF_FLUSH
         }
     } else if (warp < kEpiWarp0 + NCG * 4) {
         // ---- epilogue warps of this virtual CTA ------------------------------------------------------------
@@ -1103,7 +1062,6 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
         const bool inverse = A.inverse != 0;
         const int bar_id = 1 + vc;
         uint32_t acc_use = 0;
-        TPROF_DECL
 
         for (int it = 0; it < my_tiles; ++it) {
             const long long row0 = ((long long)my_vcta + (long long)it * n_vcta) * kRows;
@@ -1140,7 +1098,6 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                 if (etid < kRows) t_s[etid] = (A.t != nullptr && etid < nrows) ? __ldg(A.t + row0 + etid) : 0.f;
             }
             named_bar_sync(bar_id, kEpiThreads);
-            TPROF(0)
             float ld_acc = 0.f;
 #pragma unroll 1
             for (int l = 0; l < L; ++l) {
@@ -1170,11 +1127,9 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                 fence_proxy_async_smem();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&bars->a_ready);
-                TPROF(1)
                 // ---- hidden layers ------------------------------------------------------------------------
                 for (int layer = 0; layer < n_hidden; ++layer) {
                     mbar_wait_sleep(&bars->acc_ready, acc_use & 1, 32); ++acc_use;
-                    TPROF(2)
                     tc_fence_after();
                     const float sc = (layer == 0) ? 1.f : hdr->s_mid;
                     const float* bias = (layer == 0) ? b1s : b2s;
@@ -1214,11 +1169,9 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                     fence_proxy_async_smem();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&bars->a_ready);
-                    TPROF(3)
                 }
                 // ---- output layer: affine transform of this warp's transformed dims ---------------------------
                 mbar_wait_sleep(&bars->acc_ready, acc_use & 1, 32); ++acc_use;
-                TPROF(4)
                 tc_fence_after();
                 const float s_out = hdr->s_out;
                 const bool cont = hdr->cont != 0;
@@ -1249,10 +1202,8 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                     }
                 }
                 tc_fence_before();
-                TPROF(5)
                 // the next layer gathers columns other warps have just written (and reuses the accumulators)
                 named_bar_sync(bar_id, kEpiThreads);
-                TPROF(6)
             }   // layers
 
             ld_s[cg * kRows + row] = ld_acc;
@@ -1290,9 +1241,7 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
                 }
             }
             named_bar_sync(bar_id, kEpiThreads);
-            TPROF(7)
         }
-        TPROF_FLUSH
     }
     tc_fence_before();
     __syncthreads();
@@ -1503,20 +1452,12 @@ int tcm_layer_apply(const stb_layer* L, int direction, const float* x, const flo
     const long long tiles = (rows + kRows - 1) / kRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
+    const int n_sm = sm_count();
     // small conditioner on few dims (configs[3]): the 8-warp configuration, two CTAs per SM
     const uint32_t w_total = 6 * w1_block_bytes(H) + (L->net.n_linear == 3 ? (H / 16) * w2_block_bytes(H) : 0) + (H / 16) * w3_block_bytes();
     const bool small = (H == 64) && (L->dim <= 32) && (w_total <= kStages * kSlotBytes) && (tiles >= 2LL * n_sm);
-    // wide conditioners: the pipelined kernel (TMEM-resident activations, GEMMs behind the activation waves);
-    // STRIBOR_B200_NO_MLP_PIPE=1 restores the phase-by-phase kernel
-    static const bool pipe_off = [] { const char* ev = getenv("STRIBOR_B200_NO_MLP_PIPE"); return ev && ev[0] == '1'; }();
-    if (!small && !pipe_off && H >= 128) {
+    // wide conditioners: the pipelined kernel (TMEM-resident activations, GEMMs behind the activation waves)
+    if (!small && H >= 128) {
         const uint32_t psmem = pipe_smem_bytes(H);
         cudaError_t pe = cudaFuncSetAttribute(tc_mlp_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem);
         if (pe != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(pe));
@@ -1839,12 +1780,6 @@ __global__ void __launch_bounds__(kV4Threads, 1) tc_mlp_chain4_kernel(const Chai
 
 }  // namespace tcm
 
-#ifdef STB_TCM_PROF
-extern "C" int stb_tcm_prof_read(unsigned int* host, int n) {
-    return (int)cudaMemcpyFromSymbol(host, tcm::g_tcm_prof, (size_t)n * 4);
-}
-#endif
-
 // ---- a run of affine / continuous-affine couplings of one flow in ONE launch ---------------------------------
 namespace tcm {
 static uint32_t layer_w_total(const stb_layer* L) {
@@ -1880,8 +1815,7 @@ static bool chain_layout(const stb_layer* const* layers, int n, ChainArgs* A, ui
 namespace tcm {
 // four-tiles-in-flight variant: one hidden layer, <= 16 conditioner inputs (incl. t) and <= 16 transformed dims per layer
 static bool chain4_layout(const stb_layer* const* layers, int n, ChainArgs* A, uint32_t* smem_bytes) {
-    static const bool off = [] { const char* e = getenv("STRIBOR_B200_NO_CHAIN4"); return e && e[0] == '1'; }();
-    if (off || n < 2 || n > kMaxChainM) return false;
+    if (n < 2 || n > kMaxChainM) return false;
     const int d = layers[0]->dim;
     for (int i = 0; i < n; ++i) {
         const stb_layer* L = layers[i];
@@ -1930,18 +1864,11 @@ int tcm_chain_apply(const stb_layer* const* layers, int n, int direction, const 
     const long long tiles = (rows + kRows - 1) / kRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
     void (*kern)(ChainArgs) = four ? tc_mlp_chain4_kernel<0> : tc_mlp_chain_kernel<kChainV>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     const int vper = four ? kV4 : kChainV;
-    const int grid = (int)min((long long)n_sm, (tiles + vper - 1) / vper);
+    const int grid = (int)min((long long)sm_count(), (tiles + vper - 1) / vper);
     kern<<<grid, four ? kV4Threads : kChainV * kVcThreads, smem, stream>>>(A);
     count_launch();
     e = cudaGetLastError();

@@ -608,9 +608,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc_wide_kernel(const Args A) {
 namespace train {
 constexpr int kTEpiWarp0 = 3;                                     // warp 0 producer, warps 1 / 2 UMMA issuers (F / G)
 constexpr int kTThreads = (kTEpiWarp0 + kEpiWarps) * 32;          // 608
-#ifndef STB_TRAIN_EXP
-#define STB_TRAIN_EXP 0     // profiling builds only: 1 no gW2 atomics, 2 no element gradient, 4 no G products
-#endif
 constexpr int kHPad = 80;                                         // h operand columns: 64 hidden | 1 | 0 x 15
 constexpr uint32_t kHSbo = (kHPad / 8) * 128;                     // 1280: next 8 rows of the h operand
 constexpr uint32_t kHLo = kTileRows * kHPad * 2;                  // 20480: lo part
@@ -842,7 +839,7 @@ __global__ void __launch_bounds__(kTThreads, 1) tc_wide_train_kernel(const Args 
                     // [gW2chunk | gb2] = G^T . [h | 1] : K = 128 rows, both operands MN-major views
                     uint32_t acc = 0;
 #pragma unroll
-                    for (int p = (STB_TRAIN_EXP & 4) ? 2 : 0; p < 3; ++p) {
+                    for (int p = 0; p < 3; ++p) {
                         const uint32_t aa = (p == 0) ? g_lo : g_hi, bb = (p == 1) ? a_lo : a_hi;
 #pragma unroll
                         for (int ks = 0; ks < kTileRows / 16; ++ks) {
@@ -1062,7 +1059,6 @@ __global__ void __launch_bounds__(kTThreads, 1) tc_wide_train_kernel(const Args 
                         tmem_ld_wait();
 #pragma unroll
                         for (int i = 0; i < 16; i += 4) {
-                            if (STB_TRAIN_EXP & 1) { if (v[i] == 123.456f) dst[0] = v[i + 1]; continue; }
                             red_add4(dst + hh2 * 16 + i, v[i] * inv_sigma, v[i + 1] * inv_sigma, v[i + 2] * inv_sigma, v[i + 3] * inv_sigma);
                         }
                     }
@@ -1117,10 +1113,8 @@ __global__ void __launch_bounds__(kTThreads, 1) tc_wide_train_kernel(const Args 
                     kk = bs.k;
                     const float u0 = (kk == 0) ? STB_RQS_EDGE_CONST : fmaf(r0, s2, bb[2 * kBins + (kk > 0 ? kk - 1 : 0)]);
                     const float u1 = (kk == kBins - 1) ? STB_RQS_EDGE_CONST : fmaf(r1, s2, bb[2 * kBins + (kk < kBins - 1 ? kk : 0)]);
-                    if (inside && !(STB_TRAIN_EXP & 2)) {
+                    if (inside) {
                         rqs16_backward<INVERSE>(t, bs, ee, eo, u0, u1, lo, hi, xv, go, g_ld, gx, gu0, gu1);
-                    } else if (STB_TRAIN_EXP & 2) {
-                        gx = go + u0 * 1e-30f + u1 * 1e-30f + t[3].x * 1e-30f;
                     } else {
 #pragma unroll
                         for (int i = 0; i < kBins; ++i) t[i] = f2(0.f);
@@ -1498,16 +1492,9 @@ int tcw_pack_layer(const stb_layer* L, void* out, cudaStream_t stream) {
 
 static int tcw_launch(void (*kern)(tcw::Args), const tcw::Args& A, long long tiles, cudaStream_t stream, const char* what) {
     using namespace tcw;
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
     if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    const int grid = (int)min((long long)n_sm, tiles);
+    const int grid = (int)min((long long)sm_count(), tiles);
     kern<<<grid, kThreads, kSmemBytes, stream>>>(A);
     count_launch();
     e = cudaGetLastError();
@@ -1632,16 +1619,9 @@ int tcw_layer_backward_fused(const stb_layer* L, const void* image, int directio
     void (*kern)(train::Args);
     if (L->kind == STB_RQS) kern = inv ? train::tc_wide_train_kernel<STB_RQS, true> : train::tc_wide_train_kernel<STB_RQS, false>;
     else kern = inv ? train::tc_wide_train_kernel<STB_CUBIC, true> : train::tc_wide_train_kernel<STB_CUBIC, false>;
-    static thread_local int n_sm = 0;
-    if (n_sm == 0) {
-        int dev = 0;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-        if (n_sm <= 0) n_sm = 148;
-    }
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)train::kSmemBytes);
     if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    int grid = (int)min((long long)n_sm, tiles);
+    int grid = (int)min((long long)sm_count(), tiles);
     const bool det = train_deterministic();
     if (det) {
         grid = min(grid, train::kDetMaxCtas);

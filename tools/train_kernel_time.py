@@ -31,4 +31,4 @@ for _ in range(n):
     e[2].record()
     torch.cuda.synchronize()
     tb += e[1].elapsed_time(e[2])
-print(f'lib {os.environ.get("STRIBOR_B200_LIB", "default")}: forward {tf / n:.3f} ms, backward (incl. host-side ops) {tb / n:.3f} ms per layer at {rows} rows')
+print(f'forward {tf / n:.3f} ms, backward (incl. host-side ops) {tb / n:.3f} ms per layer at {rows} rows')

@@ -1,6 +1,6 @@
 // Microbenchmark: issue throughput and dependent latency of scalar vs packed fp32 (FFMA vs FFMA2,
 // FADD vs FADD2), predicated FADD2, MUFU.EX2, FMNMX3 and mixes, per SM sub-partition on sm_100a.
-//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o variants/ubench_f32x2 tools/ubench/f32x2.cu
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o /tmp/ubench_f32x2 tools/ubench/f32x2.cu
 #include <cstdio>
 #include <cuda_runtime.h>
 
