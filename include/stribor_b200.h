@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define STB_ABI_VERSION 2
+#define STB_ABI_VERSION 3
 #define STB_MAX_LINEAR 8
 
 /* error codes */
@@ -83,8 +83,29 @@ typedef struct stb_mlp {
  * Network output layout (flows/affine.py:66, flows/spline.py:82-86):
  *   affine / cont-affine: [log_scale(dim) | shift(dim)]
  *   rqs:   per dim [widths(K) | heights(K) | derivatives(K-1)]
+ *          (K+1 derivatives, boundary ones included, when spline.free_edge_derivs is set)
  *   cubic: per dim [widths(K) | heights(K) | left, right derivative]
  */
+
+/* Spline constants of the functional API: the keyword arguments of the reference's
+ * unconstrained_rational_quadratic_spline / unconstrained_cubic_spline.  custom == 0 (a zero-filled block) means the reference
+ * defaults -- rqs: minimum bin width / height / derivative 1e-3, K-1 derivatives;
+ * cubic: minimum bin width / height 1e-2, eps 1e-5, quadratic_threshold 1e-3 -- and every
+ * other field is ignored.  With custom != 0 all fields of the layer's kind are used.
+ * Layers with custom != 0 run on the CUDA-core kernels only (row_out / const_out
+ * parameters); they never take a tensor-core path. */
+typedef struct stb_spline_opts {
+    int32_t custom;
+    float min_bin_width, min_bin_height;  /* rqs and cubic; min * n_bins <= 1 each        */
+    float min_derivative;                 /* rqs: derivative = min + softplus(param), >= 0 */
+    int32_t free_edge_derivs;             /* rqs: 1 = K+1 derivative parameters per dim, the
+                                             boundary derivatives included; 0 = K-1, the
+                                             boundaries padded with log(exp(1 - min) - 1),
+                                             i.e. a boundary derivative of exactly 1       */
+    float cub_eps;                        /* cubic: root window of the inverse            */
+    float cub_quad_threshold;             /* cubic: |a| below it -> quadratic formula     */
+} stb_spline_opts;
+
 typedef struct stb_layer {
     int32_t kind;
     int32_t dim;
@@ -121,6 +142,7 @@ typedef struct stb_layer {
     const int32_t* perm_host;      /* HOST copies of perm / perm_inv (optional).  With them a permutation  */
     const int32_t* perm_inv_host;  /* between chained couplings is folded into the neighbouring kernels'    */
                                    /* gather / scatter index lists instead of costing an HBM pass           */
+    stb_spline_opts spline;        /* rqs / cubic constants; zero-filled = the reference defaults          */
 } stb_layer;
 
 int stb_abi_version(void);

@@ -10,7 +10,7 @@ import ctypes as C
 import os
 
 STB_MAX_LINEAR = 8
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 # enums (include/stribor_b200.h)
 AFFINE, RQS, CUBIC, CONT_AFFINE, PERMUTE, SIGMOID, LOGIT = 0, 1, 2, 3, 4, 5, 6
@@ -35,6 +35,12 @@ class StbMlp(C.Structure):
                 ('W', C.c_void_p * STB_MAX_LINEAR), ('b', C.c_void_p * STB_MAX_LINEAR)]
 
 
+class StbSplineOpts(C.Structure):
+    _fields_ = [('custom', C.c_int32), ('min_bin_width', C.c_float), ('min_bin_height', C.c_float),
+                ('min_derivative', C.c_float), ('free_edge_derivs', C.c_int32),
+                ('cub_eps', C.c_float), ('cub_quad_threshold', C.c_float)]
+
+
 class StbLayer(C.Structure):
     _fields_ = [('kind', C.c_int32), ('dim', C.c_int32), ('latent_dim', C.c_int32),
                 ('cond_x', C.c_int32), ('time_input', C.c_int32), ('n_bins', C.c_int32),
@@ -45,7 +51,7 @@ class StbLayer(C.Structure):
                 ('mask', C.c_void_p), ('mask_host', C.c_void_p), ('const_out', C.c_void_p), ('row_out', C.c_void_p),
                 ('time_scale', C.c_void_p), ('perm', C.c_void_p), ('perm_inv', C.c_void_p),
                 ('net', StbMlp), ('packed', C.c_void_p), ('packed_bytes', C.c_uint64),
-                ('perm_host', C.c_void_p), ('perm_inv_host', C.c_void_p)]
+                ('perm_host', C.c_void_p), ('perm_inv_host', C.c_void_p), ('spline', StbSplineOpts)]
 
 
 class StbLayerGrads(C.Structure):

@@ -12,7 +12,9 @@ A layer is described by plain data so that it can cross the op boundary:
   meta  = [kind, dim, latent_dim, cond_x, time_input, n_bins, inverse_ldj_own, zero_cond,
            activation, final_activation, n_linear, n_params, has_box, row_mode, dims[0..n_linear],
            mask[0..dim) (only when cond_x)]
-  fmeta = [lower, upper, left, right, bottom, top]
+  fmeta = [lower, upper, left, right, bottom, top] (+ [custom, min_bin_width, min_bin_height, min_derivative,
+           free_edge_derivs, cub_eps, cub_quad_threshold]: stb_spline_opts, functional spline API only;
+           without them the reference defaults)
   params = [W0, b0, W1, b1, ...] (+ [time_scale]) or [const_out]   (row_mode: const_out is a
            per-row [rows, out_width] tensor -> stb_layer.row_out; row_mode 2 = compact: only the
            transformed dims' parameters, [rows, n_tr * P])
@@ -30,6 +32,7 @@ from . import _lib
 
 META_HEADER = 14
 FMETA_LEN = 6
+SPLINE_OPTS_LEN = 7
 
 
 def _check_cuda(x: Tensor, what: str):
@@ -85,6 +88,12 @@ def _fill_struct(L: _lib.StbLayer, meta: Sequence[int], fmeta: Sequence[float], 
     L.lower, L.upper = float(fmeta[0]), float(fmeta[1])
     L.left, L.right, L.bottom, L.top = (float(v) for v in fmeta[2:6])
     L.has_box = has_box
+    if len(fmeta) > FMETA_LEN:
+        custom, mw, mh, md, free_edge, eps, quad = fmeta[FMETA_LEN:FMETA_LEN + SPLINE_OPTS_LEN]
+        o = L.spline
+        o.custom, o.free_edge_derivs = int(custom), int(free_edge)
+        o.min_bin_width, o.min_bin_height, o.min_derivative = float(mw), float(mh), float(md)
+        o.cub_eps, o.cub_quad_threshold = float(eps), float(quad)
     L.row_compact = 1 if row_mode == 2 else 0
     L.mask = _dp(mask)
     keep = None

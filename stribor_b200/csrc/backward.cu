@@ -18,7 +18,7 @@ constexpr int kBColStride = kBThreads + 1;
 constexpr int kBXsStride = kBTileRows + 1;
 
 struct BwdArgs {
-    stb_layer L;
+    LayerArgs L;
     int direction;
     int P, width, n_tr;
     const float* x;
@@ -41,12 +41,14 @@ __device__ __forceinline__ int bwd_col(const stb_layer& L, int P, int n_tr, int 
     return aff ? p * L.dim + j : j * P + p;
 }
 
-template <int KIND>
-__global__ void __launch_bounds__(kBThreads) elementwise_backward_kernel(const BwdArgs A) {
+// One tile of elementwise_backward_kernel; O holds the spline constants (stb_math.cuh).  The kernel
+// reads threadIdx.x itself: there the compiler knows its range from __launch_bounds__.
+template <int KIND, class O>
+__device__ __forceinline__ void elementwise_backward_tile(const BwdArgs& A, const O& o, const int tid) {
     extern __shared__ __align__(16) float smem[];
-    const stb_layer& L = A.L;
+    const stb_layer& L = A.L.get();
     const int d = L.dim, P = A.P;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     const long long row0 = (long long)blockIdx.x * kBTileRows;
     const int nrows = (int)min((long long)kBTileRows, A.rows - row0);
 
@@ -125,7 +127,7 @@ __global__ void __launch_bounds__(kBThreads) elementwise_backward_kernel(const B
         float g_ld = g_ld_row;
         if (A.g_ldiag != nullptr && lane < nrows) g_ld += A.g_ldiag[(row0 + lane) * d + j];
         float gx;
-        if (KIND == STB_AFFINE) {
+        if constexpr (KIND == STB_AFFINE) {
             const float ls = col[0], sh = col[1];
             if (inverse) {
                 const float e = expf(-ls), out = (xv - sh) * e;
@@ -134,12 +136,12 @@ __global__ void __launch_bounds__(kBThreads) elementwise_backward_kernel(const B
                 const float e = expf(ls);
                 gx = go * e; gcol[1] = go; gcol[0] = go * xv * e + g_ld;
             }
-        } else if (KIND == STB_RQS) {
+        } else if constexpr (KIND == STB_RQS) {
             const bool box = L.has_box != 0;
             rqs_element_grad(col, gcol, L.n_bins, box ? L.left : L.lower, box ? L.right : L.upper,
-                             box ? L.bottom : L.lower, box ? L.top : L.upper, inverse, xv, go, g_ld, gx);
+                             box ? L.bottom : L.lower, box ? L.top : L.upper, inverse, xv, go, g_ld, gx, o);
         } else {
-            cubic_element_grad(col, gcol, L.n_bins, L.lower, L.upper, inverse, xv, go, g_ld, gx);
+            cubic_element_grad(col, gcol, L.n_bins, L.lower, L.upper, inverse, xv, go, g_ld, gx, o);
         }
         gs[j * kBXsStride + lane] = gx;
         __syncwarp();
@@ -167,6 +169,17 @@ __global__ void __launch_bounds__(kBThreads) elementwise_backward_kernel(const B
             gx[i] = gs[c * kBXsStride + r];
         }
     }
+}
+
+template <int KIND>
+__global__ void __launch_bounds__(kBThreads) elementwise_backward_kernel(const BwdArgs A) {
+    elementwise_backward_tile<KIND>(A, DefaultOpts<KIND>(), threadIdx.x);
+}
+
+// splines with the functional API's non-default constants (stb_layer.spline.custom != 0)
+template <int KIND>
+__global__ void __launch_bounds__(kBThreads) elementwise_backward_opts_kernel(const BwdArgs A, const SplineOpts o) {
+    elementwise_backward_tile<KIND>(A, o, threadIdx.x);
 }
 
 // n_linear > 0 on the tensor-core path: the workspace receives the conditioner's hidden activations,
@@ -211,10 +224,11 @@ int layer_backward(const stb_layer* L, int direction, const float* x, const floa
     if (rows == 0) return STB_OK;
     if (L->row_compact && !L->mask_host && L->cond_x) return set_error(STB_EINVAL, "row_compact needs mask_host");
 
+    const bool custom = L->spline.custom && (L->kind == STB_RQS || L->kind == STB_CUBIC);
     BwdArgs A;
-    A.L = *L;
+    A.L.set(L);
     A.direction = direction;
-    A.P = bwd_params_per_dim(L->kind, L->n_bins);
+    A.P = bwd_params_per_dim(L->kind, L->n_bins) + (custom && L->kind == STB_RQS && L->spline.free_edge_derivs ? 2 : 0);
     int n_tr = L->dim;
     if (L->cond_x && L->mask_host) {
         n_tr = 0;
@@ -229,17 +243,20 @@ int layer_backward(const stb_layer* L, int direction, const float* x, const floa
                         sizeof(int) * (size_t)L->dim;
     if (smem > 227 * 1024) return set_error(STB_ENOTSUP, "layer needs %zu B of shared memory per tile", smem);
     void (*kern)(BwdArgs) = nullptr;
+    void (*kern_opts)(BwdArgs, SplineOpts) = nullptr;
     switch (L->kind) {
         case STB_AFFINE: kern = elementwise_backward_kernel<STB_AFFINE>; break;
-        case STB_RQS: kern = elementwise_backward_kernel<STB_RQS>; break;
-        default: kern = elementwise_backward_kernel<STB_CUBIC>; break;
+        case STB_RQS: kern = elementwise_backward_kernel<STB_RQS>; kern_opts = elementwise_backward_opts_kernel<STB_RQS>; break;
+        default: kern = elementwise_backward_kernel<STB_CUBIC>; kern_opts = elementwise_backward_opts_kernel<STB_CUBIC>; break;
     }
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = custom ? cudaFuncSetAttribute(kern_opts, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                               : cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     }
     const long long tiles = (rows + kBTileRows - 1) / kBTileRows;
-    kern<<<(unsigned)tiles, kBThreads, smem, stream>>>(A);
+    if (custom) kern_opts<<<(unsigned)tiles, kBThreads, smem, stream>>>(A, make_spline_opts(L->spline));
+    else kern<<<(unsigned)tiles, kBThreads, smem, stream>>>(A);
     count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_error(STB_ECUDA, "elementwise_backward_kernel launch: %s", cudaGetErrorString(e));

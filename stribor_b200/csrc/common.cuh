@@ -2,10 +2,21 @@
 // thread-local error text, launch counter, SM count, internal entry points.
 #pragma once
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
+#include <string.h>
 #include "../../include/stribor_b200.h"
 
 namespace stb {
+
+// A kernel's by-value copy of a stb_layer: its fields up to, not including, `spline`.  The spline options reach
+// only the kernels instantiated for non-default options, as a kernel parameter of their own, so the argument
+// layout of every other kernel is the one it had before the options were appended to stb_layer.
+struct LayerArgs {
+    alignas(stb_layer) unsigned char raw[offsetof(stb_layer, spline)];
+    void set(const stb_layer* L) { memcpy(raw, L, sizeof raw); }
+    __host__ __device__ __forceinline__ const stb_layer& get() const { return *reinterpret_cast<const stb_layer*>(raw); }
+};
 
 int set_error(int code, const char* fmt, ...);
 void count_launch();

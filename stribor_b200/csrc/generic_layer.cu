@@ -24,7 +24,7 @@ constexpr int kXsStride = kTileRows + 1;
 constexpr int kColStride = kGenThreads + 1;    // padded: conflict-free per-thread AND transposed access
 
 struct GenArgs {
-    stb_layer L;
+    LayerArgs L;
     int direction;
     int ldj_mode;
     int base_log_prob;
@@ -43,6 +43,12 @@ struct GenArgs {
 
 __host__ __device__ inline int params_per_dim(int kind, int K) {
     return kind == STB_RQS ? 3 * K - 1 : (kind == STB_CUBIC ? 2 * K + 2 : 2);
+}
+
+// the same, with the two free boundary derivatives of an rqs layer that asks for them
+inline int layer_params_per_dim(const stb_layer* L) {
+    const bool free_edge = L->kind == STB_RQS && L->spline.custom && L->spline.free_edge_derivs;
+    return params_per_dim(L->kind, L->n_bins) + (free_edge ? 2 : 0);
 }
 
 // row of the conditioner output holding parameter p of dim j
@@ -85,12 +91,14 @@ __device__ __forceinline__ void dot_rows(const float* __restrict__ W, int in_dim
     }
 }
 
-template <int KIND>
-__global__ void __launch_bounds__(kGenThreads) generic_layer_kernel(const GenArgs A) {
+// One tile of generic_layer_kernel; O holds the spline constants (stb_math.cuh).  The kernel reads
+// threadIdx.x itself: there the compiler knows its range from __launch_bounds__.
+template <int KIND, class O>
+__device__ __forceinline__ void generic_layer_tile(const GenArgs& A, const O& o, const int tid) {
     extern __shared__ __align__(16) float smem[];
-    const stb_layer& L = A.L;
+    const stb_layer& L = A.L.get();
     const int d = L.dim;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     const long long row0 = (long long)blockIdx.x * kTileRows;
     const int nrows = (int)min((long long)kTileRows, A.rows - row0);
     const int P = A.P;
@@ -232,27 +240,27 @@ __global__ void __launch_bounds__(kGenThreads) generic_layer_kernel(const GenArg
         }
         const float xv = xs[j * kXsStride + lane];
         float out, ld;
-        if (KIND == STB_AFFINE) {
+        if constexpr (KIND == STB_AFFINE) {
             const float ls = col[0], sh = col[1];
             if (inverse) { out = (xv - sh) * expf(-ls); ld = -ls; }
             else { out = xv * expf(ls) + sh; ld = ls; }
-        } else if (KIND == STB_CONT_AFFINE) {
+        } else if constexpr (KIND == STB_CONT_AFFINE) {
             const float tv = t_s[lane];
             const float tls = __ldg(L.time_scale + j) * tv;
             const float tsh = __ldg(L.time_scale + d + j) * tv;
             const float a = col[0] * tls, sh = col[1] * tsh;
             if (inverse) { out = (xv - sh) * expf(-a); ld = -a; }
             else { out = xv * expf(a) + sh; ld = a; }
-        } else if (KIND == STB_RQS) {
+        } else if constexpr (KIND == STB_RQS) {
             const bool box = L.has_box != 0;
             int kb;
             rqs_element(col, L.n_bins, box ? L.left : L.lower, box ? L.right : L.upper,
                         box ? L.bottom : L.lower, box ? L.top : L.upper, inverse,
-                        L.inverse_ldj_own != 0, xv, out, ld, &kb);
+                        L.inverse_ldj_own != 0, xv, out, ld, &kb, o);
             if (A.bins && lane < nrows) A.bins[(row0 + lane) * d + j] = kb;
-        } else {
+        } else if constexpr (KIND == STB_CUBIC) {
             int kb;
-            cubic_element(col, L.n_bins, L.lower, L.upper, inverse, L.inverse_ldj_own != 0, xv, out, ld, &kb);
+            cubic_element(col, L.n_bins, L.lower, L.upper, inverse, L.inverse_ldj_own != 0, xv, out, ld, &kb, o);
             if (A.bins && lane < nrows) A.bins[(row0 + lane) * d + j] = kb;
         }
         xs[j * kXsStride + lane] = out;
@@ -298,6 +306,17 @@ __global__ void __launch_bounds__(kGenThreads) generic_layer_kernel(const GenArg
             }
         }
     }
+}
+
+template <int KIND>
+__global__ void __launch_bounds__(kGenThreads) generic_layer_kernel(const GenArgs A) {
+    generic_layer_tile<KIND>(A, DefaultOpts<KIND>(), threadIdx.x);
+}
+
+// splines with the functional API's non-default constants (stb_layer.spline.custom != 0)
+template <int KIND>
+__global__ void __launch_bounds__(kGenThreads) generic_layer_opts_kernel(const GenArgs A, const SplineOpts o) {
+    generic_layer_tile<KIND>(A, o, threadIdx.x);
 }
 
 __global__ void unit_normal_kernel(const float* __restrict__ x, float* __restrict__ lp, int accumulate,
@@ -404,12 +423,23 @@ int validate_layer(const stb_layer* L) {
     if (L->cond_x && !L->mask) return set_error(STB_EINVAL, "coupling layer needs a mask");
     const stb_mlp& N = L->net;
     if (N.n_linear < 0 || N.n_linear > STB_MAX_LINEAR) return set_error(STB_EINVAL, "n_linear %d out of range", N.n_linear);
-    const int P = params_per_dim(L->kind, L->n_bins);
+    const int P = layer_params_per_dim(L);
     if (L->kind == STB_RQS || L->kind == STB_CUBIC) {
         if (L->n_bins < 1) return set_error(STB_EINVAL, "n_bins must be >= 1");
         // rational_quadratic_spline.py:96-99 / cubic_spline.py:94-97
-        const float mn = L->kind == STB_RQS ? 1e-3f : 1e-2f;
-        if (mn * L->n_bins > 1.0f) return set_error(STB_EINVAL, "Minimal bin width too large for the number of bins");
+        const stb_spline_opts& so = L->spline;
+        if (!so.custom) {
+            const float mn = L->kind == STB_RQS ? 1e-3f : 1e-2f;
+            if (mn * L->n_bins > 1.0f) return set_error(STB_EINVAL, "Minimal bin width too large for the number of bins");
+        } else {
+            const bool rqs = L->kind == STB_RQS;
+            const bool finite = isfinite(so.min_bin_width) && isfinite(so.min_bin_height) &&
+                                (rqs ? isfinite(so.min_derivative) : isfinite(so.cub_eps) && isfinite(so.cub_quad_threshold));
+            if (!finite) return set_error(STB_EINVAL, "spline options must be finite");
+            if (so.min_bin_width * L->n_bins > 1.0f) return set_error(STB_EINVAL, "Minimal bin width too large for the number of bins");
+            if (so.min_bin_height * L->n_bins > 1.0f) return set_error(STB_EINVAL, "Minimal bin height too large for the number of bins");
+            if (rqs && so.min_derivative < 0.f) return set_error(STB_EINVAL, "min_derivative must be >= 0");
+        }
         if (L->has_box) {
             if (L->kind != STB_RQS) return set_error(STB_EINVAL, "separate domain/codomain boxes are rqs-only");
             if (!(L->right > L->left) || !(L->top > L->bottom)) return set_error(STB_EINVAL, "empty spline box");
@@ -434,11 +464,11 @@ int generic_layer_apply(const stb_layer* L, int direction, const float* x, const
                         const float* t, float* y, float* ldj, int ldj_mode, int base_log_prob,
                         float* ldiag, int64_t rows, cudaStream_t stream, int32_t* bins) {
     GenArgs A;
-    A.L = *L;
+    A.L.set(L);
     A.direction = direction;
     A.ldj_mode = ldj ? ldj_mode : STB_LDJ_NONE;
     A.base_log_prob = base_log_prob;
-    A.P = params_per_dim(L->kind, L->n_bins);
+    A.P = layer_params_per_dim(L);
     A.in_dim = L->net.n_linear > 0 ? L->net.dims[0] : 0;
     int buf_rows = 1;
     for (int i = 0; i < L->net.n_linear; ++i) buf_rows = max(buf_rows, L->net.dims[i]);
@@ -450,20 +480,24 @@ int generic_layer_apply(const stb_layer* L, int direction, const float* x, const
                   sizeof(int) * (size_t)L->dim + (ldiag ? sizeof(float) * (size_t)L->dim * kXsStride : 0);
     if (smem > 227 * 1024) return set_error(STB_ENOTSUP, "layer needs %zu B of shared memory per tile (> 227 KB)", smem);
 
+    const bool custom = L->spline.custom && (L->kind == STB_RQS || L->kind == STB_CUBIC);
     void (*kern)(GenArgs) = nullptr;
+    void (*kern_opts)(GenArgs, SplineOpts) = nullptr;
     switch (L->kind) {
         case STB_AFFINE: kern = generic_layer_kernel<STB_AFFINE>; break;
-        case STB_RQS: kern = generic_layer_kernel<STB_RQS>; break;
-        case STB_CUBIC: kern = generic_layer_kernel<STB_CUBIC>; break;
+        case STB_RQS: kern = generic_layer_kernel<STB_RQS>; kern_opts = generic_layer_opts_kernel<STB_RQS>; break;
+        case STB_CUBIC: kern = generic_layer_kernel<STB_CUBIC>; kern_opts = generic_layer_opts_kernel<STB_CUBIC>; break;
         default: kern = generic_layer_kernel<STB_CONT_AFFINE>; break;
     }
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = custom ? cudaFuncSetAttribute(kern_opts, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                               : cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     }
     const long long tiles = (rows + kTileRows - 1) / kTileRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
-    kern<<<(unsigned)tiles, kGenThreads, smem, stream>>>(A);
+    if (custom) kern_opts<<<(unsigned)tiles, kGenThreads, smem, stream>>>(A, make_spline_opts(L->spline));
+    else kern<<<(unsigned)tiles, kGenThreads, smem, stream>>>(A);
     count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_error(STB_ECUDA, "generic_layer_kernel launch: %s", cudaGetErrorString(e));

@@ -111,22 +111,24 @@ __device__ __forceinline__ void rqs_bin_dual(float x, float xk, float xk1, float
 
 // Gradients of one RQS element.
 //   sw, sh : NORMALISED bin sizes (min + scale * softmax), K each;  ud: K-1 raw derivative params
+//            (K+1, the boundaries included, with o.free_edge())
 //   direction / own_ld as rqs_element;  x: the element's input;  g_out, g_ld: incoming gradients
-// Writes g_x and the gradient wrt the K + K + (K-1) RAW parameters into gp[] (same indexable type).
+// Writes g_x and the gradient wrt the K + K + (K-1 or K+1) RAW parameters into gp[] (same indexable type).
 // Domain [left, right] -> codomain [bottom, top] (rational_quadratic_spline.py:55-64); the common case is
 // left == bottom == lower, right == top == upper.
-template <class P>
+template <class P, class O = RqsDefaults>
 __device__ __forceinline__ void rqs_element_grad(P prm, P gp, int K, float left, float right, float bottom,
                                                  float top, bool inverse, float x, float g_out, float g_ld,
-                                                 float& g_x) {
-    const int Pn = 3 * K - 1;
+                                                 float& g_x, const O& o = O()) {
+    const int Pn = o.free_edge() ? 3 * K + 1 : 3 * K - 1;
     for (int i = 0; i < Pn; ++i) gp[i] = 0.f;
     g_x = g_out;                                   // identity tails
     if (!(x >= (inverse ? bottom : left) && x <= (inverse ? top : right))) return;
     OffsetView<P> W{prm, 0}, H{prm, K}, D{prm, 2 * K};
     OffsetView<P> GW{gp, 0}, GH{gp, K}, GD{gp, 2 * K};
-    softmax_bins(W, K, STB_RQS_MIN);               // normalised sizes, kept (not turned into knots)
-    softmax_bins(H, K, STB_RQS_MIN);
+    const float mw = o.min_w(), mh = o.min_h();
+    softmax_bins(W, K, mw);                        // normalised sizes, kept (not turned into knots)
+    softmax_bins(H, K, mh);
     const float spanx = right - left, spany = top - bottom;
     // bin search by running sums (same arithmetic as sizes_to_knots + knot_search)
     int k = 0;
@@ -142,9 +144,15 @@ __device__ __forceinline__ void rqs_element_grad(P prm, P gp, int K, float left,
     const float yk = (k == 0) ? bottom : spany * chk + bottom;
     const float xk1 = (k == K - 1) ? right : spanx * (cwk + wk_) + left;
     const float yk1 = (k == K - 1) ? top : spany * (chk + hk_) + bottom;
-    const float u0 = (k == 0) ? STB_RQS_EDGE_CONST : D[k - 1];
-    const float u1 = (k == K - 1) ? STB_RQS_EDGE_CONST : D[k];
-    const float d0 = STB_RQS_MIN + softplus_f(u0), d1 = STB_RQS_MIN + softplus_f(u1);
+    float u0, u1;
+    if (o.free_edge()) {
+        u0 = D[k];
+        u1 = D[k + 1];
+    } else {
+        u0 = (k == 0) ? o.edge() : D[k - 1];
+        u1 = (k == K - 1) ? o.edge() : D[k];
+    }
+    const float d0 = o.min_d() + softplus_f(u0), d1 = o.min_d() + softplus_f(u1);
 
     float xe = x;                                  // point at which S, L are expanded
     if (inverse) {
@@ -174,23 +182,30 @@ __device__ __forceinline__ void rqs_element_grad(P prm, P gp, int K, float left,
     const float g_ch = spany * ((k > 0 ? gq[RQ_YK] : 0.f) + (k < K - 1 ? gq[RQ_YK1] : 0.f));
     const float g_hk = spany * (k < K - 1 ? gq[RQ_YK1] : 0.f);
     // sizes -> raw (softmax backward): w_i = min + scale * s_i, s_i = (w_i - min) / scale
-    const float scale = 1.f - STB_RQS_MIN * (float)K;
+    // (min * K == 1 leaves scale 0: the sizes are constants and their raw parameters get no gradient)
+    const float scale_w = 1.f - mw * (float)K, scale_h = 1.f - mh * (float)K;
     float dotw = 0.f, doth = 0.f;
     for (int i = 0; i <= k; ++i) {
         const float gwi = (i < k) ? g_cw : g_wk, ghi = (i < k) ? g_ch : g_hk;
-        dotw += (W[i] - STB_RQS_MIN) * gwi;        // = scale * s_i * g_w_i
-        doth += (H[i] - STB_RQS_MIN) * ghi;
+        dotw += (W[i] - mw) * gwi;                 // = scale * s_i * g_w_i
+        doth += (H[i] - mh) * ghi;
     }
     for (int i = 0; i < K; ++i) {
         const float gwi = (i < k) ? g_cw : ((i == k) ? g_wk : 0.f);
         const float ghi = (i < k) ? g_ch : ((i == k) ? g_hk : 0.f);
-        const float sw = (W[i] - STB_RQS_MIN) / scale, sh = (H[i] - STB_RQS_MIN) / scale;
-        GW[i] = sw * (scale * gwi - dotw);
-        GH[i] = sh * (scale * ghi - doth);
+        const float sw = (O::kRuntime && scale_w == 0.f) ? 0.f : (W[i] - mw) / scale_w;
+        const float sh = (O::kRuntime && scale_h == 0.f) ? 0.f : (H[i] - mh) / scale_h;
+        GW[i] = sw * (scale_w * gwi - dotw);
+        GH[i] = sh * (scale_h * ghi - doth);
     }
     // derivatives: d = min + softplus(u), softplus' = sigmoid (1 beyond the threshold)
-    if (k > 0) GD[k - 1] = gq[RQ_D0] * (u0 > 20.f ? 1.f : sigmoid_f(u0));
-    if (k < K - 1) GD[k] = gq[RQ_D1] * (u1 > 20.f ? 1.f : sigmoid_f(u1));
+    if (o.free_edge()) {                           // the boundary parameters are free too
+        GD[k] = gq[RQ_D0] * (u0 > 20.f ? 1.f : sigmoid_f(u0));
+        GD[k + 1] = gq[RQ_D1] * (u1 > 20.f ? 1.f : sigmoid_f(u1));
+    } else {
+        if (k > 0) GD[k - 1] = gq[RQ_D0] * (u0 > 20.f ? 1.f : sigmoid_f(u0));
+        if (k < K - 1) GD[k] = gq[RQ_D1] * (u1 > 20.f ? 1.f : sigmoid_f(u1));
+    }
 }
 
 // --------------------------------------------------------------------------------------------
@@ -236,9 +251,10 @@ __device__ __forceinline__ void cubic_bin_dual(int k, int K, float u, float wp, 
 }
 
 // prm = [uw(K) | uh(K) | left, right] raw; gp receives the gradient wrt those 2K + 2 values.
-template <class P>
+template <class P, class O = CubDefaults>
 __device__ __forceinline__ void cubic_element_grad(P prm, P gp, int K, float lower, float upper, bool inverse,
-                                                   float x, float g_out, float g_ld, float& g_x) {
+                                                   float x, float g_out, float g_ld, float& g_x,
+                                                   const O& o = O()) {
     const int Pn = 2 * K + 2;
     for (int i = 0; i < Pn; ++i) gp[i] = 0.f;
     g_x = g_out;
@@ -246,8 +262,9 @@ __device__ __forceinline__ void cubic_element_grad(P prm, P gp, int K, float low
     OffsetView<P> W{prm, 0}, H{prm, K};
     OffsetView<P> GW{gp, 0}, GH{gp, K};
     const float ul = prm[2 * K], ur = prm[2 * K + 1];
-    softmax_bins(W, K, STB_CUB_MIN);
-    softmax_bins(H, K, STB_CUB_MIN);
+    const float mw = o.min_w(), mh = o.min_h();
+    softmax_bins(W, K, mw);
+    softmax_bins(H, K, mh);
     const float span = upper - lower;
     const float u = (x - lower) / span;
     float cw, ch;
@@ -256,7 +273,7 @@ __device__ __forceinline__ void cubic_element_grad(P prm, P gp, int K, float low
     if (inverse) {
         const CubBin b = cubic_bin(W, H, K, k, cw, ch, ul, ur);
         float ld_own;
-        ue = cubic_inverse_in_bin(b, u, ld_own);
+        ue = cubic_inverse_in_bin(b, u, ld_own, o);
     }
     const float wp = k > 0 ? W[k - 1] : 1.f, hp = k > 0 ? H[k - 1] : 1.f;
     const float wn = k < K - 1 ? W[k + 1] : 1.f, hn = k < K - 1 ? H[k + 1] : 1.f;
@@ -279,7 +296,7 @@ __device__ __forceinline__ void cubic_element_grad(P prm, P gp, int K, float low
         g_x = gu / span;
     }
     // neighbours / cumulative sums -> normalised sizes
-    const float scale = 1.f - STB_CUB_MIN * (float)K;
+    const float scale_w = 1.f - mw * (float)K, scale_h = 1.f - mh * (float)K;
     float dotw = 0.f, doth = 0.f;
     for (int i = 0; i < K; ++i) {
         float gwi = (i < k) ? gq[CU_CW] : 0.f, ghi = (i < k) ? gq[CU_CH] : 0.f;
@@ -288,13 +305,14 @@ __device__ __forceinline__ void cubic_element_grad(P prm, P gp, int K, float low
         if (i == k + 1) { gwi += gq[CU_WN]; ghi += gq[CU_HN]; }
         GW[i] = gwi;                                  // stash, converted below
         GH[i] = ghi;
-        dotw += (W[i] - STB_CUB_MIN) * gwi;
-        doth += (H[i] - STB_CUB_MIN) * ghi;
+        dotw += (W[i] - mw) * gwi;
+        doth += (H[i] - mh) * ghi;
     }
     for (int i = 0; i < K; ++i) {
-        const float sw = (W[i] - STB_CUB_MIN) / scale, sh = (H[i] - STB_CUB_MIN) / scale;
-        GW[i] = sw * (scale * GW[i] - dotw);
-        GH[i] = sh * (scale * GH[i] - doth);
+        const float sw = (O::kRuntime && scale_w == 0.f) ? 0.f : (W[i] - mw) / scale_w;
+        const float sh = (O::kRuntime && scale_h == 0.f) ? 0.f : (H[i] - mh) / scale_h;
+        GW[i] = sw * (scale_w * GW[i] - dotw);
+        GH[i] = sh * (scale_h * GH[i] - doth);
     }
     gp[2 * K] = (k == 0) ? gq[CU_UL] : 0.f;
     gp[2 * K + 1] = (k == K - 1) ? gq[CU_UR] : 0.f;

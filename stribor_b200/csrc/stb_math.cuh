@@ -10,6 +10,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
+#include <type_traits>
 #include "../../include/stribor_b200.h"
 
 namespace stb {
@@ -89,12 +90,71 @@ __device__ __forceinline__ void softmax_bins(P u, int K, float min_size) {
 }
 
 // ---------------------------------------------------------------------------------------
-// rational-quadratic spline
+// spline constants
 // ---------------------------------------------------------------------------------------
 #define STB_RQS_MIN 1e-3f
 // log(exp(1 - 1e-3) - 1): unconstrained value that makes the boundary derivative 1
 // (rational_quadratic_spline.py:79-83)
 #define STB_RQS_EDGE_CONST 0.5397424172369522f
+#define STB_CUB_MIN 1e-2f
+#define STB_CUB_EPS 1e-5f
+#define STB_CUB_QUAD 1e-3f
+
+// The spline functions take their constants as a template parameter O.  RqsDefaults / CubDefaults
+// are the reference defaults above, folded in at compile time: the code the modules and the
+// tensor-core kernels run.  SplineOpts holds the functional API's own values (stb_spline_opts),
+// read at run time by kernels instantiated for it.
+struct RqsDefaults {
+    static constexpr bool kRuntime = false;
+    __device__ __forceinline__ float min_w() const { return STB_RQS_MIN; }
+    __device__ __forceinline__ float min_h() const { return STB_RQS_MIN; }
+    __device__ __forceinline__ float min_d() const { return STB_RQS_MIN; }
+    __device__ __forceinline__ float edge() const { return STB_RQS_EDGE_CONST; }
+    __device__ __forceinline__ bool free_edge() const { return false; }
+};
+
+struct CubDefaults {
+    static constexpr bool kRuntime = false;
+    __device__ __forceinline__ float min_w() const { return STB_CUB_MIN; }
+    __device__ __forceinline__ float min_h() const { return STB_CUB_MIN; }
+    __device__ __forceinline__ float eps() const { return STB_CUB_EPS; }
+    __device__ __forceinline__ float quad() const { return STB_CUB_QUAD; }
+};
+
+struct SplineOpts {
+    static constexpr bool kRuntime = true;
+    float mw, mh, md;
+    float edge_;       // log(exp(1 - md) - 1), evaluated in double on the host and rounded once
+    float eps_, quad_;
+    int free_edge_;
+    __device__ __forceinline__ float min_w() const { return mw; }
+    __device__ __forceinline__ float min_h() const { return mh; }
+    __device__ __forceinline__ float min_d() const { return md; }
+    __device__ __forceinline__ float edge() const { return edge_; }
+    __device__ __forceinline__ bool free_edge() const { return free_edge_ != 0; }
+    __device__ __forceinline__ float eps() const { return eps_; }
+    __device__ __forceinline__ float quad() const { return quad_; }
+};
+
+// the reference defaults of a transform kind
+template <int KIND>
+using DefaultOpts = typename std::conditional<KIND == STB_CUBIC, CubDefaults, RqsDefaults>::type;
+
+inline SplineOpts make_spline_opts(const stb_spline_opts& s) {
+    SplineOpts o;
+    o.mw = s.min_bin_width;
+    o.mh = s.min_bin_height;
+    o.md = s.min_derivative;
+    o.edge_ = (float)log(exp(1.0 - (double)s.min_derivative) - 1.0);
+    o.eps_ = s.cub_eps;
+    o.quad_ = s.cub_quad_threshold;
+    o.free_edge_ = s.free_edge_derivs;
+    return o;
+}
+
+// ---------------------------------------------------------------------------------------
+// rational-quadratic spline
+// ---------------------------------------------------------------------------------------
 
 // bin sizes u[0..K) -> knots: u[i] := knot_{i+1}, with knot_0 = lo and knot_K forced to hi.
 // rational_quadratic_spline.py:180-184 / :187-191
@@ -126,19 +186,27 @@ struct RqsBin {
     float xk, wk, yk, hk, delta, d0, d1;
 };
 
-// W, H: knot columns (after sizes_to_knots); D: K-1 unconstrained interior derivatives.
-template <class PW, class PH, class PD>
-__device__ __forceinline__ RqsBin rqs_bin(PW W, PH H, PD D, int K, int k, float left, float bottom) {
+// W, H: knot columns (after sizes_to_knots); D: K-1 unconstrained interior derivatives
+// (K+1, the boundaries included, with o.free_edge()).
+template <class PW, class PH, class PD, class O = RqsDefaults>
+__device__ __forceinline__ RqsBin rqs_bin(PW W, PH H, PD D, int K, int k, float left, float bottom,
+                                          const O& o = O()) {
     RqsBin b;
     b.xk = knot_at(W, k, left);
     b.wk = W[k] - b.xk;                                   // widths re-derived from knots (:185)
     b.yk = knot_at(H, k, bottom);
     b.hk = H[k] - b.yk;
     b.delta = b.hk / b.wk;
-    float u0 = (k == 0) ? STB_RQS_EDGE_CONST : D[k - 1];
-    float u1 = (k == K - 1) ? STB_RQS_EDGE_CONST : D[k];
-    b.d0 = STB_RQS_MIN + softplus_f(u0);                  // :107
-    b.d1 = STB_RQS_MIN + softplus_f(u1);
+    float u0, u1;
+    if (o.free_edge()) {
+        u0 = D[k];
+        u1 = D[k + 1];
+    } else {
+        u0 = (k == 0) ? o.edge() : D[k - 1];
+        u1 = (k == K - 1) ? o.edge() : D[k];
+    }
+    b.d0 = o.min_d() + softplus_f(u0);                    // :107
+    b.d1 = o.min_d() + softplus_f(u1);
     return b;
 }
 
@@ -171,34 +239,35 @@ __device__ __forceinline__ void rqs_inverse_in_bin(const RqsBin& b, float y, flo
     ld = -logf(num) + 2.f * logf(den);
 }
 
-// Full element evaluation.  prm = [uw(K) | uh(K) | ud(K-1)] (destroyed).
+// Full element evaluation.  prm = [uw(K) | uh(K) | ud(K-1 or K+1)] (destroyed).
 // Domain [left, right] -> codomain [bottom, top]  (rational_quadratic_spline.py:55-64).
 //   inverse == false: out = f(x),      ld = log f'(x)
 //   inverse == true : out = f^-1(x),   ld = own_ld ? log (f^-1)'(x) : -log f'(out)
 // Identity (ld 0) outside the active box  (rational_quadratic_spline.py:71,86-87).
-template <class P>
+template <class P, class O = RqsDefaults>
 __device__ __forceinline__ void rqs_element(P prm, int K, float left, float right, float bottom,
                                             float top, bool inverse, bool own_ld, float x,
-                                            float& out, float& ld, int* kbin = nullptr) {
+                                            float& out, float& ld, int* kbin = nullptr,
+                                            const O& o = O()) {
     out = x;
     ld = 0.f;
     if (kbin) *kbin = -1;                     // identity tail: no search happens (:86-91)
     const float lo = inverse ? bottom : left, hi = inverse ? top : right;
     if (!(x >= lo && x <= hi)) return;
     OffsetView<P> W{prm, 0}, H{prm, K}, D{prm, 2 * K};
-    softmax_bins(W, K, STB_RQS_MIN);
-    softmax_bins(H, K, STB_RQS_MIN);
+    softmax_bins(W, K, o.min_w());
+    softmax_bins(H, K, o.min_h());
     sizes_to_knots(W, K, left, right);
     sizes_to_knots(H, K, bottom, top);
     if (!inverse) {
         int k = knot_search(W, K, left, x);
         if (kbin) *kbin = k;
-        RqsBin b = rqs_bin(W, H, D, K, k, left, bottom);
+        RqsBin b = rqs_bin(W, H, D, K, k, left, bottom, o);
         rqs_forward_in_bin(b, x, out, ld);
     } else {
         int k = knot_search(H, K, bottom, x);
         if (kbin) *kbin = k;
-        RqsBin b = rqs_bin(W, H, D, K, k, left, bottom);
+        RqsBin b = rqs_bin(W, H, D, K, k, left, bottom, o);
         float ld_own;
         rqs_inverse_in_bin(b, x, out, ld_own);
         if (own_ld) {
@@ -209,7 +278,7 @@ __device__ __forceinline__ void rqs_element(P prm, int K, float left, float righ
             ld = 0.f;
             if (out >= left && out <= right) {
                 int k2 = knot_search(W, K, left, out);
-                RqsBin b2 = (k2 == k) ? b : rqs_bin(W, H, D, K, k2, left, bottom);
+                RqsBin b2 = (k2 == k) ? b : rqs_bin(W, H, D, K, k2, left, bottom, o);
                 float y2, ldf;
                 rqs_forward_in_bin(b2, out, y2, ldf);
                 ld = -ldf;
@@ -221,10 +290,6 @@ __device__ __forceinline__ void rqs_element(P prm, int K, float left, float righ
 // ---------------------------------------------------------------------------------------
 // cubic spline
 // ---------------------------------------------------------------------------------------
-#define STB_CUB_MIN 1e-2f
-#define STB_CUB_EPS 1e-5f
-#define STB_CUB_QUAD 1e-3f
-
 __device__ __forceinline__ float sign_f(float v) { return (v > 0.f) ? 1.f : ((v < 0.f) ? -1.f : 0.f); }
 // cubic_spline.py:18-20
 __device__ __forceinline__ float cbrt_ref(float v) { return sign_f(v) * expf(logf(fabsf(v)) / 3.0f); }
@@ -294,7 +359,8 @@ __device__ __forceinline__ float cubic_forward_in_bin(const CubBin& b, float u, 
 }
 
 // cubic_spline.py:153-228
-__device__ __forceinline__ float cubic_inverse_in_bin(const CubBin& k, float u, float& ld) {
+template <class O = CubDefaults>
+__device__ __forceinline__ float cubic_inverse_in_bin(const CubBin& k, float u, float& ld, const O& o = O()) {
     float b_ = (k.b / k.a) / 3.f;
     float c_ = (k.c / k.a) / 3.f;
     float d_ = (k.d - u) / k.a;
@@ -313,7 +379,7 @@ __device__ __forceinline__ float cubic_inverse_in_bin(const CubBin& k, float u, 
         float r1 = c1 * scale + shift;
         float r2 = (-0.5f * c1 - 0.5f * 1.7320508075688772f * c2) * scale + shift;
         float r3 = (-0.5f * c1 + 0.5f * 1.7320508075688772f * c2) * scale + shift;
-        float lo = k.xl - STB_CUB_EPS, hi = k.xr + STB_CUB_EPS;
+        float lo = k.xl - o.eps(), hi = k.xr + o.eps();
         bool ok1 = (lo < r1) && (r1 < hi), ok2 = (lo < r2) && (r2 < hi), ok3 = (lo < r3) && (r3 < hi);
         out = ok1 ? r1 : (ok2 ? r2 : (ok3 ? r3 : r1));      // argsort(masks, desc)[..., 0]  (:212)
     } else {
@@ -322,7 +388,7 @@ __device__ __forceinline__ float cubic_inverse_in_bin(const CubBin& k, float u, 
         float q = cbrt_ref((-dep_1 - sq) / 2.f);
         out = (p + q) - b_ + k.xl;
     }
-    if (fabsf(k.a) < STB_CUB_QUAD) {                         // :217-223
+    if (fabsf(k.a) < o.quad()) {                             // :217-223
         float qc = k.d - u;
         float alpha = (-k.c + sqrtf(k.c * k.c - 4.f * k.b * qc)) / (2.f * k.b);
         out = alpha + k.xl;
@@ -333,18 +399,18 @@ __device__ __forceinline__ float cubic_inverse_in_bin(const CubBin& k, float u, 
 }
 
 // prm = [uw(K) | uh(K) | left, right]  (destroyed).  Same contract as rqs_element.
-template <class P>
+template <class P, class O = CubDefaults>
 __device__ __forceinline__ void cubic_element(P prm, int K, float lower, float upper, bool inverse,
                                               bool own_ld, float x, float& out, float& ld,
-                                              int* kbin = nullptr) {
+                                              int* kbin = nullptr, const O& o = O()) {
     out = x;
     ld = 0.f;
     if (kbin) *kbin = -1;
     if (!(x >= lower && x <= upper)) return;
     OffsetView<P> W{prm, 0}, H{prm, K};
     const float ul = prm[2 * K], ur = prm[2 * K + 1];
-    softmax_bins(W, K, STB_CUB_MIN);
-    softmax_bins(H, K, STB_CUB_MIN);
+    softmax_bins(W, K, o.min_w());
+    softmax_bins(H, K, o.min_h());
     const float span = upper - lower;
     float u = (x - lower) / span;                            // :99-102
     float cw, ch;
@@ -352,15 +418,15 @@ __device__ __forceinline__ void cubic_element(P prm, int K, float lower, float u
         int k = cubic_search(W, H, K, false, u, cw, ch);
         if (kbin) *kbin = k;
         CubBin b = cubic_bin(W, H, K, k, cw, ch, ul, ur);
-        float o = cubic_forward_in_bin(b, u, ld);
-        out = o * span + lower;                              // :244-245 (log terms cancel: same box)
+        float v = cubic_forward_in_bin(b, u, ld);
+        out = v * span + lower;                              // :244-245 (log terms cancel: same box)
     } else {
         int k = cubic_search(W, H, K, true, u, cw, ch);
         if (kbin) *kbin = k;
         CubBin b = cubic_bin(W, H, K, k, cw, ch, ul, ur);
         float ld_own;
-        float o = cubic_inverse_in_bin(b, u, ld_own);
-        out = o * span + lower;
+        float v = cubic_inverse_in_bin(b, u, ld_own, o);
+        out = v * span + lower;
         if (own_ld) {
             ld = ld_own;
         } else {

@@ -707,6 +707,7 @@ bool tch_layer_supported(const stb_layer* L) {
     if (L->kind != STB_RQS && L->kind != STB_CUBIC) return false;
     if (L->n_bins < 2 || L->n_bins > kBins || !L->cond_x || L->zero_cond || L->latent_dim < 0 || L->time_input) return false;
     if (L->has_box || L->row_out || L->dim < 2 || L->dim > kMaxDim || L->inverse_ldj_own) return false;
+    if (L->spline.custom) return false;                    // non-default spline constants: CUDA-core kernels only
     const stb_mlp& N = L->net;
     if ((N.n_linear != 2 && N.n_linear != 3) || N.final_activation != STB_ACT_NONE) return false;
     const int H = N.dims[1];

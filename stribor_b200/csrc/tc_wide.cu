@@ -1458,6 +1458,7 @@ bool tcw_layer_supported(const stb_layer* L) {
     if (L->kind != STB_RQS && L->kind != STB_CUBIC) return false;
     if (L->n_bins < 2 || L->n_bins > kBins || !L->cond_x || L->zero_cond || L->latent_dim < 0 || L->time_input) return false;
     if (L->has_box || L->row_out || L->dim < 2 || L->dim > kMaxDim) return false;
+    if (L->spline.custom) return false;                    // non-default spline constants: CUDA-core kernels only
     const stb_mlp& N = L->net;
     if (N.n_linear != 2 || N.dims[1] != kHid || N.final_activation != STB_ACT_NONE) return false;
     // The hidden activations feed the next GEMM as fp16 hi | lo parts: only activations bounded by 1 are safe

@@ -19,6 +19,10 @@ def cubic_spline_latent_dim(dim: int, n_bins: int) -> int:
     return dim * (2 * n_bins + 2)
 
 
+RQS_DEFAULTS = (1e-3, 1e-3, 1e-3)             # min_bin_width, min_bin_height, min_derivative
+CUBIC_DEFAULTS = (1e-2, 1e-2, 1e-5, 1e-3)      # min_bin_width, min_bin_height, eps, quadratic_threshold
+
+
 def _row_params_call(kind, inputs, pieces, n_bins, inverse, fmeta, has_box):
     _ops._check_cuda(inputs, 'inputs')
     shape = inputs.shape
@@ -35,13 +39,17 @@ def unconstrained_rational_quadratic_spline(inputs, unnorm_widths, unnorm_height
                                             inverse=False, lower=-1., upper=1., left=None, right=None,
                                             bottom=None, top=None, min_bin_width=1e-3,
                                             min_bin_height=1e-3, min_derivative=1e-3):
-    """(outputs, log-Jacobian diagonal), identity outside the box.  Derivatives must have
-    ``n_bins - 1`` entries (boundary derivatives fixed to 1) and the minimums their defaults."""
+    """(outputs, log-Jacobian diagonal), identity outside the box.  ``unnorm_derivatives`` has
+    ``n_bins - 1`` entries (boundary derivatives fixed to 1) or ``n_bins + 1`` (boundary derivatives
+    free).  Widths are ``min_bin_width + (1 - min_bin_width * n_bins) * softmax`` (heights alike),
+    derivatives ``min_derivative + softplus``; ``min_bin_width * n_bins > 1`` raises ValueError."""
     K = unnorm_widths.shape[-1]
-    if (min_bin_width, min_bin_height, min_derivative) != (1e-3, 1e-3, 1e-3):
-        raise NotImplementedError('only the default minimum bin sizes / derivative are built')
-    if unnorm_derivatives.shape[-1] != K - 1:
-        raise NotImplementedError('boundary derivatives are fixed to 1 (K-1 derivative parameters)')
+    n_der = unnorm_derivatives.shape[-1]
+    if n_der not in (K - 1, K + 1):
+        raise ValueError(f'unnorm_derivatives must have n_bins - 1 = {K - 1} or n_bins + 1 = {K + 1} '
+                         f'entries, got {n_der}')
+    free_edge = n_der == K + 1
+    mins = (float(min_bin_width), float(min_bin_height), float(min_derivative))
     has_box = all(v is not None for v in (left, right, bottom, top))
     if has_box and any(torch.is_tensor(v) for v in (left, right, bottom, top)):
         raise NotImplementedError('tensor-valued boxes are not built')
@@ -49,6 +57,8 @@ def unconstrained_rational_quadratic_spline(inputs, unnorm_widths, unnorm_height
         left = bottom = lower
         right = top = upper
     fmeta = [float(lower), float(upper), float(left), float(right), float(bottom), float(top)]
+    if free_edge or mins != RQS_DEFAULTS:
+        fmeta += [1., *mins, float(free_edge), 0., 0.]
     return _row_params_call(_lib.RQS, inputs, [unnorm_widths, unnorm_heights, unnorm_derivatives], K,
                             inverse, fmeta, has_box)
 
@@ -58,9 +68,10 @@ def unconstrained_cubic_spline(inputs, unnormalized_widths, unnormalized_heights
                                min_bin_height=1e-2, eps=1e-5, quadratic_threshold=1e-3):
     if tails != 'linear':
         raise RuntimeError('{} tails are not implemented.'.format(tails))
-    if (min_bin_width, min_bin_height, eps, quadratic_threshold) != (1e-2, 1e-2, 1e-5, 1e-3):
-        raise NotImplementedError('only the default cubic-spline constants are built')
+    consts = (float(min_bin_width), float(min_bin_height), float(eps), float(quadratic_threshold))
     K = unnormalized_widths.shape[-1]
     fmeta = [float(lower), float(upper)] * 3
+    if consts != CUBIC_DEFAULTS:
+        fmeta += [1., consts[0], consts[1], 0., 0., consts[2], consts[3]]
     return _row_params_call(_lib.CUBIC, inputs, [unnormalized_widths, unnormalized_heights,
                                                  unnorm_derivatives], K, inverse, fmeta, False)
