@@ -30,10 +30,6 @@ struct BwdArgs {
     long long rows;
 };
 
-__host__ __device__ inline int bwd_params_per_dim(int kind, int K) {
-    return kind == STB_RQS ? 3 * K - 1 : (kind == STB_CUBIC ? 2 * K + 2 : 2);
-}
-
 // index of parameter p of the it-th transformed dim (original dim j) in the network output
 __device__ __forceinline__ int bwd_col(const stb_layer& L, int P, int n_tr, int it, int j, int p) {
     const bool aff = (L.kind == STB_AFFINE || L.kind == STB_CONT_AFFINE);
@@ -200,7 +196,8 @@ int layer_backward(const stb_layer* L, int direction, const float* x, const floa
         // conditioner fused: recompute it on the tensor cores, differentiate the spline in registers
         // (tc_wide.cu).  Outputs: g_x, grads->g_row_out = gradient wrt the network output of the
         // transformed dims [rows, n_tr * 48], workspace = augmented hidden activations [rows, 72].
-        if (!(L->packed && tcw_backward_supported(L) && tcw_image_present(L)))
+        const void* image = (L->packed && tcw_backward_supported(L)) ? tcw_image(L) : nullptr;
+        if (!image)
             return set_error(STB_ENOTSUP, "fused conditioner backward needs the tensor-core path (quadratic spline, 16 bins, MLP[64], packed): run the MLP through autograd and pass its output as row_out");
         if (direction != STB_FORWARD && direction != STB_INVERSE) return set_error(STB_EINVAL, "bad direction");
         if (rows < 0 || !x || !g_out || !g_x || !workspace) return set_error(STB_EINVAL, "bad argument");
@@ -212,9 +209,9 @@ int layer_backward(const stb_layer* L, int direction, const float* x, const floa
             //     conditioning slots [64 hidden, 64 slots], then gb_first [64]; all ACCUMULATED (caller zeroes)
             //   grads != NULL (g_row_out == NULL): workspace[0 : rows * 64] = g_pre and the image; the first
             //     Linear's three K = 64 products are left to the caller
-            return tcw_layer_backward_fused(L, tcw_image(L), direction, x, g_out, g_ldj, g_x,
+            return tcw_layer_backward_fused(L, image, direction, x, g_out, g_ldj, g_x,
                                             static_cast<float*>(workspace), grads == nullptr, rows, stream);
-        return tcw_layer_backward(L, tcw_image(L), direction, x, g_out, g_ldj, g_x, grads->g_row_out,
+        return tcw_layer_backward(L, image, direction, x, g_out, g_ldj, g_x, grads->g_row_out,
                                   static_cast<float*>(workspace), rows, stream);
     }
     if (L->kind == STB_CONT_AFFINE) return set_error(STB_ENOTSUP, "continuous-affine backward is not built yet");
@@ -228,7 +225,7 @@ int layer_backward(const stb_layer* L, int direction, const float* x, const floa
     BwdArgs A;
     A.L.set(L);
     A.direction = direction;
-    A.P = bwd_params_per_dim(L->kind, L->n_bins) + (custom && L->kind == STB_RQS && L->spline.free_edge_derivs ? 2 : 0);
+    A.P = spline_params_per_dim(L->kind, L->n_bins) + (custom && L->kind == STB_RQS && L->spline.free_edge_derivs ? 2 : 0);
     int n_tr = L->dim;
     if (L->cond_x && L->mask_host) {
         n_tr = 0;

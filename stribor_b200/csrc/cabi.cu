@@ -28,6 +28,28 @@ int sm_count() {
     return n_sm;
 }
 
+int layer_images(const stb_layer* L, PackedImage img[2]) {
+    int n = 0;
+    uint64_t off = 0;
+    auto add = [&](int family, uint64_t bytes) { img[n++] = PackedImage{family, off, bytes}; off += bytes; };
+    if (tc_layer_supported(L)) {
+        add(IMG_TC, tc_packed_bytes(L));
+        if (tcw_layer_supported(L)) add(IMG_TCW, tcw_packed_bytes(L));
+    } else if (tcw_layer_supported(L)) add(IMG_TCW, tcw_packed_bytes(L));
+    else if (tch_layer_supported(L)) add(IMG_TCH, tch_packed_bytes(L));
+    else if (tcm_layer_supported(L)) add(IMG_TCM, tcm_packed_bytes(L));
+    return n;
+}
+
+const void* tcw_image(const stb_layer* L) {
+    PackedImage img[2];
+    const int n = layer_images(L, img);
+    for (int i = 0; i < n; ++i)
+        if (img[i].family == IMG_TCW && L->packed && L->packed_bytes >= img[i].offset + img[i].bytes)
+            return static_cast<const uint8_t*>(L->packed) + img[i].offset;
+    return nullptr;
+}
+
 static int apply_one(const stb_layer* L, int direction, const float* x, const float* latent,
                      const float* t, float* y, float* ldj, int ldj_mode, int base_lp, int64_t rows,
                      cudaStream_t s, float* ldiag = nullptr, int32_t* bins = nullptr) {
@@ -50,8 +72,9 @@ static int apply_one(const stb_layer* L, int direction, const float* x, const fl
     if (ldj_mode != STB_LDJ_NONE && !ldj) return set_error(STB_EINVAL, "ldj_mode set but ldj is NULL");
     if (L->packed && !ldiag && tc_layer_supported(L) && !(bins && L->n_bins != 16))
         return tc_layer_apply(L, direction, x, latent, y, ldj, ldj_mode, base_lp, rows, s, bins);
-    if (L->packed && !ldiag && tcw_layer_supported(L) && tcw_image_present(L))
-        return tcw_layer_apply(L, tcw_image(L), direction, x, latent, y, ldj, ldj_mode, base_lp, rows, s, bins);
+    const void* wide = (L->packed && !ldiag) ? tcw_image(L) : nullptr;
+    if (wide)
+        return tcw_layer_apply(L, wide, direction, x, latent, y, ldj, ldj_mode, base_lp, rows, s, bins);
     if (L->packed && !ldiag && tch_layer_supported(L))
         return tch_layer_apply(L, direction, x, latent, y, ldj, ldj_mode, base_lp, rows, s, bins);
     if (L->packed && !ldiag && tcm_layer_supported(L))
@@ -274,33 +297,35 @@ int stb_layer_backward_diag(const stb_layer* layer, int direction, const float* 
 
 uint64_t stb_packed_bytes(const stb_layer* layer) {
     if (validate_layer(layer)) return 0;
-    if (tc_layer_supported(layer))                                                            // both images
-        return tc_packed_bytes(layer) + (tcw_layer_supported(layer) ? tcw_packed_bytes(layer) : 0);
-    if (tcw_layer_supported(layer)) return tcw_packed_bytes(layer);
-    if (tch_layer_supported(layer)) return tch_packed_bytes(layer);
-    return tcm_layer_supported(layer) ? tcm_packed_bytes(layer) : 0;
+    PackedImage img[2];
+    const int n = layer_images(layer, img);
+    return n ? img[n - 1].offset + img[n - 1].bytes : 0;
 }
 
 int stb_pack_layer(const stb_layer* layer, void* packed_out, void* stream) {
     int rc = validate_layer(layer);
     if (rc) return rc;
     if (!packed_out) return set_error(STB_EINVAL, "packed_out is NULL");
-    if (tc_layer_supported(layer)) {
-        // the 256-row inference kernel's image, then the 128-row / backward kernel's (tc_wide.cu)
-        rc = tc_pack_layer(layer, packed_out, (cudaStream_t)stream);
-        if (rc || !tcw_layer_supported(layer)) return rc;          // (`latent=` layers: inference image only)
-        return tcw_pack_layer(layer, static_cast<uint8_t*>(packed_out) + tc_packed_bytes(layer), (cudaStream_t)stream);
+    PackedImage img[2];
+    const int n = layer_images(layer, img);
+    if (n == 0) return set_error(STB_ENOTSUP, "layer has no tensor-core path");
+    for (int i = 0; i < n && rc == 0; ++i) {
+        void* out = static_cast<uint8_t*>(packed_out) + img[i].offset;
+        const cudaStream_t s = (cudaStream_t)stream;
+        switch (img[i].family) {
+            case IMG_TC: rc = tc_pack_layer(layer, out, s); break;
+            case IMG_TCW: rc = tcw_pack_layer(layer, out, s); break;
+            case IMG_TCH: rc = tch_pack_layer(layer, out, s); break;
+            default: rc = tcm_pack_layer(layer, out, s); break;
+        }
     }
-    if (tcw_layer_supported(layer)) return tcw_pack_layer(layer, packed_out, (cudaStream_t)stream);
-    if (tch_layer_supported(layer)) return tch_pack_layer(layer, packed_out, (cudaStream_t)stream);
-    if (tcm_layer_supported(layer)) return tcm_pack_layer(layer, packed_out, (cudaStream_t)stream);
-    return set_error(STB_ENOTSUP, "layer has no tensor-core path");
+    return rc;
 }
 
 int stb_layer_uses_tensor_path(const stb_layer* layer) {
     if (validate_layer(layer)) return 0;
-    return (layer->packed && (tc_layer_supported(layer) || tcw_layer_supported(layer) || tch_layer_supported(layer) ||
-                              tcm_layer_supported(layer))) ? 1 : 0;
+    PackedImage img[2];
+    return (layer->packed && layer_images(layer, img) > 0) ? 1 : 0;
 }
 
 }  // extern "C"

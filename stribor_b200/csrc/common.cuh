@@ -25,6 +25,11 @@ int sm_count();
 
 int validate_layer(const stb_layer* L);
 
+// network outputs per transformed dim: rqs 3K - 1, cubic 2K + 2, affine kinds 2 (log-scale, shift)
+__host__ __device__ inline int spline_params_per_dim(int kind, int K) {
+    return kind == STB_RQS ? 3 * K - 1 : (kind == STB_CUBIC ? 2 * K + 2 : 2);
+}
+
 int generic_layer_apply(const stb_layer* L, int direction, const float* x, const float* latent,
                         const float* t, float* y, float* ldj, int ldj_mode, int base_log_prob,
                         float* ldiag, int64_t rows, cudaStream_t stream, int32_t* bins = nullptr);
@@ -55,8 +60,7 @@ int tc_chain_apply(const stb_layer* const* layers, int n, int direction, const f
                    float* ldj, int ldj_mode, int base_log_prob, int64_t rows, cudaStream_t stream,
                    const ChainPerm* perm = nullptr);
 
-// tcgen05 path for dim <= 128 and the training backward (tc_wide.cu).  `image` is the wide packed image:
-// it follows the tc_layer.cu image when the layer has both (tcw_image).
+// tcgen05 path for dim <= 128 and the training backward (tc_wide.cu).  `image` is the wide packed image (tcw_image).
 bool tcw_layer_supported(const stb_layer* L);
 bool tcw_backward_supported(const stb_layer* L);
 uint64_t tcw_packed_bytes(const stb_layer* L);
@@ -71,12 +75,8 @@ uint64_t tcw_train_workspace_floats(const stb_layer* L, int64_t rows);
 int tcw_layer_backward_fused(const stb_layer* L, const void* image, int direction, const float* x, const float* g_out,
                              const float* g_ldj, float* g_x, float* workspace, int first_linear, int64_t rows,
                              cudaStream_t stream);
-inline const void* tcw_image(const stb_layer* L) {
-    return static_cast<const uint8_t*>(L->packed) + (tc_layer_supported(L) ? tc_packed_bytes(L) : 0);
-}
-inline bool tcw_image_present(const stb_layer* L) {
-    return L->packed && L->packed_bytes >= (tc_layer_supported(L) ? tc_packed_bytes(L) : 0) + tcw_packed_bytes(L);
-}
+// the layer's wide image (layer_images), NULL when it has none or `packed` is too small to hold it
+const void* tcw_image(const stb_layer* L);
 
 // tcgen05 path for spline couplings with a wide conditioner, MLP[H] / MLP[H,H], H <= 256 (tc_hwide.cu)
 bool tch_layer_supported(const stb_layer* L);
@@ -97,6 +97,12 @@ bool tcm_chain_supported(const stb_layer* const* layers, int n);
 int tcm_chain_apply(const stb_layer* const* layers, int n, int direction, const float* x, const float* t, float* y,
                     float* ldj, int ldj_mode, int base_log_prob, int64_t rows, cudaStream_t stream,
                     const ChainPerm* perm = nullptr);
+
+// The packed images of a layer (stb_pack_layer), in the order they sit in stb_layer.packed: an MLP[64] spline layer
+// that fits tc_layer.cu carries that image and then the tc_wide.cu one.  Returns how many (0 .. 2).  (cabi.cu)
+enum { IMG_TC, IMG_TCW, IMG_TCH, IMG_TCM };
+struct PackedImage { int family; uint64_t offset, bytes; };
+int layer_images(const stb_layer* L, PackedImage img[2]);
 
 // backward (backward.cu)
 uint64_t layer_backward_workspace_bytes(const stb_layer* L, int64_t rows);

@@ -41,14 +41,10 @@ struct GenArgs {
     long long rows;
 };
 
-__host__ __device__ inline int params_per_dim(int kind, int K) {
-    return kind == STB_RQS ? 3 * K - 1 : (kind == STB_CUBIC ? 2 * K + 2 : 2);
-}
-
-// the same, with the two free boundary derivatives of an rqs layer that asks for them
+// spline_params_per_dim, with the two free boundary derivatives of an rqs layer that asks for them
 inline int layer_params_per_dim(const stb_layer* L) {
     const bool free_edge = L->kind == STB_RQS && L->spline.custom && L->spline.free_edge_derivs;
-    return params_per_dim(L->kind, L->n_bins) + (free_edge ? 2 : 0);
+    return spline_params_per_dim(L->kind, L->n_bins) + (free_edge ? 2 : 0);
 }
 
 // row of the conditioner output holding parameter p of dim j

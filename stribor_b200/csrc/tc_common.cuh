@@ -1,6 +1,7 @@
 // sm_100a building blocks used by the tensor-core path: mbarrier, bulk async copy (TMA
-// engine, 1-D), tcgen05 (TMEM allocation, UMMA issue / commit, TMEM loads) and the shared-
-// memory matrix descriptors.  Everything is inline PTX; nothing here exists on older parts.
+// engine, 1-D), tcgen05 (TMEM allocation, UMMA issue / commit, TMEM loads), the shared-
+// memory matrix descriptors, named barriers, MUFU-based exp2 / division and the precision
+// splits.  Everything is inline PTX; nothing here exists on older parts.
 //
 // Operand layout (both A and B are K-major, SWIZZLE_NONE "interleaved" canonical layout):
 // a matrix of R rows x K elements is stored as 8-row x 16-byte core matrices,
@@ -257,6 +258,31 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(
                      smem_u32(bar))
                  : "memory");
+}
+
+// ---- arithmetic ---------------------------------------------------------------------------------
+__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
+    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+// exp through ex2.approx.  In the spline softmaxes, with the maximum subtracted, the arguments are <= 0, so the absolute
+// error of every term is <= ~2.5 ulp of the LARGEST term (= 1), i.e. the same absolute accuracy on
+// the bin sizes as a 2-ulp expf.  Measured on the GPU against the fp64 oracle
+// (profiles/r01_tc_accuracy.txt): accurate expf, IEEE division and a true e_i / sum quotient change
+// the mean log-det error by < 7 %; only compensated cumulative sums help (12 %) and cost ~90
+// instructions per element.
+__device__ __forceinline__ float ex2_approx(float v) {
+    float r;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(v));
+    return r;
+}
+
+// a / b to ~1 ulp: MUFU.RCP + one residual correction (4 instructions instead of ~10 for the
+// IEEE sequence; the operands here are never subnormal / huge)
+__device__ __forceinline__ float fdiv(float a, float b) {
+    float r;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(b));
+    const float q = a * r;
+    return fmaf(fmaf(-q, b, a), r, q);
 }
 
 // ---- precision splits -----------------------------------------------------------------------------

@@ -25,6 +25,7 @@
 #include "common.cuh"
 #include "stb_math.cuh"
 #include "tc_common.cuh"
+#include "tc_pack.cuh"
 #include "tc_spline16.cuh"
 
 namespace stb {
@@ -111,10 +112,6 @@ struct Args {
     long long rows;
     int n_tiles;
 };
-
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
 
 // two hidden units: activation of (acc * sc + bias), fp16 hi | lo parts packed for the TMEM A operand
 template <bool TANH>
@@ -538,31 +535,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_hw_spline_kernel(const Args A)
 struct PackArgs {
     const float *W1, *b1, *W2, *b2, *W3, *b3;
     uint8_t* out;
-    int kind, dim, n_cond, n_tr, H, n_hidden, P, act, n_lat, n_bins;
-    int cond_idx[kK1];
-    int tr_idx[kMaxTr];
+    int kind, dim, H, n_hidden, P, act, n_lat, n_bins;
+    MaskSplit m;
 };
-
-// column c of a dim's 48 -> parameter index: the 32 softmax columns are interleaved (w_i, h_i)
-// -> parameter index in the network's [w(K) | h(K) | rest] order, -1 for padding (as tc_layer.cu)
-__host__ __device__ __forceinline__ int param_of_col(int c, int K, int P) {
-    if (c < 2 * kBins) {
-        const int i = c >> 1;
-        return (i < K) ? ((c & 1) ? K + i : i) : -1;
-    }
-    const int p = 2 * K + (c - 2 * kBins);
-    return (p < P) ? p : -1;
-}
-// element (n, k) of an [N x 16] K-major block: 2 chunks of 8 elements per row
-__device__ __forceinline__ uint32_t blk_off(int n, int k) {
-    return (uint32_t)((n >> 3) * 256 + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2);
-}
-__device__ __forceinline__ float pow2_scale(float mx) {
-    if (!(mx > 0.f) || !isfinite(mx)) return 1.f;
-    int ex;
-    const float fr = frexpf(mx, &ex);
-    return ldexpf(1.f, (fr == 0.5f) ? ex - 1 : ex);
-}
 
 __global__ void tch_maxabs_kernel(const PackArgs a) {
     Header* hdr = reinterpret_cast<Header*>(a.out);
@@ -570,20 +545,13 @@ __global__ void tch_maxabs_kernel(const PackArgs a) {
     const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
     if (a.n_hidden == 2)
         for (int i = gtid; i < a.H * a.H; i += gsz) m2 = fmaxf(m2, fabsf(a.W2[i]));
-    const int total = a.n_tr * a.P * a.H;
+    const int total = a.m.n_tr * a.P * a.H;
     for (int i = gtid; i < total; i += gsz) {
         const int k = i % a.H, rp = i / a.H, p = rp % a.P, ji = rp / a.P;
-        m3 = fmaxf(m3, fabsf(a.W3[((size_t)a.tr_idx[ji] * a.P + p) * a.H + k]));
+        m3 = fmaxf(m3, fabsf(a.W3[((size_t)a.m.tr_idx[ji] * a.P + p) * a.H + k]));
     }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) {
-        m2 = fmaxf(m2, __shfl_xor_sync(0xffffffffu, m2, o));
-        m3 = fmaxf(m3, __shfl_xor_sync(0xffffffffu, m3, o));
-    }
-    if ((threadIdx.x & 31) == 0) {
-        atomicMax(&hdr->max_mid, __float_as_uint(m2));
-        atomicMax(&hdr->max_out, __float_as_uint(m3));
-    }
+    warp_max_to(&hdr->max_mid, m2);
+    warp_max_to(&hdr->max_out, m3);
 }
 
 __global__ void tch_pack_kernel(const PackArgs a) {
@@ -592,49 +560,25 @@ __global__ void tch_pack_kernel(const PackArgs a) {
     const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
     const int H = a.H;
     if (gtid == 0) {
-        hdr->magic = kMagic; hdr->kind = a.kind; hdr->dim = a.dim; hdr->n_cond = a.n_cond; hdr->n_tr = a.n_tr; hdr->H = H;
+        hdr->magic = kMagic; hdr->kind = a.kind; hdr->dim = a.dim; hdr->n_cond = a.m.n_cond; hdr->n_tr = a.m.n_tr; hdr->H = H;
         hdr->n_hidden = a.n_hidden; hdr->P = a.P; hdr->act = a.act; hdr->s_mid = s_mid; hdr->s_out = s_out; hdr->n_lat = a.n_lat; hdr->n_bins = a.n_bins;
-        for (int i = 0; i < kK1; ++i) hdr->cond_idx[i] = a.cond_idx[i];
-        for (int i = 0; i < kMaxTr; ++i) hdr->tr_idx[i] = a.tr_idx[i];
+        for (int i = 0; i < kK1; ++i) hdr->cond_idx[i] = a.m.cond_idx[i];
+        for (int i = 0; i < kMaxTr; ++i) hdr->tr_idx[i] = a.m.tr_idx[i];
     }
     float* b1 = reinterpret_cast<float*>(a.out + kOffB1);
     float* b2 = reinterpret_cast<float*>(a.out + kOffB2);
-    float* b3 = reinterpret_cast<float*>(a.out + kOffB3);
     for (int i = gtid; i < kMaxH; i += gsz) {
         b1[i] = (i < H) ? a.b1[i] : 0.f;
         b2[i] = (i < H && a.n_hidden == 2) ? a.b2[i] : 0.f;
     }
-    for (int i = gtid; i < kMaxTr * kPPad; i += gsz) {
-        const int ji = i / kPPad, col = i % kPPad, p = param_of_col(col, a.n_bins, a.P);
-        float bv = (ji < a.n_tr && p >= 0) ? a.b3[a.tr_idx[ji] * a.P + p] : 0.f;
-        if (col < 2 * kBins && p < 0 && ji < a.n_tr) bv = -INFINITY;         // padded bin: numerator exactly 0
-        b3[i] = (col < 2 * kBins) ? bv * 1.4426950408889634f : bv;         // softmax columns: log2 domain
-    }
-    // first Linear: blocks (pb = 2, 1, 0) x (kb = 0, 1), each [H x 16] of bf16 part pb (conditioning columns only)
-    uint8_t* w = a.out + kOffW;
+    fill_spline_bias(reinterpret_cast<float*>(a.out + kOffB3), kMaxTr, a.b3, a.m, a.P, a.n_bins, gtid, gsz);
     for (int i = gtid; i < H * kK1; i += gsz) {
         const int n = i / kK1, k = i % kK1;
-        const size_t in1 = (size_t)(a.dim + a.n_lat);          // the first Linear reads [x * mask | latent]
-        const float v = (k < a.n_cond) ? a.W1[n * in1 + a.cond_idx[k]]
-                                       : ((k < a.n_cond + a.n_lat) ? a.W1[n * in1 + a.dim + (k - a.n_cond)] : 0.f);
-        __nv_bfloat16 qv[3];
-        split_bf16x3(v, qv[0], qv[1], qv[2]);
-        for (int pb = 0; pb < 3; ++pb) {
-            const int b = (2 - pb) * 2 + (k >> 4);
-            *reinterpret_cast<__nv_bfloat16*>(w + (size_t)b * w1_block(H) + blk_off(n, k & 15)) = qv[pb];
-        }
+        store_w1_blocks(a.out + kOffW, H, n, k, first_linear_w(a.W1, n, k, a.dim + a.n_lat, a.dim, a.m, -1, a.m.n_cond, a.n_lat));
     }
     if (a.n_hidden == 2) {
-        uint8_t* w2 = a.out + off_w2(H);
         const float inv = 1.f / s_mid;
-        for (int i = gtid; i < H * H; i += gsz) {
-            const int n = i / H, k = i % H;
-            __half hi, lo;
-            split_f16(a.W2[i] * inv, hi, lo);
-            uint8_t* blk = w2 + (size_t)(k >> 4) * w2_block(H);
-            *reinterpret_cast<__half*>(blk + blk_off(n, k & 15)) = hi;
-            *reinterpret_cast<__half*>(blk + H * 32 + blk_off(n, k & 15)) = lo;
-        }
+        for (int i = gtid; i < H * H; i += gsz) store_hilo_blocks(a.out + off_w2(H), H, i / H, i % H, a.W2[i] * inv);
     }
     {   // last Linear: per chunk of two transformed dims a lo item and a hi item
         uint8_t* w3 = a.out + off_w3(H, a.n_hidden);
@@ -644,7 +588,7 @@ __global__ void tch_pack_kernel(const PackArgs a) {
             const int ji = i / per_dim, rem = i % per_dim, n = rem / H, k = rem % H;
             const int p = param_of_col(n, a.n_bins, a.P);
             float v = 0.f;
-            if (ji < a.n_tr && p >= 0) v = a.W3[((size_t)a.tr_idx[ji] * a.P + p) * H + k] * inv;
+            if (ji < a.m.n_tr && p >= 0) v = a.W3[((size_t)a.m.tr_idx[ji] * a.P + p) * H + k] * inv;
             __half hi, lo;
             split_f16(v, hi, lo);
             // chunk c = ji / 2 (two dims, 96 rows): item 2c holds the lo parts, item 2c + 1 the hi parts, each as H / 16
@@ -657,66 +601,23 @@ __global__ void tch_pack_kernel(const PackArgs a) {
     }
 }
 
-// |logit_p| <= |b_p| + sum_k |W3[p][k]| for hidden activations bounded by 1: if <= 100 (log2 units) for all 32 softmax rows
-// of a dim, 2^logit neither overflows nor flushes and the kernel skips the max subtraction (as tc_layer.cu)
-__global__ void tch_bound_kernel(const PackArgs a) {
-    const int ji = threadIdx.x >> 5, p = threadIdx.x & 31;
-    bool ok = false;
-    if (ji < a.n_tr) {
-        ok = true;
-        if (p < 2 * a.n_bins) {                              // the 2 K softmax rows of the dim
-            const size_t rowi = (size_t)a.tr_idx[ji] * a.P + p;
-            float l1 = fabsf(a.b3[rowi]);
-            for (int k = 0; k < a.H; ++k) l1 += fabsf(a.W3[rowi * a.H + k]);
-            ok = (l1 * 1.4426950408889634f <= 100.f);
-        }
-    }
-    ok = __all_sync(0xffffffffu, ok);
-    if (p == 0 && ok) atomicOr(&reinterpret_cast<Header*>(a.out)->noshift_mask, 1u << ji);
-}
-
-static bool fill_pack_args(const stb_layer* L, PackArgs& a) {
-    if (!L->mask_host) return false;
-    a.n_cond = a.n_tr = 0;
-    for (int j = 0; j < L->dim; ++j) {
-        if (L->mask_host[j]) { if (a.n_cond >= kK1) return false; a.cond_idx[a.n_cond++] = j; }
-        else { if (a.n_tr >= kMaxTr) return false; a.tr_idx[a.n_tr++] = j; }
-    }
-    for (int i = a.n_cond; i < kK1; ++i) a.cond_idx[i] = 0;
-    for (int i = a.n_tr; i < kMaxTr; ++i) a.tr_idx[i] = 0;
-    if (a.n_tr < 1) return false;
+// the shared spline gate, then this file's conditioner: MLP[H] or MLP[H, H], H a multiple of 64 up to 256, not MLP[64]
+// (tc_layer.cu / tc_wide.cu)
+static_assert(kMaxTr == kK1, "spline_gate bounds the transformed dims by GEMM1's K");
+static bool admit(const stb_layer* L, MaskSplit& m) {
+    if (!spline_gate(L, kMaxDim, kK1, m)) return false;
     const stb_mlp& N = L->net;
-    a.n_lat = L->latent_dim;
-    if (a.n_cond + a.n_lat > kK1 || N.dims[0] != L->dim + a.n_lat) return false;
-    a.kind = L->kind; a.dim = L->dim; a.H = N.dims[1]; a.n_hidden = N.n_linear - 1;
-    a.n_bins = L->n_bins;
-    if (a.n_bins < 2 || a.n_bins > kBins) return false;
-    a.P = L->kind == STB_RQS ? 3 * a.n_bins - 1 : 2 * a.n_bins + 2;
-    if (N.dims[N.n_linear] != L->dim * a.P) return false;
-    a.act = N.activation;
-    a.W1 = N.W[0]; a.b1 = N.b[0];
-    a.W2 = a.n_hidden == 2 ? N.W[1] : nullptr; a.b2 = a.n_hidden == 2 ? N.b[1] : nullptr;
-    a.W3 = N.W[N.n_linear - 1]; a.b3 = N.b[N.n_linear - 1];
-    return true;
+    const int H = N.dims[1];
+    if (H < 64 || H > kMaxH || (H % 64) != 0) return false;
+    if (N.n_linear == 2 && H == 64) return false;
+    return N.n_linear == 2 || N.dims[2] == H;
 }
 
 }  // namespace tch
 
 bool tch_layer_supported(const stb_layer* L) {
-    using namespace tch;
-    if (L->kind != STB_RQS && L->kind != STB_CUBIC) return false;
-    if (L->n_bins < 2 || L->n_bins > kBins || !L->cond_x || L->zero_cond || L->latent_dim < 0 || L->time_input) return false;
-    if (L->has_box || L->row_out || L->dim < 2 || L->dim > kMaxDim || L->inverse_ldj_own) return false;
-    if (L->spline.custom) return false;                    // non-default spline constants: CUDA-core kernels only
-    const stb_mlp& N = L->net;
-    if ((N.n_linear != 2 && N.n_linear != 3) || N.final_activation != STB_ACT_NONE) return false;
-    const int H = N.dims[1];
-    if (H < 64 || H > kMaxH || (H % 64) != 0) return false;
-    if (N.n_linear == 2 && H == 64) return false;                 // MLP[64]: tc_layer.cu / tc_wide.cu
-    if (N.n_linear == 3 && N.dims[2] != H) return false;
-    if (N.activation != STB_ACT_TANH && N.activation != STB_ACT_SIGMOID) return false;    // bounded: fp16 hi | lo parts
-    PackArgs a;
-    return fill_pack_args(L, a);
+    tch::MaskSplit m;
+    return tch::admit(L, m);
 }
 
 uint64_t tch_packed_bytes(const stb_layer* L) { return tch::packed_bytes(L->net.dims[1], L->net.n_linear - 1); }
@@ -724,19 +625,21 @@ uint64_t tch_packed_bytes(const stb_layer* L) { return tch::packed_bytes(L->net.
 int tch_pack_layer(const stb_layer* L, void* out, cudaStream_t stream) {
     using namespace tch;
     PackArgs a;
-    if (!fill_pack_args(L, a)) return set_error(STB_ENOTSUP, "layer has no wide-conditioner tensor-core path");
+    if (!admit(L, a.m)) return set_error(STB_ENOTSUP, "layer has no wide-conditioner tensor-core path");
+    const stb_mlp& N = L->net;
     a.out = static_cast<uint8_t*>(out);
-    cudaError_t e = cudaMemsetAsync(out, 0, sizeof(Header), stream);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "memset: %s", cudaGetErrorString(e));
-    tch_maxabs_kernel<<<128, 256, 0, stream>>>(a);
-    count_launch();
-    tch_pack_kernel<<<592, 256, 0, stream>>>(a);
-    count_launch();
-    tch_bound_kernel<<<1, kMaxTr * 32, 0, stream>>>(a);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tch_pack launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    a.kind = L->kind; a.dim = L->dim; a.H = N.dims[1]; a.n_hidden = N.n_linear - 1; a.act = N.activation;
+    a.n_lat = L->latent_dim; a.n_bins = L->n_bins; a.P = spline_params_per_dim(L->kind, L->n_bins);
+    a.W1 = N.W[0]; a.b1 = N.b[0];
+    a.W2 = a.n_hidden == 2 ? N.W[1] : nullptr; a.b2 = a.n_hidden == 2 ? N.b[1] : nullptr;
+    a.W3 = N.W[N.n_linear - 1]; a.b3 = N.b[N.n_linear - 1];
+    const BoundArgs b = spline_bound_args(a.m, a.W3, a.b3, a.H, a.P, a.n_bins, a.act,
+                                          a.out + offsetof(Header, noshift_mask));
+    return pack_image(out, sizeof(Header), stream, "tch_pack", [&] {
+        pack_pass(tch_maxabs_kernel, 128, 256, stream, a);
+        pack_pass(tch_pack_kernel, 592, 256, stream, a);
+        pack_pass(tc_bound_kernel, 1, kMaxTr * 32, stream, b);
+    });
 }
 
 int tch_layer_apply(const stb_layer* L, int direction, const float* x, const float* latent, float* y, float* ldj,
@@ -756,26 +659,11 @@ int tch_layer_apply(const stb_layer* L, int direction, const float* x, const flo
     const long long tiles = (rows + kRows - 1) / kRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    const bool inv = direction == STB_INVERSE;
-    void (*kern)(Args);
-    if (L->n_bins == kBins) {
-        if (L->kind == STB_RQS) kern = inv ? tc_hw_spline_kernel<STB_RQS, true> : tc_hw_spline_kernel<STB_RQS, false>;
-        else kern = inv ? tc_hw_spline_kernel<STB_CUBIC, true> : tc_hw_spline_kernel<STB_CUBIC, false>;
-    } else {
-        if (L->kind == STB_RQS) kern = inv ? tc_hw_spline_kernel<STB_RQS, true, false> : tc_hw_spline_kernel<STB_RQS, false, false>;
-        else kern = inv ? tc_hw_spline_kernel<STB_CUBIC, true, false> : tc_hw_spline_kernel<STB_CUBIC, false, false>;
-    }
-    const uint32_t smem = smem_bytes(H);
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    void (*kern)(Args) = pick_variant(L->kind, direction == STB_INVERSE, L->n_bins == kBins,
+                                      [](auto K, auto I, auto F) { return tc_hw_spline_kernel<K, I, F>; });
     // one CTA per SM, each streaming its own weights: clusters of CTAs sharing one weight stream measured slower
     // (DESIGN.md 4.1f)
-    const int grid = (int)min((long long)sm_count(), tiles);
-    kern<<<grid, kThreads, smem, stream>>>(A);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_hw_spline_kernel launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    return launch_persistent(kern, A, tiles, 1, kThreads, smem_bytes(H), stream, "tc_hw_spline_kernel");
 }
 
 }  // namespace stb

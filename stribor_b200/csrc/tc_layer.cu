@@ -30,6 +30,7 @@
 #include "common.cuh"
 #include "stb_math.cuh"
 #include "tc_common.cuh"
+#include "tc_pack.cuh"
 #include "tc_spline16.cuh"
 
 namespace stb {
@@ -134,10 +135,6 @@ struct Args {
     int permuted;                      // CHAIN: permutations between the layers, folded into the index lists
     ChainPerm perm;
 };
-
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
 
 // -----------------------------------------------------------------------------------------------
 // the kernel
@@ -1004,202 +1001,58 @@ __global__ void __launch_bounds__(kPThreads, 2) tc_spline_pair_kernel(const Args
 // -----------------------------------------------------------------------------------------------
 // packing
 // -----------------------------------------------------------------------------------------------
-struct PackArgs {
-    const float *W1, *b1, *W2, *b2;
-    uint8_t* out;
-    int kind, dim, n_cond, n_tr, n_chunks, P, act, n_lat, n_bins;
-    int cond_idx[kK1];
-    int tr_idx[kMaxTr];
+// the image's layout for spline64_pack_kernel (tc_pack.cuh)
+struct PackLayout {
+    using Hdr = Header;
+    static constexpr uint32_t kMagic = tcl::kMagic, kOffB1 = tcl::kOffB1, kOffW1 = tcl::kOffW1;
+    static constexpr int kK1 = tcl::kK1, kMaxTr = tcl::kMaxTr;
+    static __device__ void header_extra(Header*, const SplinePackArgs&) {}
 };
 
-__global__ void tc_maxabs_kernel(const PackArgs a) {
-    float m = 0.f;
-    const int total = a.n_tr * a.P * kHid;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
-        const int k = i % kHid, rp = i / kHid, p = rp % a.P, ji = rp / a.P;
-        m = fmaxf(m, fabsf(a.W2[((size_t)a.tr_idx[ji] * a.P + p) * kHid + k]));
-    }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-    if ((threadIdx.x & 31) == 0) atomicMax(&reinterpret_cast<Header*>(a.out)->maxbits, __float_as_uint(m));
-}
-
-// column c of a dim's 48 -> parameter index in the network's [w(K) | h(K) | rest] order, -1 for padding: the 32
-// softmax columns are interleaved (w_i, h_i), i < 16; columns 32 .. 47 carry the K - 1 derivatives (cubic: the 2 end slopes)
-__host__ __device__ __forceinline__ int param_of_col(int c, int K, int P) {
-    if (c < 2 * kBins) {
-        const int i = c >> 1;
-        return (i < K) ? ((c & 1) ? K + i : i) : -1;
-    }
-    const int p = 2 * K + (c - 2 * kBins);
-    return (p < P) ? p : -1;
-}
-
-__device__ __forceinline__ uint32_t core_off(int r, int k, int K, int elem) {
-    const int epc = 16 / elem, chunks = K / epc;
-    return (uint32_t)((r >> 3) * (chunks * 128) + (k / epc) * 128 + (r & 7) * 16 + (k % epc) * elem);
-}
-
-__global__ void tc_pack_kernel(const PackArgs a) {
-    Header* hdr = reinterpret_cast<Header*>(a.out);
-    const float mx = __uint_as_float(hdr->maxbits);
-    // power of two >= max |W2|, so W2 / s2 is exact and within [-1, 1]
-    float s2 = 1.f;
-    if (mx > 0.f && isfinite(mx)) {
-        int ex;
-        const float fr = frexpf(mx, &ex);            // mx = fr * 2^ex, fr in [0.5, 1)
-        s2 = ldexpf(1.f, (fr == 0.5f) ? ex - 1 : ex);
-    }
-    const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
-    if (gtid == 0) {
-        hdr->magic = kMagic; hdr->kind = a.kind; hdr->dim = a.dim; hdr->n_cond = a.n_cond; hdr->n_tr = a.n_tr;
-        hdr->n_chunks = a.n_chunks; hdr->P = a.P; hdr->act = a.act; hdr->s2 = s2; hdr->n_lat = a.n_lat;
-        hdr->n_bins = a.n_bins;
-        for (int i = 0; i < kK1; ++i) hdr->cond_idx[i] = a.cond_idx[i];
-        for (int i = 0; i < kMaxTr; ++i) hdr->tr_idx[i] = a.tr_idx[i];
-    }
-    float* b1 = reinterpret_cast<float*>(a.out + kOffB1);
-    float* b2 = reinterpret_cast<float*>(a.out + kOffB2);
-    for (int i = gtid; i < kHid; i += gsz) b1[i] = a.b1[i];
-    for (int i = gtid; i < kMaxChunks * kChunkN; i += gsz) {
-        const int ji = i / kPPad, col = i % kPPad, p = param_of_col(col, a.n_bins, a.P);
-        float bv = (ji < a.n_tr && p >= 0) ? a.b2[a.tr_idx[ji] * a.P + p] : 0.f;
-        if (col < 2 * kBins && p < 0 && ji < a.n_tr) bv = -INFINITY;   // padded bin: numerator 2^-inf = 0 exactly
-        b2[i] = (col < 2 * kBins) ? bv * 1.4426950408889634f : bv;    // softmax columns: log2 domain
-    }
-    // first Linear, conditioning columns only: [64][32] as three bf16 parts
-    for (int i = gtid; i < kHid * kK1; i += gsz) {
-        const int n = i / kK1, k = i % kK1;
-        const size_t in1 = (size_t)(a.dim + a.n_lat);          // the first Linear reads [x * mask | latent]
-        const float v = (k < a.n_cond) ? a.W1[n * in1 + a.cond_idx[k]]
-                                       : ((k < a.n_cond + a.n_lat) ? a.W1[n * in1 + a.dim + (k - a.n_cond)] : 0.f);
-        __nv_bfloat16 q0, q1, q2;
-        split_bf16x3(v, q0, q1, q2);
-        const uint32_t off = kOffW1 + core_off(n, k, kK1, 2);
-        *reinterpret_cast<__nv_bfloat16*>(a.out + off) = q0;
-        *reinterpret_cast<__nv_bfloat16*>(a.out + off + kW1Part) = q1;
-        *reinterpret_cast<__nv_bfloat16*>(a.out + off + 2 * kW1Part) = q2;
-    }
-    // last Linear, rows of the transformed dims, padded to 48 per dim, 2 dims per chunk
-    const float inv = 1.f / s2;
-    for (int i = gtid; i < kMaxChunks * kChunkN * kHid; i += gsz) {
-        const int k = i % kHid, rn = i / kHid, n = rn % kChunkN, c = rn / kChunkN;
-        const int ji = c * kG + n / kPPad, p = param_of_col(n % kPPad, a.n_bins, a.P);
-        float v = 0.f;
-        if (c < a.n_chunks && ji < a.n_tr && p >= 0) v = a.W2[((size_t)a.tr_idx[ji] * a.P + p) * kHid + k] * inv;
-        __half hi, lo;
-        split_f16(v, hi, lo);
-        const uint32_t off = kOffW2 + (uint32_t)c * kChunkBytes + core_off(n, k, kHid, 2);
-        *reinterpret_cast<__half*>(a.out + off) = hi;
-        *reinterpret_cast<__half*>(a.out + off + 12288) = lo;
-    }
-}
-
-// One warp per transformed dim: |logit_p| <= |b_p| + sum_k |W2[p][k]| when the hidden activation is
-// bounded by 1 (tanh, sigmoid).  If that bound is <= 100 in log2 units for all 32 softmax rows of
-// the dim, 2^logit cannot overflow or flush to zero and the kernel skips the max subtraction.
-__global__ void tc_bound_kernel(const PackArgs a) {
-    const int ji = threadIdx.x >> 5, p = threadIdx.x & 31;
-    bool ok = false;
-    if (ji < a.n_tr && (a.act == STB_ACT_TANH || a.act == STB_ACT_SIGMOID)) {
-        ok = true;
-        if (p < 2 * a.n_bins) {                              // the 2 K softmax rows of the dim: [w(K) | h(K)]
-            const size_t row = (size_t)a.tr_idx[ji] * a.P + p;
-            float l1 = fabsf(a.b2[row]);
-            for (int k = 0; k < kHid; ++k) l1 += fabsf(a.W2[row * kHid + k]);
-            ok = (l1 * 1.4426950408889634f <= 100.f);        // false for NaN / inf
-        }
-    }
-    ok = __all_sync(0xffffffffu, ok);
-    if (p == 0 && ok) atomicOr(&reinterpret_cast<Header*>(a.out)->noshift_mask, 1u << ji);
-}
-
-static bool fill_pack_args(const stb_layer* L, PackArgs& a) {
-    if (!L->mask_host) return false;
-    a.n_cond = a.n_tr = 0;
-    for (int j = 0; j < L->dim; ++j) {
-        if (L->mask_host[j]) { if (a.n_cond >= kK1) return false; a.cond_idx[a.n_cond++] = j; }
-        else { if (a.n_tr >= kMaxTr) return false; a.tr_idx[a.n_tr++] = j; }
-    }
-    for (int i = a.n_cond; i < kK1; ++i) a.cond_idx[i] = 0;
-    for (int i = a.n_tr; i < kMaxTr; ++i) a.tr_idx[i] = 0;
-    if (a.n_tr < 1) return false;
-    a.n_lat = L->latent_dim;
-    if (a.n_cond + a.n_lat > kK1) return false;              // [conditioning columns | latent] share GEMM1's 32 K columns
-    a.n_chunks = (a.n_tr + kG - 1) / kG;
-    a.n_bins = L->n_bins;
-    if (a.n_bins < 2 || a.n_bins > kBins) return false;
-    a.kind = L->kind; a.dim = L->dim; a.P = L->kind == STB_RQS ? 3 * a.n_bins - 1 : 2 * a.n_bins + 2;
-    a.act = L->net.activation;
-    a.W1 = L->net.W[0]; a.b1 = L->net.b[0]; a.W2 = L->net.W[1]; a.b2 = L->net.b[1];
-    return true;
+// the shared spline gate, then this file's conditioner: MLP[64]
+static_assert(kMaxTr == kK1, "spline_gate bounds the transformed dims by GEMM1's K");
+static bool admit(const stb_layer* L, MaskSplit& m) {
+    return spline_gate(L, kMaxDim, kK1, m) && L->net.n_linear == 2 && L->net.dims[1] == kHid;
 }
 
 }  // namespace tcl
 
 bool tc_layer_supported(const stb_layer* L) {
-    using namespace tcl;
-    if (L->kind != STB_RQS && L->kind != STB_CUBIC) return false;
-    if (L->n_bins < 2 || L->n_bins > kBins || !L->cond_x || L->zero_cond || L->latent_dim < 0 || L->time_input) return false;
-    if (L->has_box || L->row_out || L->dim < 2 || L->dim > kMaxDim) return false;
-    if (L->spline.custom) return false;                    // non-default spline constants: CUDA-core kernels only
-    const stb_mlp& N = L->net;
-    if (N.n_linear != 2 || N.dims[1] != kHid || N.final_activation != STB_ACT_NONE) return false;
-    if (N.dims[0] != L->dim + L->latent_dim) return false;
-    if (N.dims[2] != L->dim * (L->kind == STB_RQS ? 3 * L->n_bins - 1 : 2 * L->n_bins + 2)) return false;
-    // The hidden activations feed the next GEMM as fp16 hi | lo parts: only activations bounded by 1 are safe
-    // (a ReLU / ELU / ... output above 65504 would split into +inf, -inf -> NaN, where the reference and the
-    // CUDA-core kernel stay finite).  Other activations take the generic kernel.
-    if (N.activation != STB_ACT_TANH && N.activation != STB_ACT_SIGMOID) return false;
-    // the tensor-core epilogues evaluate the inverse log-det as -(forward log-derivative): the Coupling convention
-    if (L->inverse_ldj_own) return false;
-    PackArgs a;
-    return fill_pack_args(L, a);
+    tcl::MaskSplit m;
+    return tcl::admit(L, m);
 }
 
 uint64_t tc_packed_bytes(const stb_layer*) { return tcl::kPackedBytes; }
 
 int tc_pack_layer(const stb_layer* L, void* out, cudaStream_t stream) {
     using namespace tcl;
-    PackArgs a;
-    if (!fill_pack_args(L, a)) return set_error(STB_ENOTSUP, "layer has no tensor-core path");
+    SplinePackArgs a;
+    if (!admit(L, a.m)) return set_error(STB_ENOTSUP, "layer has no tensor-core path");
     a.out = static_cast<uint8_t*>(out);
-    cudaError_t e = cudaMemsetAsync(out, 0, sizeof(Header), stream);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "memset: %s", cudaGetErrorString(e));
-    tc_maxabs_kernel<<<64, 256, 0, stream>>>(a);
-    count_launch();
-    tc_pack_kernel<<<296, 256, 0, stream>>>(a);
-    count_launch();
-    tc_bound_kernel<<<1, kMaxTr * 32, 0, stream>>>(a);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_pack launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    a.n_chunks = (a.m.n_tr + kG - 1) / kG;
+    a.n_lat = L->latent_dim; a.n_bins = L->n_bins;
+    a.kind = L->kind; a.dim = L->dim; a.P = spline_params_per_dim(L->kind, L->n_bins);
+    a.act = L->net.activation;
+    a.W1 = L->net.W[0]; a.b1 = L->net.b[0]; a.W2 = L->net.W[1]; a.b2 = L->net.b[1];
+    const BoundArgs b = spline_bound_args(a.m, a.W2, a.b2, kHid, a.P, a.n_bins, a.act,
+                                          a.out + offsetof(Header, noshift_mask));
+    return pack_image(out, sizeof(Header), stream, "tc_pack", [&] {
+        pack_pass(spline64_maxabs_kernel<PackLayout>, 64, 256, stream, a);
+        pack_pass(spline64_pack_kernel<PackLayout>, 296, 256, stream, a);
+        pack_pass(tc_bound_kernel, 1, kMaxTr * 32, stream, b);
+    });
 }
 
 namespace tcl {
 // the two-CTA whole-flow kernel over A.n_layers >= 1 layers (A.chain_packed / lower_l / upper_l / n_chunks_l filled)
 static int launch_pair(Args& A, int kind, bool full, int64_t rows, cudaStream_t stream) {
-    void (*kern)(Args);
-    if (full) {
-        if (kind == STB_RQS) kern = A.inverse ? tc_spline_pair_kernel<STB_RQS, true, true> : tc_spline_pair_kernel<STB_RQS, false, true>;
-        else kern = A.inverse ? tc_spline_pair_kernel<STB_CUBIC, true, true> : tc_spline_pair_kernel<STB_CUBIC, false, true>;
-    } else {
-        if (kind == STB_RQS) kern = A.inverse ? tc_spline_pair_kernel<STB_RQS, true, false> : tc_spline_pair_kernel<STB_RQS, false, false>;
-        else kern = A.inverse ? tc_spline_pair_kernel<STB_CUBIC, true, false> : tc_spline_pair_kernel<STB_CUBIC, false, false>;
-    }
+    void (*kern)(Args) = pick_variant(kind, A.inverse, full, [](auto K, auto I, auto F) { return tc_spline_pair_kernel<K, I, F>; });
     const long long ptiles = (rows + kPRows - 1) / kPRows;
     if (ptiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)ptiles;
-    cudaError_t pe = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPSmemBytes);
-    if (pe == cudaSuccess) pe = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    const cudaError_t pe = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (pe != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(pe));
-    const int pgrid = (int)min((long long)2 * sm_count(), ptiles);
-    kern<<<pgrid, kPThreads, kPSmemBytes, stream>>>(A);
-    count_launch();
-    pe = cudaGetLastError();
-    if (pe != cudaSuccess) return set_error(STB_ECUDA, "tc_spline_pair_kernel launch: %s", cudaGetErrorString(pe));
-    return STB_OK;
+    return launch_persistent(kern, A, ptiles, 2, kPThreads, kPSmemBytes, stream, "tc_spline_pair_kernel");
 }
 }  // namespace tcl
 
@@ -1213,8 +1066,8 @@ int tc_layer_apply(const stb_layer* L, int direction, const float* x, const floa
     A.lat_stride = L->latent_dim;
     if (L->n_bins != kBins) {            // fewer than 16 bins: the padded-bin variant lives in the two-CTA kernel
         if (bins) return set_error(STB_ENOTSUP, "the bin-index instrument of the tensor-core path covers 16-bin layers");
-        PackArgs pa;
-        if (!fill_pack_args(L, pa)) return set_error(STB_EINVAL, "layer has no tensor-core path");
+        MaskSplit m;
+        if (!admit(L, m)) return set_error(STB_EINVAL, "layer has no tensor-core path");
         A.x = x; A.y = y; A.ldj = ldj;
         A.ldj_mode = ldj ? ldj_mode : STB_LDJ_NONE;
         A.base_log_prob = base_log_prob;
@@ -1223,7 +1076,7 @@ int tc_layer_apply(const stb_layer* L, int direction, const float* x, const floa
         A.n_layers = 1; A.dim = L->dim;
         A.chain_packed[0] = static_cast<const uint8_t*>(L->packed);
         A.lower_l[0] = L->lower; A.upper_l[0] = L->upper;
-        A.n_chunks_l[0] = pa.n_chunks;
+        A.n_chunks_l[0] = (m.n_tr + kG - 1) / kG;
         return launch_pair(A, L->kind, false, rows, stream);
     }
     A.packed = static_cast<const uint8_t*>(L->packed);
@@ -1237,21 +1090,9 @@ int tc_layer_apply(const stb_layer* L, int direction, const float* x, const floa
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
 
-    void (*kern)(Args);
-    if (L->kind == STB_RQS) kern = A.inverse ? tc_spline_layer_kernel<STB_RQS, true, false> : tc_spline_layer_kernel<STB_RQS, false, false>;
-    else kern = A.inverse ? tc_spline_layer_kernel<STB_CUBIC, true, false> : tc_spline_layer_kernel<STB_CUBIC, false, false>;
-    if (bins) {
-        if (L->kind == STB_RQS) kern = A.inverse ? tc_spline_layer_kernel<STB_RQS, true, false, true> : tc_spline_layer_kernel<STB_RQS, false, false, true>;
-        else kern = A.inverse ? tc_spline_layer_kernel<STB_CUBIC, true, false, true> : tc_spline_layer_kernel<STB_CUBIC, false, false, true>;
-    }
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    const int grid = (int)min((long long)sm_count(), tiles);
-    kern<<<grid, kThreads, kSmemBytes, stream>>>(A);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_spline_layer_kernel launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    void (*kern)(Args) = pick_variant(L->kind, A.inverse, bins != nullptr,
+                                      [](auto K, auto I, auto B) { return tc_spline_layer_kernel<K, I, false, B>; });
+    return launch_persistent(kern, A, tiles, 1, kThreads, kSmemBytes, stream, "tc_spline_layer_kernel");
 }
 
 
@@ -1288,17 +1129,15 @@ int tc_chain_apply(const stb_layer* const* layers, int n, int direction, const f
     A.n_layers = n;
     A.dim = layers[0]->dim;
     for (int i = 0; i < n; ++i) {
-        PackArgs pa;
-        if (!fill_pack_args(layers[i], pa)) return set_error(STB_EINVAL, "layer has no tensor-core path");
+        MaskSplit m;
+        if (!admit(layers[i], m)) return set_error(STB_EINVAL, "layer has no tensor-core path");
         A.chain_packed[i] = static_cast<const uint8_t*>(layers[i]->packed);
         A.lower_l[i] = layers[i]->lower; A.upper_l[i] = layers[i]->upper;
-        A.n_chunks_l[i] = pa.n_chunks;
+        A.n_chunks_l[i] = (m.n_tr + kG - 1) / kG;
     }
     const long long tiles = (rows + kTileRows - 1) / kTileRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    const int n_sm = sm_count();
-    void (*kern)(Args);
     // Two independent 128-row CTAs per SM instead of one 256-row CTA.  Measured on the headline workload (2^22 rows):
     // 1.73e8 vs 1.77e8 samples/s -- the heads do fall into the other CTA's chunk phases, but the kernel is bound by
     // the epilogue's instruction stream, not by that bubble, so nothing is gained; it IS faster when there are fewer
@@ -1306,18 +1145,10 @@ int tc_chain_apply(const stb_layer* const* layers, int n, int direction, const f
     // is the kernel of layers with fewer than 16 bins.
     bool full = true;
     for (int i = 0; i < n; ++i) full = full && layers[i]->n_bins == kBins;
-    const bool use_pair = !full || tiles < (long long)n_sm;
+    const bool use_pair = !full || tiles < (long long)sm_count();
     if (use_pair) return launch_pair(A, layers[0]->kind, full, rows, stream);
-    if (layers[0]->kind == STB_RQS) kern = A.inverse ? tc_spline_layer_kernel<STB_RQS, true, true> : tc_spline_layer_kernel<STB_RQS, false, true>;
-    else kern = A.inverse ? tc_spline_layer_kernel<STB_CUBIC, true, true> : tc_spline_layer_kernel<STB_CUBIC, false, true>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    const int grid = (int)min((long long)n_sm, tiles);
-    kern<<<grid, kThreads, kSmemBytes, stream>>>(A);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_spline_layer_kernel (chain) launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    void (*kern)(Args) = pick_variant(layers[0]->kind, A.inverse, [](auto K, auto I) { return tc_spline_layer_kernel<K, I, true>; });
+    return launch_persistent(kern, A, tiles, 1, kThreads, kSmemBytes, stream, "tc_spline_layer_kernel (chain)");
 }
 
 }  // namespace stb

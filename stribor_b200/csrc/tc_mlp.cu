@@ -30,6 +30,7 @@
 #include "common.cuh"
 #include "stb_math.cuh"
 #include "tc_common.cuh"
+#include "tc_pack.cuh"
 
 namespace stb {
 using namespace tc;
@@ -120,20 +121,6 @@ struct Args {
     int n_tiles;
 };
 
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-__device__ __forceinline__ float ex2_approx(float v) {
-    float r;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(v));
-    return r;
-}
-__device__ __forceinline__ float fdiv(float a, float b) {
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(b));
-    const float q = a * r;
-    return fmaf(fmaf(-q, b, a), r, q);
-}
 // exp(v) for the affine scale: 2^p on MUFU.EX2 with p = v log2(e), and the rounding error of that product put back
 // as a first-order correction (e ln 2) -- ~3e-7 relative like expf, 5 instructions instead of ~18
 __device__ __forceinline__ float exp_fast(float v) {
@@ -142,13 +129,9 @@ __device__ __forceinline__ float exp_fast(float v) {
     const float r = ex2_approx(p);
     return fmaf(r, e * 0.6931471805599453f, r);
 }
-__device__ __forceinline__ float tanh_fast(float v) {                 // ~3e-7 absolute error
-    const float t = ex2_approx(-2.885390081777927f * fabsf(v));
-    return copysignf(fdiv(1.f - t, 1.f + t), v);
-}
 
 // Hidden layer of the conditioner for TWO units at a time on Blackwell's packed fp32 pipe (FADD2 / FMUL2 / FFMA2):
-// h = tanh((main + corr) * sc + bias) with the same arithmetic as tanh_fast, then the fp16 hi | lo split, each
+// h = tanh((main + corr) * sc + bias) with the arithmetic of tanh_fast (tc_spline16.cuh), then the fp16 hi | lo split, each
 // part as one packed conversion.  Half the issue slots of the scalar form -- the activation passes were 45 % of
 // the chain kernel's clocks and ~40 % of the MLP[256,256] kernel's stall samples.
 __device__ __forceinline__ void tanh_split2(float2 vm, float2 vc, float2 sc, float2 bias, uint32_t& hi, uint32_t& lo) {
@@ -1254,14 +1237,13 @@ __global__ void __launch_bounds__(V * kVcThreads, 1) tc_mlp_chain_kernel(const C
 struct PackArgs {
     const float *W1, *b1, *W2, *b2, *W3, *b3, *time_scale;
     uint8_t* out;
-    int dim, n_cond, n_tr, H, n_hidden, act, in_dim, cont, time_col, lat0, n_lat;
-    int cond_idx[kK1];
-    int tr_idx[kMaxTr];
+    int dim, H, n_hidden, act, in_dim, cont, time_col, lat0, n_lat;
+    MaskSplit m;
 };
 
 __device__ __forceinline__ int out_row_affine(const PackArgs& a, int n) {     // packed output column -> Linear row
     const int p = n / kMaxTr, ji = n % kMaxTr;
-    return (ji < a.n_tr) ? p * a.dim + a.tr_idx[ji] : -1;
+    return (ji < a.m.n_tr) ? p * a.dim + a.m.tr_idx[ji] : -1;
 }
 
 __global__ void tcm_maxabs_kernel(const PackArgs a) {
@@ -1274,26 +1256,8 @@ __global__ void tcm_maxabs_kernel(const PackArgs a) {
         const int r = out_row_affine(a, i / a.H);
         if (r >= 0) m3 = fmaxf(m3, fabsf(a.W3[(size_t)r * a.H + i % a.H]));
     }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) {
-        m2 = fmaxf(m2, __shfl_xor_sync(0xffffffffu, m2, o));
-        m3 = fmaxf(m3, __shfl_xor_sync(0xffffffffu, m3, o));
-    }
-    if ((threadIdx.x & 31) == 0) {
-        atomicMax(&hdr->max_mid, __float_as_uint(m2));
-        atomicMax(&hdr->max_out, __float_as_uint(m3));
-    }
-}
-
-__device__ __forceinline__ float pow2_scale(float mx) {
-    if (!(mx > 0.f) || !isfinite(mx)) return 1.f;
-    int ex;
-    const float fr = frexpf(mx, &ex);
-    return ldexpf(1.f, (fr == 0.5f) ? ex - 1 : ex);
-}
-// element (n, k) of an [N x 16] K-major block: 2 chunks of 8 elements per row
-__device__ __forceinline__ uint32_t blk_off(int n, int k) {
-    return (uint32_t)((n >> 3) * 256 + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2);
+    warp_max_to(&hdr->max_mid, m2);
+    warp_max_to(&hdr->max_out, m3);
 }
 
 __global__ void tcm_pack_kernel(const PackArgs a) {
@@ -1302,14 +1266,14 @@ __global__ void tcm_pack_kernel(const PackArgs a) {
     const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
     const int H = a.H;
     if (gtid == 0) {
-        hdr->magic = kMagic; hdr->dim = a.dim; hdr->n_cond = a.n_cond; hdr->n_tr = a.n_tr; hdr->H = H;
+        hdr->magic = kMagic; hdr->dim = a.dim; hdr->n_cond = a.m.n_cond; hdr->n_tr = a.m.n_tr; hdr->H = H;
         hdr->n_hidden = a.n_hidden; hdr->act = a.act; hdr->s_mid = s_mid; hdr->s_out = s_out;
-        for (int i = 0; i < kK1; ++i) hdr->cond_idx[i] = a.cond_idx[i];
-        for (int i = 0; i < kMaxTr; ++i) hdr->tr_idx[i] = a.tr_idx[i];
+        for (int i = 0; i < kK1; ++i) hdr->cond_idx[i] = a.m.cond_idx[i];
+        for (int i = 0; i < kMaxTr; ++i) hdr->tr_idx[i] = a.m.tr_idx[i];
         hdr->cont = a.cont; hdr->time_col = a.time_col; hdr->lat0 = a.lat0; hdr->n_lat = a.n_lat;
         for (int i = 0; i < kMaxTr; ++i) {
-            hdr->ts_ls[i] = (a.cont && i < a.n_tr) ? a.time_scale[a.tr_idx[i]] : 0.f;
-            hdr->ts_sh[i] = (a.cont && i < a.n_tr) ? a.time_scale[a.dim + a.tr_idx[i]] : 0.f;
+            hdr->ts_ls[i] = (a.cont && i < a.m.n_tr) ? a.time_scale[a.m.tr_idx[i]] : 0.f;
+            hdr->ts_sh[i] = (a.cont && i < a.m.n_tr) ? a.time_scale[a.dim + a.m.tr_idx[i]] : 0.f;
         }
     }
     float* b1 = reinterpret_cast<float*>(a.out + kOffB1);
@@ -1323,68 +1287,39 @@ __global__ void tcm_pack_kernel(const PackArgs a) {
         const int r = out_row_affine(a, i);
         b3[i] = (r >= 0) ? a.b3[r] : 0.f;
     }
-    // layer 1: blocks (pb = 2, 1, 0) x (kb = 0, 1), each [H x 16] of bf16 part pb
     uint8_t* w = a.out + kOffW;
     for (int i = gtid; i < H * kK1; i += gsz) {
         const int n = i / kK1, k = i % kK1;
-        float v = (k < a.n_cond) ? a.W1[(size_t)n * a.in_dim + a.cond_idx[k]]
-                                 : ((k == a.time_col) ? a.W1[(size_t)n * a.in_dim + a.in_dim - 1] : 0.f);
-        if (k >= a.lat0 && k < a.lat0 + a.n_lat) v = a.W1[(size_t)n * a.in_dim + a.dim + (k - a.lat0)];   // [x * mask | latent | t]
-        __nv_bfloat16 q[3];
-        split_bf16x3(v, q[0], q[1], q[2]);
-        for (int pb = 0; pb < 3; ++pb) {
-            const int b = (2 - pb) * 2 + (k >> 4);
-            *reinterpret_cast<__nv_bfloat16*>(w + (size_t)b * w1_block_bytes(H) + blk_off(n, k & 15)) = q[pb];
-        }
+        store_w1_blocks(w, H, n, k, first_linear_w(a.W1, n, k, a.in_dim, a.dim, a.m, a.time_col, a.lat0, a.n_lat));
     }
     w += 6 * w1_block_bytes(H);
     if (a.n_hidden == 2) {
         const float inv = 1.f / s_mid;
-        for (int i = gtid; i < H * H; i += gsz) {
-            const int n = i / H, k = i % H;
-            __half hi, lo;
-            split_f16(a.W2[i] * inv, hi, lo);
-            uint8_t* blk = w + (size_t)(k >> 4) * w2_block_bytes(H);
-            *reinterpret_cast<__half*>(blk + blk_off(n, k & 15)) = hi;
-            *reinterpret_cast<__half*>(blk + H * 32 + blk_off(n, k & 15)) = lo;
-        }
+        for (int i = gtid; i < H * H; i += gsz) store_hilo_blocks(w, H, i / H, i % H, a.W2[i] * inv);
         w += (size_t)(H / 16) * w2_block_bytes(H);
     }
-    {
-        const float inv = 1.f / s_out;
-        for (int i = gtid; i < kNOut * H; i += gsz) {
-            const int n = i / H, k = i % H;
-            const int r = out_row_affine(a, n);
-            __half hi, lo;
-            split_f16(r >= 0 ? a.W3[(size_t)r * H + k] * inv : 0.f, hi, lo);
-            uint8_t* blk = w + (size_t)(k >> 4) * w3_block_bytes();
-            *reinterpret_cast<__half*>(blk + blk_off(n, k & 15)) = hi;
-            *reinterpret_cast<__half*>(blk + kNOut * 32 + blk_off(n, k & 15)) = lo;
-        }
+    const float inv = 1.f / s_out;
+    for (int i = gtid; i < kNOut * H; i += gsz) {
+        const int n = i / H, k = i % H;
+        const int r = out_row_affine(a, n);
+        store_hilo_blocks(w, kNOut, n, k, r >= 0 ? a.W3[(size_t)r * H + k] * inv : 0.f);
     }
 }
 
+// the mask split, then the GEMM1 slots: [conditioning columns | t (continuous-affine) | latent] within K = 32
 static bool fill_pack_args(const stb_layer* L, PackArgs& a) {
-    if (!L->mask_host) return false;
-    a.n_cond = a.n_tr = 0;
-    for (int j = 0; j < L->dim; ++j) {
-        if (L->mask_host[j]) { if (a.n_cond >= kK1) return false; a.cond_idx[a.n_cond++] = j; }
-        else { if (a.n_tr >= kMaxTr) return false; a.tr_idx[a.n_tr++] = j; }
-    }
-    for (int i = a.n_cond; i < kK1; ++i) a.cond_idx[i] = 0;
-    for (int i = a.n_tr; i < kMaxTr; ++i) a.tr_idx[i] = 0;
-    if (a.n_tr < 1) return false;
+    if (!split_mask(L, kK1, kMaxTr, a.m)) return false;
     const stb_mlp& N = L->net;
     a.in_dim = N.dims[0];
     a.cont = L->kind == STB_CONT_AFFINE;
     a.time_col = -1;
     if (L->time_input) {
-        if (a.n_cond >= kK1) return false;
-        a.time_col = a.n_cond;                                  // first free A1 column
+        if (a.m.n_cond >= kK1) return false;
+        a.time_col = a.m.n_cond;                                // first free A1 column
     }
     a.n_lat = L->latent_dim;
-    a.lat0 = a.n_cond + (a.time_col >= 0 ? 1 : 0);
-    if (a.lat0 + a.n_lat > kK1) return false;                   // conditioning columns, t and latent share GEMM1's 32 K columns
+    a.lat0 = a.m.n_cond + (a.time_col >= 0 ? 1 : 0);
+    if (a.lat0 + a.n_lat > kK1) return false;
     if (a.in_dim != L->dim + a.n_lat + (a.time_col >= 0 ? 1 : 0)) return false;
     a.time_scale = L->time_scale;
     a.dim = L->dim; a.H = N.dims[1]; a.n_hidden = N.n_linear - 1; a.act = N.activation;
@@ -1407,12 +1342,7 @@ bool tcm_layer_supported(const stb_layer* L) {
     const int H = N.dims[1];
     if (H < 64 || H > kMaxH || (H % 64) != 0) return false;
     if (N.n_linear == 3 && N.dims[2] != H) return false;
-    // The hidden activations feed the next GEMM as fp16 hi | lo parts: only activations bounded by 1 are safe
-    // (a ReLU / ELU / ... output above 65504 would split into +inf, -inf -> NaN, where the reference and the
-    // CUDA-core kernel stay finite).  Other activations take the generic kernel.
-    if (N.activation != STB_ACT_TANH && N.activation != STB_ACT_SIGMOID) return false;
-    // the tensor-core epilogues evaluate the inverse log-det as -(forward log-derivative): the Coupling convention
-    if (L->inverse_ldj_own) return false;
+    if (!tc_epilogue_ok(L)) return false;
     PackArgs a;
     return fill_pack_args(L, a);
 }
@@ -1424,15 +1354,10 @@ int tcm_pack_layer(const stb_layer* L, void* out, cudaStream_t stream) {
     PackArgs a;
     if (!fill_pack_args(L, a)) return set_error(STB_ENOTSUP, "layer has no tensor-core path");
     a.out = static_cast<uint8_t*>(out);
-    cudaError_t e = cudaMemsetAsync(out, 0, kOffW, stream);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "memset: %s", cudaGetErrorString(e));
-    tcm_maxabs_kernel<<<64, 256, 0, stream>>>(a);
-    count_launch();
-    tcm_pack_kernel<<<296, 256, 0, stream>>>(a);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tcm_pack launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    return pack_image(out, kOffW, stream, "tcm_pack", [&] {
+        pack_pass(tcm_maxabs_kernel, 64, 256, stream, a);
+        pack_pass(tcm_pack_kernel, 296, 256, stream, a);
+    });
 }
 
 int tcm_layer_apply(const stb_layer* L, int direction, const float* x, const float* latent, const float* t, float* y,
@@ -1457,28 +1382,12 @@ int tcm_layer_apply(const stb_layer* L, int direction, const float* x, const flo
     const uint32_t w_total = 6 * w1_block_bytes(H) + (L->net.n_linear == 3 ? (H / 16) * w2_block_bytes(H) : 0) + (H / 16) * w3_block_bytes();
     const bool small = (H == 64) && (L->dim <= 32) && (w_total <= kStages * kSlotBytes) && (tiles >= 2LL * n_sm);
     // wide conditioners: the pipelined kernel (TMEM-resident activations, GEMMs behind the activation waves)
-    if (!small && H >= 128) {
-        const uint32_t psmem = pipe_smem_bytes(H);
-        cudaError_t pe = cudaFuncSetAttribute(tc_mlp_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem);
-        if (pe != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(pe));
-        const int pgrid = (int)min((long long)n_sm, tiles);
-        tc_mlp_pipe_kernel<<<pgrid, kPipeThreads, psmem, stream>>>(A);
-        count_launch();
-        pe = cudaGetLastError();
-        if (pe != cudaSuccess) return set_error(STB_ECUDA, "tc_mlp_pipe_kernel launch: %s", cudaGetErrorString(pe));
-        return STB_OK;
-    }
+    if (!small && H >= 128)
+        return launch_persistent(tc_mlp_pipe_kernel, A, tiles, 1, kPipeThreads, pipe_smem_bytes(H), stream, "tc_mlp_pipe_kernel");
     const uint32_t smem = small ? Cfg<2>::smem_bytes(H) : Cfg<4>::smem_bytes(H);
     if (smem > 227 * 1024) return set_error(STB_ENOTSUP, "hidden width %d needs %u B of shared memory", H, smem);
-    void (*kern)(Args) = small ? tc_mlp_affine_kernel<2> : tc_mlp_affine_kernel<4>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    const int grid = (int)min((long long)(small ? 2 * n_sm : n_sm), tiles);
-    kern<<<grid, small ? Cfg<2>::kThreads : Cfg<4>::kThreads, smem, stream>>>(A);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_mlp_affine_kernel launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    return small ? launch_persistent(tc_mlp_affine_kernel<2>, A, tiles, 2, Cfg<2>::kThreads, smem, stream, "tc_mlp_affine_kernel")
+                 : launch_persistent(tc_mlp_affine_kernel<4>, A, tiles, 1, Cfg<4>::kThreads, smem, stream, "tc_mlp_affine_kernel");
 }
 
 namespace tcm {
@@ -1824,7 +1733,7 @@ static bool chain4_layout(const stb_layer* const* layers, int n, ChainArgs* A, u
         if (L->net.n_linear != 2 || L->packed_bytes < packed_bytes(64, 1)) return false;
         PackArgs pa;
         if (!fill_pack_args(L, pa)) return false;
-        if (pa.n_cond + (pa.time_col >= 0 ? 1 : 0) > 16 || pa.n_tr > 16) return false;
+        if (pa.m.n_cond + (pa.time_col >= 0 ? 1 : 0) > 16 || pa.m.n_tr > 16) return false;
         if (A) A->packed[i] = static_cast<const uint8_t*>(L->packed);
     }
     const int xs_stride = d | 1;
@@ -1865,15 +1774,9 @@ int tcm_chain_apply(const stb_layer* const* layers, int n, int direction, const 
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
     void (*kern)(ChainArgs) = four ? tc_mlp_chain4_kernel<0> : tc_mlp_chain_kernel<kChainV>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     const int vper = four ? kV4 : kChainV;
-    const int grid = (int)min((long long)sm_count(), (tiles + vper - 1) / vper);
-    kern<<<grid, four ? kV4Threads : kChainV * kVcThreads, smem, stream>>>(A);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tc_mlp_chain_kernel launch: %s", cudaGetErrorString(e));
-    return STB_OK;
+    return launch_persistent(kern, A, (tiles + vper - 1) / vper, 1, four ? kV4Threads : kChainV * kVcThreads, smem, stream,
+                             "tc_mlp_chain_kernel");
 }
 
 }  // namespace stb

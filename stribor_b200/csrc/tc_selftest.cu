@@ -5,14 +5,10 @@
 // PyTorch matmul for fp16 / tf32, single-pass and the 3-pass hi/lo split the layer kernel uses.
 #include "common.cuh"
 #include "tc_common.cuh"
+#include "tc_pack.cuh"
 
 namespace stb {
 using namespace tc;
-
-__device__ __forceinline__ uint32_t core_offset(int r, int k, int K, int elem) {
-    const int epc = 16 / elem, chunks = K / epc;
-    return (uint32_t)((r >> 3) * (chunks * 128) + (k / epc) * 128 + (r & 7) * 16 + (k % epc) * elem);
-}
 
 __device__ void pack_operand(uint8_t* hi_s, uint8_t* lo_s, const float* g, int rows, int K, int tf32) {
     for (int i = threadIdx.x; i < rows * K; i += blockDim.x) {
@@ -21,13 +17,13 @@ __device__ void pack_operand(uint8_t* hi_s, uint8_t* lo_s, const float* g, int r
         if (tf32) {
             float hi, lo;
             split_tf32(v, hi, lo);
-            const uint32_t off = core_offset(r, k, K, 4);
+            const uint32_t off = core_off(r, k, K, 4);
             *reinterpret_cast<float*>(hi_s + off) = hi;
             *reinterpret_cast<float*>(lo_s + off) = lo;
         } else {
             __half hi, lo;
             split_f16(v, hi, lo);
-            const uint32_t off = core_offset(r, k, K, 2);
+            const uint32_t off = core_off(r, k, K, 2);
             *reinterpret_cast<__half*>(hi_s + off) = hi;
             *reinterpret_cast<__half*>(lo_s + off) = lo;
         }

@@ -28,6 +28,7 @@
 #include "common.cuh"
 #include "stb_math.cuh"
 #include "tc_common.cuh"
+#include "tc_pack.cuh"
 #include "tc_spline16.cuh"
 
 namespace stb {
@@ -126,9 +127,6 @@ struct Args {
     const float* latent;      // FWD, optional: [rows, n_lat]
 };
 
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
 // i / dv for 0 <= i < 2^16, 1 <= dv <= 2^7 with a precomputed magic = ceil(2^32 / dv): exact (i * (magic * dv - 2^32) <
 // 2^23), one IMAD.HI instead of the ~20-instruction runtime division in the tile staging loops
 // (dv == 1: the magic 2^32 does not fit and is stored as 0 = "divide by one")
@@ -1311,196 +1309,57 @@ __global__ void __launch_bounds__(kTThreads, 1) tc_wide_train_kernel(const Args 
 // -----------------------------------------------------------------------------------------------
 // packing
 // -----------------------------------------------------------------------------------------------
-struct PackArgs {
-    const float *W1, *b1, *W2, *b2;
-    uint8_t* out;
-    int kind, dim, n_cond, n_tr, n_chunks, P, act, n_lat, n_bins;
-    int16_t colmap[kMaxDim];
-    uint8_t cond_idx[kK1];
-    uint8_t tr_idx[kMaxTr];
+// the image's layout for spline64_pack_kernel (tc_pack.cuh), plus this file's header fields: the division magics and
+// the column -> slot map
+struct PackLayout {
+    using Hdr = Header;
+    static constexpr uint32_t kMagic = tcw::kMagic, kOffB1 = tcw::kOffB1, kOffW1 = tcw::kOffW1;
+    static constexpr int kK1 = tcw::kK1, kMaxTr = tcw::kMaxTr;
+    static __device__ void header_extra(Header* hdr, const SplinePackArgs& a) {
+        const int n_cond = a.m.n_cond;
+        hdr->k1pad = (n_cond + a.n_lat + 15) & ~15;
+        if (hdr->k1pad == 0) hdr->k1pad = 16;
+        hdr->m_d = div_magic(a.dim); hdr->m_d4 = div_magic(max(a.dim >> 2, 1)); hdr->m_ntr = div_magic(a.m.n_tr);
+        hdr->m_npad = div_magic(max(hdr->k1pad - n_cond - a.n_lat, 1));
+        hdr->m_npad64 = div_magic(max(kK1 - n_cond, 1));
+        for (int j = 0; j < kMaxDim; ++j) hdr->colmap[j] = 0;
+        for (int i = 0; i < n_cond; ++i) hdr->colmap[a.m.cond_idx[i]] = (int16_t)i;
+        for (int i = 0; i < a.m.n_tr; ++i) hdr->colmap[a.m.tr_idx[i]] = (int16_t)(-i - 1);
+    }
 };
 
-__global__ void tcw_maxabs_kernel(const PackArgs a) {
-    float m = 0.f;
-    const int total = a.n_tr * a.P * kHid;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
-        const int k = i % kHid, rp = i / kHid, p = rp % a.P, ji = rp / a.P;
-        m = fmaxf(m, fabsf(a.W2[((size_t)a.tr_idx[ji] * a.P + p) * kHid + k]));
-    }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-    if ((threadIdx.x & 31) == 0) atomicMax(&reinterpret_cast<Header*>(a.out)->maxbits, __float_as_uint(m));
-}
-
-// -> parameter index in the network's [w(K) | h(K) | rest] order, -1 for padding (as tc_layer.cu)
-__host__ __device__ __forceinline__ int param_of_col(int c, int K, int P) {
-    if (c < 2 * kBins) {
-        const int i = c >> 1;
-        return (i < K) ? ((c & 1) ? K + i : i) : -1;
-    }
-    const int p = 2 * K + (c - 2 * kBins);
-    return (p < P) ? p : -1;
-}
-__device__ __forceinline__ uint32_t core_off(int r, int k, int K, int elem) {
-    const int epc = 16 / elem, chunks = K / epc;
-    return (uint32_t)((r >> 3) * (chunks * 128) + (k / epc) * 128 + (r & 7) * 16 + (k % epc) * elem);
-}
-
-__global__ void tcw_pack_kernel(const PackArgs a) {
-    Header* hdr = reinterpret_cast<Header*>(a.out);
-    const float mx = __uint_as_float(hdr->maxbits);
-    float s2 = 1.f;
-    if (mx > 0.f && isfinite(mx)) {
-        int ex;
-        const float fr = frexpf(mx, &ex);
-        s2 = ldexpf(1.f, (fr == 0.5f) ? ex - 1 : ex);
-    }
-    const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
-    if (gtid == 0) {
-        hdr->magic = kMagic; hdr->kind = a.kind; hdr->dim = a.dim; hdr->n_cond = a.n_cond; hdr->n_tr = a.n_tr;
-        hdr->n_chunks = a.n_chunks; hdr->P = a.P; hdr->act = a.act; hdr->s2 = s2;
-        hdr->n_lat = a.n_lat; hdr->n_bins = a.n_bins;
-        hdr->k1pad = (a.n_cond + a.n_lat + 15) & ~15;
-        if (hdr->k1pad == 0) hdr->k1pad = 16;
-        hdr->m_d = div_magic(a.dim); hdr->m_d4 = div_magic(max(a.dim >> 2, 1)); hdr->m_ntr = div_magic(a.n_tr);
-        hdr->m_npad = div_magic(max(hdr->k1pad - a.n_cond - a.n_lat, 1));
-        hdr->m_npad64 = div_magic(max(kK1 - a.n_cond, 1));
-        if (hdr->k1pad == 0) hdr->k1pad = 16;
-        for (int i = 0; i < kK1; ++i) hdr->cond_idx[i] = a.cond_idx[i];
-        for (int i = 0; i < kMaxTr; ++i) hdr->tr_idx[i] = a.tr_idx[i];
-        for (int i = 0; i < kMaxDim; ++i) hdr->colmap[i] = a.colmap[i];
-    }
-    float* b1 = reinterpret_cast<float*>(a.out + kOffB1);
-    float* b2 = reinterpret_cast<float*>(a.out + kOffB2);
-    for (int i = gtid; i < kHid; i += gsz) b1[i] = a.b1[i];
-    for (int i = gtid; i < kMaxChunks * kChunkN; i += gsz) {
-        const int ji = i / kPPad, col = i % kPPad, p = param_of_col(col, a.n_bins, a.P);
-        float bv = (ji < a.n_tr && p >= 0) ? a.b2[a.tr_idx[ji] * a.P + p] : 0.f;
-        if (col < 2 * kBins && p < 0 && ji < a.n_tr) bv = -INFINITY;   // padded bin: numerator exactly 0
-        b2[i] = (col < 2 * kBins) ? bv * 1.4426950408889634f : bv;
-    }
-    for (int i = gtid; i < kHid * kK1; i += gsz) {
-        const int n = i / kK1, k = i % kK1;
-        const size_t in1 = (size_t)(a.dim + a.n_lat);          // the first Linear reads [x * mask | latent]
-        const float v = (k < a.n_cond) ? a.W1[n * in1 + a.cond_idx[k]]
-                                       : ((k < a.n_cond + a.n_lat) ? a.W1[n * in1 + a.dim + (k - a.n_cond)] : 0.f);
-        __nv_bfloat16 q0, q1, q2;
-        split_bf16x3(v, q0, q1, q2);
-        const uint32_t off = kOffW1 + core_off(n, k, kK1, 2);
-        *reinterpret_cast<__nv_bfloat16*>(a.out + off) = q0;
-        *reinterpret_cast<__nv_bfloat16*>(a.out + off + kW1Part) = q1;
-        *reinterpret_cast<__nv_bfloat16*>(a.out + off + 2 * kW1Part) = q2;
-    }
-    const float inv = 1.f / s2;
-    for (int i = gtid; i < kMaxChunks * kChunkN * kHid; i += gsz) {
-        const int k = i % kHid, rn = i / kHid, n = rn % kChunkN, c = rn / kChunkN;
-        const int ji = c * kG + n / kPPad, p = param_of_col(n % kPPad, a.n_bins, a.P);
-        float v = 0.f;
-        if (c < a.n_chunks && ji < a.n_tr && p >= 0) v = a.W2[((size_t)a.tr_idx[ji] * a.P + p) * kHid + k] * inv;
-        __half hi, lo;
-        split_f16(v, hi, lo);
-        const uint32_t off = kOffW2 + (uint32_t)c * kChunkBytes + core_off(n, k, kHid, 2);
-        *reinterpret_cast<__half*>(a.out + off) = hi;
-        *reinterpret_cast<__half*>(a.out + off + 12288) = lo;
-    }
-}
-
-__global__ void tcw_bound_kernel(const PackArgs a) {
-    const int ji = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), p = threadIdx.x & 31;
-    bool ok = false;
-    if (ji < a.n_tr && (a.act == STB_ACT_TANH || a.act == STB_ACT_SIGMOID)) {
-        ok = true;
-        if (p < 2 * a.n_bins) {                              // the 2 K softmax rows of the dim
-            const size_t row = (size_t)a.tr_idx[ji] * a.P + p;
-            float l1 = fabsf(a.b2[row]);
-            for (int k = 0; k < kHid; ++k) l1 += fabsf(a.W2[row * kHid + k]);
-            ok = (l1 * 1.4426950408889634f <= 100.f);
-        }
-    }
-    ok = __all_sync(0xffffffffu, ok);
-    if (p == 0 && ok && ji < kMaxTr) atomicOr(&reinterpret_cast<Header*>(a.out)->noshift_mask[ji >> 5], 1u << (ji & 31));
-}
-
-static bool fill_pack_args(const stb_layer* L, PackArgs& a) {
-    if (!L->mask_host) return false;
-    a.n_cond = a.n_tr = 0;
-    for (int j = 0; j < L->dim; ++j) {
-        if (L->mask_host[j]) {
-            if (a.n_cond >= kK1) return false;
-            a.colmap[j] = (int16_t)a.n_cond;
-            a.cond_idx[a.n_cond++] = (uint8_t)j;
-        } else {
-            if (a.n_tr >= kMaxTr) return false;
-            a.colmap[j] = (int16_t)(-a.n_tr - 1);
-            a.tr_idx[a.n_tr++] = (uint8_t)j;
-        }
-    }
-    for (int j = L->dim; j < kMaxDim; ++j) a.colmap[j] = 0;
-    for (int i = a.n_cond; i < kK1; ++i) a.cond_idx[i] = 0;
-    for (int i = a.n_tr; i < kMaxTr; ++i) a.tr_idx[i] = 0;
-    if (a.n_tr < 1) return false;
-    a.n_lat = L->latent_dim;
-    if (a.n_lat < 0 || a.n_cond + a.n_lat > kK1 || L->net.dims[0] != L->dim + a.n_lat) return false;
-    a.n_chunks = (a.n_tr + kG - 1) / kG;
-    a.n_bins = L->n_bins;
-    if (a.n_bins < 2 || a.n_bins > kBins) return false;
-    a.kind = L->kind; a.dim = L->dim; a.P = L->kind == STB_RQS ? 3 * a.n_bins - 1 : 2 * a.n_bins + 2;
-    if (L->net.dims[2] != L->dim * a.P) return false;
-    a.act = L->net.activation;
-    a.W1 = L->net.W[0]; a.b1 = L->net.b[0]; a.W2 = L->net.W[1]; a.b2 = L->net.b[1];
-    return true;
+// the shared spline gate, then this file's conditioner: MLP[64]
+static_assert(kMaxTr == kK1, "spline_gate bounds the transformed dims by GEMM1's K");
+static bool admit(const stb_layer* L, MaskSplit& m) {
+    return spline_gate(L, kMaxDim, kK1, m) && L->net.n_linear == 2 && L->net.dims[1] == kHid;
 }
 
 }  // namespace tcw
 
 bool tcw_layer_supported(const stb_layer* L) {
-    using namespace tcw;
-    if (L->kind != STB_RQS && L->kind != STB_CUBIC) return false;
-    if (L->n_bins < 2 || L->n_bins > kBins || !L->cond_x || L->zero_cond || L->latent_dim < 0 || L->time_input) return false;
-    if (L->has_box || L->row_out || L->dim < 2 || L->dim > kMaxDim) return false;
-    if (L->spline.custom) return false;                    // non-default spline constants: CUDA-core kernels only
-    const stb_mlp& N = L->net;
-    if (N.n_linear != 2 || N.dims[1] != kHid || N.final_activation != STB_ACT_NONE) return false;
-    // The hidden activations feed the next GEMM as fp16 hi | lo parts: only activations bounded by 1 are safe
-    // (a ReLU / ELU / ... output above 65504 would split into +inf, -inf -> NaN, where the reference and the
-    // CUDA-core kernel stay finite).  Other activations take the generic kernel.
-    if (N.activation != STB_ACT_TANH && N.activation != STB_ACT_SIGMOID) return false;
-    // the tensor-core epilogues evaluate the inverse log-det as -(forward log-derivative): the Coupling convention
-    if (L->inverse_ldj_own) return false;
-    PackArgs a;
-    return fill_pack_args(L, a);
+    tcw::MaskSplit m;
+    return tcw::admit(L, m);
 }
 
 uint64_t tcw_packed_bytes(const stb_layer*) { return tcw::kPackedBytes; }
 
 int tcw_pack_layer(const stb_layer* L, void* out, cudaStream_t stream) {
     using namespace tcw;
-    PackArgs a;
-    if (!fill_pack_args(L, a)) return set_error(STB_ENOTSUP, "layer has no wide tensor-core path");
+    SplinePackArgs a;
+    if (!admit(L, a.m)) return set_error(STB_ENOTSUP, "layer has no wide tensor-core path");
     a.out = static_cast<uint8_t*>(out);
-    cudaError_t e = cudaMemsetAsync(out, 0, sizeof(Header), stream);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "memset: %s", cudaGetErrorString(e));
-    tcw_maxabs_kernel<<<64, 256, 0, stream>>>(a);
-    count_launch();
-    tcw_pack_kernel<<<296, 256, 0, stream>>>(a);
-    count_launch();
-    tcw_bound_kernel<<<(kMaxTr + 7) / 8, 256, 0, stream>>>(a);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "tcw_pack launch: %s", cudaGetErrorString(e));
-    return STB_OK;
-}
-
-static int tcw_launch(void (*kern)(tcw::Args), const tcw::Args& A, long long tiles, cudaStream_t stream, const char* what) {
-    using namespace tcw;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes);
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-    const int grid = (int)min((long long)sm_count(), tiles);
-    kern<<<grid, kThreads, kSmemBytes, stream>>>(A);
-    count_launch();
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return set_error(STB_ECUDA, "%s launch: %s", what, cudaGetErrorString(e));
-    return STB_OK;
+    a.n_chunks = (a.m.n_tr + kG - 1) / kG;
+    a.n_lat = L->latent_dim; a.n_bins = L->n_bins;
+    a.kind = L->kind; a.dim = L->dim; a.P = spline_params_per_dim(L->kind, L->n_bins);
+    a.act = L->net.activation;
+    a.W1 = L->net.W[0]; a.b1 = L->net.b[0]; a.W2 = L->net.W[1]; a.b2 = L->net.b[1];
+    const BoundArgs b = spline_bound_args(a.m, a.W2, a.b2, kHid, a.P, a.n_bins, a.act,
+                                          a.out + offsetof(Header, noshift_mask));
+    return pack_image(out, sizeof(Header), stream, "tcw_pack", [&] {
+        pack_pass(spline64_maxabs_kernel<PackLayout>, 64, 256, stream, a);
+        pack_pass(spline64_pack_kernel<PackLayout>, 296, 256, stream, a);
+        pack_pass(tc_bound_kernel, (kMaxTr + 7) / 8, 256, stream, b);
+    });
 }
 
 int tcw_layer_apply(const stb_layer* L, const void* image, int direction, const float* x, const float* latent, float* y,
@@ -1518,16 +1377,9 @@ int tcw_layer_apply(const stb_layer* L, const void* image, int direction, const 
     const long long tiles = (rows + kTileRows - 1) / kTileRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    const bool inv = direction == STB_INVERSE;
-    void (*kern)(Args);
-    if (L->n_bins == kBins) {
-        if (L->kind == STB_RQS) kern = inv ? tc_wide_kernel<STB_RQS, true, false> : tc_wide_kernel<STB_RQS, false, false>;
-        else kern = inv ? tc_wide_kernel<STB_CUBIC, true, false> : tc_wide_kernel<STB_CUBIC, false, false>;
-    } else {
-        if (L->kind == STB_RQS) kern = inv ? tc_wide_kernel<STB_RQS, true, false, false> : tc_wide_kernel<STB_RQS, false, false, false>;
-        else kern = inv ? tc_wide_kernel<STB_CUBIC, true, false, false> : tc_wide_kernel<STB_CUBIC, false, false, false>;
-    }
-    return tcw_launch(kern, A, tiles, stream, "tc_wide_kernel");
+    void (*kern)(Args) = pick_variant(L->kind, direction == STB_INVERSE, L->n_bins == kBins,
+                                      [](auto K, auto I, auto F) { return tc_wide_kernel<K, I, false, F>; });
+    return launch_persistent(kern, A, tiles, 1, kThreads, kSmemBytes, stream, "tc_wide_kernel");
 }
 
 // quadratic and cubic (fused variant); `latent=` layers train through the element-wise kernels + autograd
@@ -1549,7 +1401,7 @@ int tcw_layer_backward(const stb_layer* L, const void* image, int direction, con
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
     void (*kern)(Args) = (direction == STB_INVERSE) ? tc_wide_kernel<STB_RQS, true, true> : tc_wide_kernel<STB_RQS, false, true>;
-    return tcw_launch(kern, A, tiles, stream, "tc_wide_kernel (backward)");
+    return launch_persistent(kern, A, tiles, 1, kThreads, kSmemBytes, stream, "tc_wide_kernel (backward)");
 }
 
 
@@ -1616,10 +1468,8 @@ int tcw_layer_backward_fused(const stb_layer* L, const void* image, int directio
     const long long tiles = (rows + kTileRows - 1) / kTileRows;
     if (tiles > 0x7fffffffLL) return set_error(STB_EINVAL, "too many rows");
     A.n_tiles = (int)tiles;
-    const bool inv = direction == STB_INVERSE;
-    void (*kern)(train::Args);
-    if (L->kind == STB_RQS) kern = inv ? train::tc_wide_train_kernel<STB_RQS, true> : train::tc_wide_train_kernel<STB_RQS, false>;
-    else kern = inv ? train::tc_wide_train_kernel<STB_CUBIC, true> : train::tc_wide_train_kernel<STB_CUBIC, false>;
+    void (*kern)(train::Args) = pick_variant(L->kind, direction == STB_INVERSE,
+                                             [](auto K, auto I) { return train::tc_wide_train_kernel<K, I>; });
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)train::kSmemBytes);
     if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     int grid = (int)min((long long)sm_count(), tiles);

@@ -167,18 +167,27 @@ def test_backward_workspace_layout_constants_match_the_kernels():
     assert all(param_of_col(c) == p for p, c in enumerate(cols))
 
 
-def _spline_struct(dim, kind='quadratic', hidden=64, n_bins=16, latent_dim=0):
-    """stb_layer for Coupling(Spline(dim, n_bins), MLP(dim, [hidden], dim * P)) with an ordered mask; the weight
-    pointers are CPU tensors -- the host-side entry points below never dereference them."""
-    import ctypes as C
+def _spline_struct(dim, kind='quadratic', hidden=64, n_bins=16, latent_dim=0, act='Tanh', time_input=0, inv_own=0,
+                   custom=0, mask=None):
+    """stb_layer for Coupling(Spline(dim, n_bins), MLP(dim, [hidden], dim * P)) with an ordered mask (kind 'affine' /
+    'cont': Affine / ContinuousAffineCoupling, hidden may be a list); the weight pointers are CPU tensors -- the
+    host-side entry points below never dereference them."""
     from stribor_b200 import _lib, _ops
-    P = 3 * n_bins - 1 if kind == 'quadratic' else 2 * n_bins + 2
-    mask_list = [0] * (dim // 2) + [1] * (dim - dim // 2)
-    meta = [_lib.RQS if kind == 'quadratic' else _lib.CUBIC, dim, latent_dim, 1, 0, n_bins, 0, 0, _lib.ACTIVATIONS['Tanh'], 0,
-            2, 4, 0, 0, dim + latent_dim, hidden, dim * P] + mask_list
-    params = [torch.zeros(hidden, dim + latent_dim), torch.zeros(hidden), torch.zeros(dim * P, hidden), torch.zeros(dim * P)]
+    kinds = {'quadratic': _lib.RQS, 'cubic': _lib.CUBIC, 'affine': _lib.AFFINE, 'cont': _lib.CONT_AFFINE}
+    P = {'quadratic': 3 * n_bins - 1, 'cubic': 2 * n_bins + 2}.get(kind, 2)
+    hidden = list(hidden) if isinstance(hidden, (list, tuple)) else [hidden]
+    dims = [dim + latent_dim + time_input] + hidden + [dim * P]
+    mask_list = mask if mask is not None else [0] * (dim // 2) + [1] * (dim - dim // 2)
+    params = []
+    for i in range(len(dims) - 1):
+        params += [torch.zeros(dims[i + 1], dims[i]), torch.zeros(dims[i + 1])]
+    if kind == 'cont':
+        params.append(torch.zeros(2 * dim))                    # TimeLinear.scale
+    meta = [kinds[kind], dim, latent_dim, 1, time_input, n_bins, inv_own, 0, _lib.ACTIVATIONS[act], 0,
+            len(dims) - 1, len(params), 0, 0] + dims + mask_list
+    fmeta = [-4., 4., 0., 1., 0., 1.] + ([1, 1e-2, 1e-2, 1e-2, 0, 1e-6, 1e-3] if custom else [])
     mask = torch.tensor(mask_list, dtype=torch.uint8)
-    L = _ops.make_struct(meta, [-4., 4., 0., 1., 0., 1.], mask, params, None)
+    L = _ops.make_struct(meta, fmeta, mask, params, None)
     L._keep = (params, mask)
     return L
 
@@ -213,6 +222,33 @@ def test_cabi_host_side_dispatch_without_a_gpu():
     assert lib.stb_layer_backward_workspace_bytes(C.byref(_spline_struct(32, latent_dim=8)), 10) == 0
     big = lib.stb_packed_bytes(C.byref(_spline_struct(64, hidden=256, n_bins=10)))                      # wide conditioner, MLP[256]
     assert big > tc_bytes and lib.stb_packed_bytes(C.byref(_spline_struct(64, hidden=256, n_bins=16))) == big
+    # wide-conditioner splines (tc_hwide.cu): header + biases 9216 B, W1 6 blocks of [H x 16] bf16, W2 (H / 16) blocks of
+    # [H x 16] hi | lo, W3 32 dims x [48 x H] hi | lo
+    hw = lambda H, n_hidden: 9216 + 6 * H * 32 + (H // 16 * H * 64 if n_hidden == 2 else 0) + 32 * H * 192
+    assert big == hw(256, 1)
+    assert lib.stb_packed_bytes(C.byref(_spline_struct(64, hidden=[64, 64]))) == hw(64, 2)
+    assert lib.stb_packed_bytes(C.byref(_spline_struct(64, hidden=128, kind='cubic'))) == hw(128, 1)
+    # affine / continuous-affine (tc_mlp.cu): 4096 B header + biases, W1 6 blocks, W2 (H / 16) blocks, W3 (H / 16) x [64 x 16]
+    mlp = lambda H, n_hidden: 4096 + 6 * H * 32 + (H // 16 * H * 64 if n_hidden == 2 else 0) + H // 16 * 4096
+    assert lib.stb_packed_bytes(C.byref(_spline_struct(32, kind='affine'))) == mlp(64, 1)
+    assert lib.stb_packed_bytes(C.byref(_spline_struct(64, kind='affine', hidden=[256, 256]))) == mlp(256, 2)
+    assert lib.stb_packed_bytes(C.byref(_spline_struct(16, kind='cont', time_input=1))) == mlp(64, 1)
+    # no tensor-core path: H = 96, an unbounded activation, conditioning + t + latent over GEMM1's 32 columns, custom
+    # spline constants, the layer's own inverse log-det
+    for L in (_spline_struct(64, hidden=96), _spline_struct(64, kind='affine', hidden=96), _spline_struct(64, act='ReLU'),
+              _spline_struct(32, kind='affine', act='ReLU'), _spline_struct(64, kind='cont', time_input=1, latent_dim=0),
+              _spline_struct(32, kind='cont', time_input=1, latent_dim=16), _spline_struct(64, custom=1),
+              _spline_struct(64, hidden=256, custom=1), _spline_struct(64, inv_own=1), _spline_struct(32, kind='affine', inv_own=1)):
+        assert lib.stb_packed_bytes(C.byref(L)) == 0
+        assert lib.stb_layer_uses_tensor_path(C.byref(L)) == 0
+    # log_prob without the [rows, dim] scratch: two packed layers of each chain family go out as one launch
+    for a, b in ((_spline_struct(64), _spline_struct(64, mask=[1] * 32 + [0] * 32)),
+                 (_spline_struct(16, kind='affine'), _spline_struct(16, kind='affine')),
+                 (_spline_struct(16, kind='cont', time_input=1), _spline_struct(16, kind='cont', time_input=1))):
+        for L in (a, b):
+            L.packed, L.packed_bytes = 0x1000, lib.stb_packed_bytes(C.byref(L))
+            assert lib.stb_layer_uses_tensor_path(C.byref(L)) == 1
+        assert lib.stb_flow_log_prob_needs_x_out((_lib.StbLayer * 2)(a, b), 2) == 0
     # argument validation returns STB_EINVAL (-1) before anything is launched
     L = _spline_struct(64)
     dummy = C.c_void_p(0x1000)
