@@ -23,8 +23,13 @@
  * or a negative STB_E* code; stb_last_error() gives a thread-local message.  The CALLER owns
  * every buffer (device pointers unless stated), the library never allocates device memory,
  * never synchronises and keeps no global mutable state, so calls are re-entrant across
- * streams, devices and host threads.  All tensors are fp32, row-major, rows contiguous:
- * x/y [rows, dim], latent [rows, latent_dim], t [rows, 1], ldj/lp [rows].
+ * streams, devices and host threads.  Tensors are row-major, rows contiguous:
+ * x/y [rows, dim], latent [rows, latent_dim], t [rows, 1], ldj/lp [rows].  They are fp32, or fp64
+ * when the layers say so (stb_layer.dtype == STB_F64): then EVERY float pointer of the call and of
+ * its layers -- x, y, latent, t, ldj / lp, ldiag, x_out, g_* and the layer's W / b, const_out,
+ * row_out, time_scale -- points to double, while the float fields of the structs (spline boxes,
+ * stb_spline_opts) stay float.  fp64 runs on the CUDA-core kernels only: no packed image, no
+ * tensor-core path and no fused conditioner backward.  stb_unit_normal_log_prob is fp32 only.
  */
 #ifndef STRIBOR_B200_H_
 #define STRIBOR_B200_H_
@@ -36,7 +41,7 @@
 extern "C" {
 #endif
 
-#define STB_ABI_VERSION 3
+#define STB_ABI_VERSION 4
 #define STB_MAX_LINEAR 8
 
 /* error codes */
@@ -55,6 +60,9 @@ enum { STB_AFFINE = 0, STB_RQS = 1, STB_CUBIC = 2, STB_CONT_AFFINE = 3,
 /* activations by torch.nn class name (net/mlp.py:38-41) */
 enum { STB_ACT_NONE = 0, STB_ACT_TANH = 1, STB_ACT_RELU = 2, STB_ACT_SIGMOID = 3, STB_ACT_ELU = 4,
        STB_ACT_SOFTPLUS = 5, STB_ACT_LEAKY_RELU = 6, STB_ACT_SILU = 7, STB_ACT_GELU = 8 };
+
+/* scalar type of a layer's tensors (stb_layer.dtype) */
+enum { STB_F32 = 0, STB_F64 = 1 };
 
 /* directions */
 enum { STB_FORWARD = 0, STB_INVERSE = 1 };
@@ -143,6 +151,9 @@ typedef struct stb_layer {
     const int32_t* perm_inv_host;  /* between chained couplings is folded into the neighbouring kernels'    */
                                    /* gather / scatter index lists instead of costing an HBM pass           */
     stb_spline_opts spline;        /* rqs / cubic constants; zero-filled = the reference defaults          */
+    int32_t dtype;                 /* STB_F32 (0, so a zero-filled field means fp32) or STB_F64: the type   */
+                                   /* every float pointer of the call and of the layer points to; all the   */
+                                   /* layers of one chain share it (STB_EINVAL otherwise)                    */
 } stb_layer;
 
 int stb_abi_version(void);
@@ -189,7 +200,8 @@ int stb_flow_log_prob_needs_x_out(const stb_layer* layers, int n_layers);
 int stb_flow_log_prob(const stb_layer* layers, int n_layers, const float* y, const float* latent,
                       const float* t, float* x_out, float* lp, int64_t rows, void* stream);
 
-/* lp[row] (+)= sum_j -x_j^2/2 - log(sqrt(2 pi))   (dist/normal.py:37) */
+/* lp[row] (+)= sum_j -x_j^2/2 - log(sqrt(2 pi))   (dist/normal.py:37); fp32 only (fp64 callers get the base
+ * term from stb_flow_log_prob) */
 int stb_unit_normal_log_prob(const float* x, float* lp, int accumulate, int32_t dim, int64_t rows,
                              void* stream);
 
@@ -226,7 +238,8 @@ int stb_unit_normal_log_prob(const float* x, float* lp, int accumulate, int32_t 
  *          workspace[0 : rows*72]            [hidden(64) | 1 | 0 x 7] per row; the caller forms
  *                                            g_pre = (g_row_out W_last) * act'(hidden) and all four products
  *      gW / gb pointers of stb_layer_grads are not used by this family.
- *      Any other layer with n_linear > 0 returns STB_ENOTSUP. */
+ *      Any other layer with n_linear > 0 returns STB_ENOTSUP, fp64 layers included (family (2) is fp32 only;
+ *      their workspace size is 0).  Family (1) runs in fp64 as in fp32. */
 typedef struct stb_layer_grads {
     float* gW[STB_MAX_LINEAR];
     float* gb[STB_MAX_LINEAR];
@@ -263,7 +276,8 @@ int stb_layer_backward_diag(const stb_layer* layer, int direction, const float* 
 uint64_t stb_packed_bytes(const stb_layer* layer);
 int stb_pack_layer(const stb_layer* layer, void* packed_out, void* stream);
 
-/* 1 if stb_layer_apply would take the tcgen05 path for this (packed) layer. */
+/* 1 if stb_layer_apply would take the tcgen05 path for this (packed) layer.
+ * fp64 layers (STB_F64): stb_packed_bytes returns 0, stb_pack_layer STB_EINVAL, stb_layer_uses_tensor_path 0. */
 int stb_layer_uses_tensor_path(const stb_layer* layer);
 
 /* Bring-up check of the tcgen05 building blocks: D[128,N] = A[128,K] * B[N,K]^T on one CTA.

@@ -10,10 +10,11 @@ import ctypes as C
 import os
 
 STB_MAX_LINEAR = 8
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 # enums (include/stribor_b200.h)
 AFFINE, RQS, CUBIC, CONT_AFFINE, PERMUTE, SIGMOID, LOGIT = 0, 1, 2, 3, 4, 5, 6
+F32, F64 = 0, 1
 FORWARD, INVERSE = 0, 1
 LDJ_NONE, LDJ_SET, LDJ_ADD = 0, 1, 2
 ACTIVATIONS = {None: 0, 'Identity': 0, 'Tanh': 1, 'ReLU': 2, 'Sigmoid': 3, 'ELU': 4, 'Softplus': 5,
@@ -51,7 +52,8 @@ class StbLayer(C.Structure):
                 ('mask', C.c_void_p), ('mask_host', C.c_void_p), ('const_out', C.c_void_p), ('row_out', C.c_void_p),
                 ('time_scale', C.c_void_p), ('perm', C.c_void_p), ('perm_inv', C.c_void_p),
                 ('net', StbMlp), ('packed', C.c_void_p), ('packed_bytes', C.c_uint64),
-                ('perm_host', C.c_void_p), ('perm_inv_host', C.c_void_p), ('spline', StbSplineOpts)]
+                ('perm_host', C.c_void_p), ('perm_inv_host', C.c_void_p), ('spline', StbSplineOpts),
+                ('dtype', C.c_int32)]
 
 
 class StbLayerGrads(C.Structure):

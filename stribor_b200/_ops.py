@@ -35,20 +35,25 @@ FMETA_LEN = 6
 SPLINE_OPTS_LEN = 7
 
 
+DTYPES = {torch.float32: _lib.F32, torch.float64: _lib.F64}
+
+
 def _check_cuda(x: Tensor, what: str):
     if not x.is_cuda:
         raise RuntimeError(
             f'stribor_b200: {what} is on {x.device}; this package runs its transforms in CUDA '
             'kernels only (sm_100a) and has no CPU fallback -- move the module and inputs to a GPU.')
-    if x.dtype != torch.float32:
-        raise TypeError(f'stribor_b200: {what} must be float32, got {x.dtype}')
+    if x.dtype not in DTYPES:
+        raise TypeError(f'stribor_b200: {what} must be float32 or float64, got {x.dtype}')
 
 
 def check_layer_tensors(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor], mask: Optional[Tensor],
                         params: Sequence[Tensor], packed: Optional[Tensor] = None, int_params: bool = False):
     """Every tensor whose raw pointer is handed to the kernels must live on x's device with the dtype the
-    kernels read: a float64 ``t`` / ``latent`` would be reinterpreted as float32, a module left on the CPU
-    (or another GPU) would hand a foreign pointer to the kernel.  Raise the reference-style Python error instead."""
+    kernels read -- x's, float32 or float64, for every floating tensor of the call (mixed dtypes are not
+    promoted): a float64 ``t`` / ``latent`` next to a float32 input would be reinterpreted as float32 pairs, a
+    module left on the CPU (or another GPU) would hand a foreign pointer to the kernel.  Raise the
+    reference-style Python error instead."""
     _check_cuda(x, 'input')
     dev = x.device
 
@@ -63,11 +68,11 @@ def check_layer_tensors(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor]
         if not v.is_contiguous():
             raise ValueError(f'stribor_b200: {what} must be contiguous')
 
-    same(latent, '`latent`', torch.float32)
-    same(t, '`t`', torch.float32)
+    same(latent, '`latent`', x.dtype)
+    same(t, '`t`', x.dtype)
     same(mask, 'the coupling mask', torch.uint8)
     for i, p in enumerate(params):
-        same(p, f'layer parameter {i}', torch.int32 if int_params else torch.float32)
+        same(p, f'layer parameter {i}', torch.int32 if int_params else x.dtype)
     same(packed, 'the packed weight image', torch.uint8)
 
 
@@ -80,7 +85,8 @@ def _stream(x: Tensor):
 
 
 def _fill_struct(L: _lib.StbLayer, meta: Sequence[int], fmeta: Sequence[float], mask: Optional[Tensor],
-                 params: Sequence[Tensor], packed: Optional[Tensor]):
+                 params: Sequence[Tensor], packed: Optional[Tensor], dtype: torch.dtype = torch.float32):
+    """``dtype``: the input tensor's, which every float pointer of the call points to (stb_layer.dtype)."""
     (kind, dim, latent_dim, cond_x, time_input, n_bins, inv_own, zero_cond, act, fact, n_linear,
      n_params, has_box, row_mode) = meta[:META_HEADER]
     L.kind, L.dim, L.latent_dim, L.cond_x = kind, dim, latent_dim, cond_x
@@ -88,6 +94,7 @@ def _fill_struct(L: _lib.StbLayer, meta: Sequence[int], fmeta: Sequence[float], 
     L.lower, L.upper = float(fmeta[0]), float(fmeta[1])
     L.left, L.right, L.bottom, L.top = (float(v) for v in fmeta[2:6])
     L.has_box = has_box
+    L.dtype = DTYPES[dtype]
     if len(fmeta) > FMETA_LEN:
         custom, mw, mh, md, free_edge, eps, quad = fmeta[FMETA_LEN:FMETA_LEN + SPLINE_OPTS_LEN]
         o = L.spline
@@ -149,9 +156,9 @@ def _fill_struct(L: _lib.StbLayer, meta: Sequence[int], fmeta: Sequence[float], 
     return keep
 
 
-def make_struct(meta, fmeta, mask, params, packed=None) -> _lib.StbLayer:
+def make_struct(meta, fmeta, mask, params, packed=None, dtype=torch.float32) -> _lib.StbLayer:
     L = _lib.StbLayer()
-    L._keepalive = _fill_struct(L, meta, fmeta, mask, params, packed)
+    L._keepalive = _fill_struct(L, meta, fmeta, mask, params, packed, dtype)
     return L
 
 
@@ -174,7 +181,7 @@ def layer_apply(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor], mask: 
     ldj = torch.empty(rows if want_ldj else 0, dtype=x.dtype, device=x.device)
     if rows == 0:
         return y, ldj
-    L = make_struct(meta, fmeta, mask, params, packed)
+    L = make_struct(meta, fmeta, mask, params, packed, x.dtype)
     with torch.cuda.device(x.device):
         rc = _lib.lib().stb_layer_apply(C.byref(L), direction, x.data_ptr(), _dp(latent), _dp(t),
                                         y.data_ptr(), _dp(ldj), _lib.LDJ_SET if want_ldj else _lib.LDJ_NONE,
@@ -199,7 +206,7 @@ def layer_apply_diag(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor], m
     ldiag = torch.empty_like(x)
     if rows == 0:
         return y, ldiag
-    L = make_struct(meta, fmeta, mask, params, None)
+    L = make_struct(meta, fmeta, mask, params, None, x.dtype)
     with torch.cuda.device(x.device):
         rc = _lib.lib().stb_layer_apply_diag(C.byref(L), direction, x.data_ptr(), _dp(latent), _dp(t),
                                              y.data_ptr(), ldiag.data_ptr(), rows, _stream(x))
@@ -221,8 +228,8 @@ def _const_param_slabs(rows: int, numel: int):
     return [(s0, min(slab, rows - s0)) for s0 in range(0, rows, slab)]
 
 
-def _off(ptr, count, width=1):
-    return None if ptr is None else ptr + 4 * count * width
+def _off(ptr, count, width=1, esize=4):
+    return None if ptr is None else ptr + esize * count * width
 
 
 @torch.library.custom_op('stribor_b200::layer_backward_diag', mutates_args=(), device_types='cuda')
@@ -238,7 +245,7 @@ def layer_backward_diag(x: Tensor, mask: Optional[Tensor], params: List[Tensor],
     g_x = torch.empty_like(x)
     if rows == 0:
         return [g_x, torch.zeros_like(p0)]
-    L = make_struct(meta, fmeta, mask, params, None)
+    L = make_struct(meta, fmeta, mask, params, None, x.dtype)
     G = _lib.StbLayerGrads()
     lib = _lib.lib()
     if row_mode:
@@ -252,11 +259,12 @@ def layer_backward_diag(x: Tensor, mask: Optional[Tensor], params: List[Tensor],
     g_rows = x.new_empty(slabs[0][1], p0.numel())
     g_p = x.new_zeros(p0.numel())
     G.g_row_out = g_rows.data_ptr()
+    es = x.element_size()
     with torch.cuda.device(x.device):
         for s0, n in slabs:
             g_rows[:n].zero_()
-            _lib.check(lib.stb_layer_backward_diag(C.byref(L), direction, _off(x.data_ptr(), s0, dim), _off(g_y.data_ptr(), s0, dim),
-                                                   _off(_dp(g_ld), s0, dim), _off(g_x.data_ptr(), s0, dim), C.byref(G), n, _stream(x)))
+            _lib.check(lib.stb_layer_backward_diag(C.byref(L), direction, _off(x.data_ptr(), s0, dim, es), _off(g_y.data_ptr(), s0, dim, es),
+                                                   _off(_dp(g_ld), s0, dim, es), _off(g_x.data_ptr(), s0, dim, es), C.byref(G), n, _stream(x)))
             g_p += g_rows[:n].sum(0)
     return [g_x, g_p.view_as(p0)]
 
@@ -298,7 +306,7 @@ def layer_apply_bins(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor], m
     bins = torch.full((rows, dim), -1, dtype=torch.int32, device=x.device)
     if rows == 0:
         return y, ldj, bins
-    L = make_struct(meta, fmeta, mask, params, packed)
+    L = make_struct(meta, fmeta, mask, params, packed, x.dtype)
     with torch.cuda.device(x.device):
         rc = _lib.lib().stb_layer_apply_bins(C.byref(L), direction, x.data_ptr(), _dp(latent), _dp(t),
                                              y.data_ptr(), ldj.data_ptr(), _lib.LDJ_SET, bins.data_ptr(),
@@ -366,7 +374,7 @@ def _fused_conditioner_backward(x, mask, params, packed, meta, fmeta, direction,
     if rows == 0:
         g_x.zero_()
         return [g_x, x.new_empty(0), x.new_empty(0), gW1, gb1, gW2, gb2]
-    L = make_struct(meta, fmeta, mask, params, packed)
+    L = make_struct(meta, fmeta, mask, params, packed, x.dtype)
     lib = _lib.lib()
     ws_bytes = int(lib.stb_layer_backward_workspace_bytes(C.byref(L), rows)) if packed is not None else 0
     if act not in (_lib.ACTIVATIONS['Tanh'], _lib.ACTIVATIONS['Sigmoid'], _lib.ACTIVATIONS['ReLU']):
@@ -473,7 +481,7 @@ def layer_backward(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor], mas
         g_x.zero_()
         return [g_x, g_latent, g_t, torch.zeros_like(p0)]
     # per-row gradient wrt the network output; a broadcast (const) parameter sums it over rows, slab by slab
-    L = make_struct(meta, fmeta, mask, params, None)
+    L = make_struct(meta, fmeta, mask, params, None, x.dtype)
     G = _lib.StbLayerGrads()
     lib = _lib.lib()
     if row_mode:
@@ -489,12 +497,13 @@ def layer_backward(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor], mas
     g_p = x.new_zeros(p0.numel())
     G.g_row_out = g_rows.data_ptr()
     lat_w = 0 if latent is None else latent.shape[-1]
+    es = x.element_size()
     with torch.cuda.device(x.device):
         for s0, n in slabs:
             g_rows[:n].zero_()
-            _lib.check(lib.stb_layer_backward(C.byref(L), direction, _off(x.data_ptr(), s0, dim), _off(_dp(latent), s0, lat_w),
-                                              _off(_dp(t), s0), _off(g_y.data_ptr(), s0, dim), _off(_dp(g_ldj), s0),
-                                              _off(g_x.data_ptr(), s0, dim), None, None, C.byref(G), None, n, _stream(x)))
+            _lib.check(lib.stb_layer_backward(C.byref(L), direction, _off(x.data_ptr(), s0, dim, es), _off(_dp(latent), s0, lat_w, es),
+                                              _off(_dp(t), s0, 1, es), _off(g_y.data_ptr(), s0, dim, es), _off(_dp(g_ldj), s0, 1, es),
+                                              _off(g_x.data_ptr(), s0, dim, es), None, None, C.byref(G), None, n, _stream(x)))
             g_p += g_rows[:n].sum(0)
     return [g_x, g_latent, g_t, g_p.view_as(p0)]
 
@@ -541,8 +550,8 @@ CHAIN_FORWARD, CHAIN_INVERSE, CHAIN_LOG_PROB, CHAIN_LOG_PROB_ONLY = 0, 1, 2, 3
 
 
 def build_layer_array(masks: List[Tensor], params: List[Tensor], packed: List[Tensor], meta: List[int],
-                      fmeta: List[float]):
-    """-> (ctypes array of stb_layer, objects that must outlive it)."""
+                      fmeta: List[float], dtype: torch.dtype = torch.float32):
+    """-> (ctypes array of stb_layer, objects that must outlive it); ``dtype`` is the input's."""
     n_layers = len(masks)
     arr = (_lib.StbLayer * n_layers)()
     keep = []
@@ -552,7 +561,7 @@ def build_layer_array(masks: List[Tensor], params: List[Tensor], packed: List[Te
         m = meta[mo:mo + ml]
         npar = m[11]
         keep.append(_fill_struct(arr[i], m, fmeta[FMETA_LEN * i:FMETA_LEN * (i + 1)], masks[i],
-                                 params[po:po + npar], packed[i]))
+                                 params[po:po + npar], packed[i], dtype))
         mo += ml
         po += npar
     return arr, keep
@@ -590,7 +599,7 @@ def flow_chain_direct(x: Tensor, latent: Optional[Tensor], t: Optional[Tensor], 
                       mode: int, want_ldj: bool) -> Tuple[Tensor, Tensor]:
     """mode FORWARD/INVERSE: (out [rows,dim], ldj [rows] or empty);
     mode LOG_PROB: (latent x [rows,dim], log_prob [rows])."""
-    arr, keep = build_layer_array(masks, params, packed, meta, fmeta)
+    arr, keep = build_layer_array(masks, params, packed, meta, fmeta, x.dtype)
     out = flow_chain_launch(arr, len(masks), x, latent, t, mode, want_ldj)
     del keep
     return out

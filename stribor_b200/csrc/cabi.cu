@@ -196,6 +196,15 @@ static int apply_sequence(const stb_layer* const* seq, int n, int direction, con
     return STB_OK;
 }
 
+// one dtype per chain: the kernels hand each layer's output to the next as it is
+static int check_one_dtype(const stb_layer* layers, int n_layers) {
+    for (int i = 1; i < n_layers; ++i)
+        if (layers[i].dtype != layers[0].dtype)
+            return set_error(STB_EINVAL, "layer %d has dtype %d but layer 0 has %d: a flow runs in one dtype", i,
+                             layers[i].dtype, layers[0].dtype);
+    return STB_OK;
+}
+
 }  // namespace stb
 
 using namespace stb;
@@ -239,6 +248,7 @@ int stb_flow_apply(const stb_layer* layers, int n_layers, int direction, const f
     cudaStream_t s = (cudaStream_t)stream;
     if (n_layers == 0) return set_error(STB_EINVAL, "empty flow: nothing to apply");
     if (n_layers > 64) return set_error(STB_EINVAL, "more than 64 layers");
+    if (int rc = check_one_dtype(layers, n_layers)) return rc;
     const stb_layer* order[64];
     for (int i = 0; i < n_layers; ++i) order[i] = &layers[direction == STB_FORWARD ? i : n_layers - 1 - i];
     return apply_sequence(order, n_layers, direction, x, latent, t, out, ldj, ldj_mode, 0, rows, s);
@@ -257,6 +267,7 @@ int stb_flow_log_prob(const stb_layer* layers, int n_layers, const float* y, con
     if (!lp) return set_error(STB_EINVAL, "lp is NULL");
     cudaStream_t s = (cudaStream_t)stream;
     if (n_layers > 64) return set_error(STB_EINVAL, "more than 64 layers");
+    if (int rc = check_one_dtype(layers, n_layers)) return rc;
     const stb_layer* order[64];
     for (int i = 0; i < n_layers; ++i) order[i] = &layers[n_layers - 1 - i];
     if (!x_out && !(stb_flow_log_prob_needs_x_out(layers, n_layers) == 0))
@@ -306,6 +317,7 @@ int stb_pack_layer(const stb_layer* layer, void* packed_out, void* stream) {
     int rc = validate_layer(layer);
     if (rc) return rc;
     if (!packed_out) return set_error(STB_EINVAL, "packed_out is NULL");
+    if (layer->dtype != STB_F32) return set_error(STB_EINVAL, "fp64 layers have no packed image (CUDA-core kernels only)");
     PackedImage img[2];
     const int n = layer_images(layer, img);
     if (n == 0) return set_error(STB_ENOTSUP, "layer has no tensor-core path");

@@ -20,6 +20,22 @@ struct LayerArgs {
 
 int set_error(int code, const char* fmt, ...);
 void count_launch();
+
+// Launch `kern` (raising its dynamic shared-memory limit first when it needs more than 48 KB), count the
+// launch and report a failed launch as STB_ECUDA.
+template <class... KArgs, class... Args>
+int launch_kernel(void (*kern)(KArgs...), unsigned grid, int threads, size_t smem, cudaStream_t stream,
+                  const char* name, Args... args) {
+    if (smem > 48 * 1024) {
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return set_error(STB_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    }
+    kern<<<grid, threads, smem, stream>>>(args...);
+    count_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_error(STB_ECUDA, "%s launch: %s", name, cudaGetErrorString(e));
+    return STB_OK;
+}
 // multiprocessors of the current device, looked up once per host thread (148, a B200's count, if the query fails)
 int sm_count();
 

@@ -15,6 +15,7 @@ bool split_mask(const stb_layer* L, int max_cond, int max_tr, MaskSplit& m) {
 }
 
 bool tc_epilogue_ok(const stb_layer* L) {
+    if (L->dtype != STB_F32) return false;                  // the tensor-core kernels read and write fp32 only
     // The hidden activations feed the next GEMM as fp16 hi | lo parts: only activations bounded by 1 are safe
     // (a ReLU / ELU / ... output above 65504 would split into +inf, -inf -> NaN, where the reference and the
     // CUDA-core kernel stay finite).  Other activations take the generic kernel.

@@ -62,7 +62,7 @@ struct MaskSplit {
 // transform
 bool split_mask(const stb_layer* L, int max_cond, int max_tr, MaskSplit& m);
 
-// What every tensor-core epilogue needs of a coupling: a hidden activation bounded by 1 (tanh, sigmoid) and the Coupling's
+// What every tensor-core epilogue needs of a coupling: fp32 tensors (STB_F32), a hidden activation bounded by 1 (tanh, sigmoid) and the Coupling's
 // inverse log-det convention.
 bool tc_epilogue_ok(const stb_layer* L);
 

@@ -167,7 +167,7 @@ def _build_plan(transforms, dim, latent_dim, x, latent, t) -> _Plan:
         pl.fmeta += d['fmeta']
         if getattr(f, '_packed', None) is not None:
             pl.caches.append(f._packed)
-    pl.arr, pl.keep = _ops.build_layer_array(pl.masks, pl.params, pl.packed, pl.meta, pl.fmeta)
+    pl.arr, pl.keep = _ops.build_layer_array(pl.masks, pl.params, pl.packed, pl.meta, pl.fmeta, x.dtype)
     pl.n = len(pl.masks)
     return pl
 
@@ -178,7 +178,8 @@ def run_chain(transforms, mode, x, latent=None, t=None, want_ldj=False):
     latent_dim = 0 if latent is None else latent.shape[-1]
     latent, t = _flat(latent, lead), _flat(t, lead)
     rec = _record(transforms)
-    key = (dim, latent_dim, x.device, os.environ.get('STRIBOR_B200_FORCE_GENERIC'))
+    # (x.dtype: a plan's layers carry its dtype; an input of the other dtype builds -- and dtype-checks -- its own)
+    key = (dim, latent_dim, x.device, x.dtype, os.environ.get('STRIBOR_B200_FORCE_GENERIC'))
     epoch = _epoch.value
     plan = rec.plans.get(key)
     if plan is None:

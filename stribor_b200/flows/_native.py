@@ -63,6 +63,8 @@ class PackedCache:
     def get(self, meta, fmeta, mask, params):
         if not params or not params[0].is_cuda or os.environ.get('STRIBOR_B200_FORCE_GENERIC') == '1':
             return None
+        if params[0].dtype != torch.float32:
+            return None               # float64 layers run on the CUDA-core kernels only: no image
         key = (tuple(meta), tuple(fmeta), tuple((p.data_ptr(), p._version) for p in params))
         if key == self.key:
             if self.buf is not None:

@@ -158,7 +158,7 @@ class Coupling(PackedOwner, Transform):
             return None
         key = ('fused_bwd', x.shape[-1], str(x.device), tuple(d['meta']))
         if key not in self._masks:
-            L = _ops.make_struct(d['meta'], d['fmeta'], d['mask'], [p.detach() for p in d['params']], d['packed'])
+            L = _ops.make_struct(d['meta'], d['fmeta'], d['mask'], [p.detach() for p in d['params']], d['packed'], x.dtype)
             act_ok = d['meta'][8] in (_lib.ACTIVATIONS['Tanh'], _lib.ACTIVATIONS['Sigmoid'], _lib.ACTIVATIONS['ReLU'])
             self._masks[key] = bool(act_ok and _ops.fused_backward_ok(L))
         return d if self._masks[key] else None

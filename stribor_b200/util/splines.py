@@ -28,6 +28,9 @@ def _row_params_call(kind, inputs, pieces, n_bins, inverse, fmeta, has_box):
     shape = inputs.shape
     dim = shape[-1]
     x = inputs.reshape(-1, dim).contiguous()
+    for p in pieces:
+        if p.dtype != inputs.dtype:
+            raise TypeError(f'stribor_b200: spline parameters must be {inputs.dtype} like the inputs, got {p.dtype}')
     prm = torch.cat([p.expand(*shape, p.shape[-1]) for p in pieces], -1).reshape(x.shape[0], -1).contiguous()
     meta = [kind, dim, 0, 0, 0, n_bins, 1, 0, 0, 0, 0, 1, int(has_box), 1]
     y, ld = _ops.layer_apply_diag(x, None, None, None, [prm], meta, fmeta,
